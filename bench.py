@@ -129,7 +129,8 @@ def cpu_step(o, ch, cores, ncnst=0):
         do2 = np.zeros(ncnst, np.int32); do2[3:] = 1
         dry = np.zeros(ncnst, np.int32); dry[3::3] = 1
         r = o.conv_tend_batch(ch, nthreads=cores, convtran1=dict(doconvtran=do1, cnst_is_dry=dry, q=q3, fracis=fracis))
-        o.conv_tend_2_batch(do2, q3, pdeldry, fracis, ch.ztodt, dry, r, ptend_q=r["ptend_qc"], nthreads=cores)
+        r["ptend_qc"] = o.conv_tend_2_batch(do2, q3, pdeldry, fracis, ch.ztodt, dry, r, ptend_q=r["ptend_qc"],
+                                            nthreads=cores)
     if r["rc"]:
         raise RuntimeError("oracle Brent failure")
     return r
@@ -160,6 +161,29 @@ def shard_of(rank, world, ncols, scaling):
     return 16 * c0, min(ncols, 16 * c1) - 16 * c0
 
 
+DUMP_BYTES = 60_000_000     # --dump-outputs stays under 64 MB in all, .npy headers included
+DUMP_SEED = 20261020
+
+
+def dump_outputs(path, chunked, totals=None):
+    """Writes every output array as <path>/<name>.npy in float64 (integer fields convert exactly).  `chunked` arrays
+    lead with the chunk dimension: when they exceed DUMP_BYTES in all, every one keeps the same sample of whole chunks,
+    the first ones of a seeded permutation of all chunks, so two runs with the same arguments write the same elements
+    and a smaller sample is a subset of a larger one.  The chosen chunks go to chunk_index.npy (0-based, ascending).
+    `totals` are written whole."""
+    import numpy as np
+    nch = len(next(iter(chunked.values())))
+    per_chunk = sum(np.asarray(a)[0].size for a in chunked.values()) * 8
+    keep = min(nch, max(1, (DUMP_BYTES - 8 * nch) // per_chunk))
+    idx = np.sort(np.random.default_rng(DUMP_SEED).permutation(nch)[:keep])
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "chunk_index.npy"), idx.astype(np.float64))
+    for k, a in chunked.items():
+        np.save(os.path.join(path, k + ".npy"), np.asarray(a)[idx].astype(np.float64))
+    for k, a in (totals or {}).items():
+        np.save(os.path.join(path, k + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -177,7 +201,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true", help="skip the config 2 / config 4 lines of the default run")
     ap.add_argument("--parcel-pbl", action="store_true", help="zmconv_parcel_pbl=.true. (CAM6 L58 default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float64; "
+                         "rank 0's shard; above 60 MB a fixed seeded sample of whole chunks)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     # stdout carries the JSON line and nothing else: libraries that write to file descriptor 1 (NCCL prints its
     # version banner there) are sent to stderr for the whole run, the line goes to the saved descriptor
@@ -222,10 +251,12 @@ def main():
         times = []
         for i in range(args.warmup + args.steps):
             t0 = time.perf_counter()
-            cpu_step(o, ch, cores, args.convtran)
+            r = cpu_step(o, ch, cores, args.convtran)
             dt = time.perf_counter() - t0
             if i >= args.warmup:
                 times.append(dt)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {k: v for k, v in r.items() if k != "rc"})
         t = statistics.mean(times)
         rate = args.ncols / t
         line = {"impl": "reference", "metric": METRIC, "value": rate, "unit": UNIT, "n_gpus": args.gpus,
@@ -317,6 +348,11 @@ def main():
     ms_per_step, launches, nfail, cons = timed_run(dev, args.steps, args.warmup)
     value = ncols_job / (ms_per_step * 1e-3)
     cons_h = cons.cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        outs = {k: v.cpu().numpy() for k, v in dev.out.items()}
+        if dev.ncnst:
+            outs["ptend_qc"] = dev.ptend_qc.cpu().numpy()
+        dump_outputs(args.dump_outputs, outs, {"conservation": cons_h})
     kavg = kernel_profile(dev, min(args.steps, 10))
     gptl = Z.timers() if hasattr(Z, "timers") else {}
 

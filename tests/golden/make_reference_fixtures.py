@@ -1,6 +1,6 @@
 """Generates tests/golden/reftext_*.npz: outputs of the REFERENCE'S OWN SOURCE TEXT for seeded inputs.
 
-physics/zm_conv.F90 is read from /root/reference (this container only), every routine on the hot path is translated
+physics/zm_conv.F90 is read from the CAM-Nor source tree named by $CAM_NOR_SRC, every routine on the hot path is translated
 mechanically to Python by fortran_exec.py (statement by statement; nothing is re-derived by hand) and executed:
 zm_convi, zm_convr (-> buoyan_dilute, parcel_dilute, entropy, enthalpy, ientropy, ienthalpy, qsat_hPa, cldprp,
 closure, q1q2_pjr, buoyan for cam3), zm_conv_evap, momtran, convtran.  Inputs, namelist values and outputs are stored;
@@ -11,7 +11,7 @@ The externals that are NOT part of the reference tree (wv_saturation::qsat_water
 physconst values, constituents::cnst_get_type_byind) are supplied here in Python with the formulas SURVEY.md 8c
 lists -- those stay unpinned (there is no reference text for them).
 
-usage:  python tests/golden/make_reference_fixtures.py        (needs /root/reference; ~1 minute)
+usage:  CAM_NOR_SRC=<CAM-Nor checkout> python tests/golden/make_reference_fixtures.py        (~1 minute)
 """
 import math
 import os
@@ -25,9 +25,13 @@ sys.path.insert(0, HERE); sys.path.insert(0, ROOT); sys.path.insert(0, os.path.j
 import fortran_exec as F                      # noqa: E402
 from cam_nor_physics_b200 import soundings as S   # noqa: E402
 
-SRC = "/root/reference/physics/zm_conv.F90"
-INTR = "/root/reference/physics/zm_conv_intr.F90"
-PTYPES = "/root/reference/physics/physics_types.F90"
+PHYSICS = os.path.join(os.environ.get("CAM_NOR_SRC", ""), "physics")
+if not os.environ.get("CAM_NOR_SRC") or not os.path.isfile(os.path.join(PHYSICS, "zm_conv.F90")):
+    raise SystemExit("CAM_NOR_SRC must name a CAM-Nor source tree (with physics/zm_conv.F90); it is %r"
+                     % os.environ.get("CAM_NOR_SRC"))
+SRC = os.path.join(PHYSICS, "zm_conv.F90")
+INTR = os.path.join(PHYSICS, "zm_conv_intr.F90")
+PTYPES = os.path.join(PHYSICS, "physics_types.F90")
 ROUTINES = ["zm_convi", "qsat_hpa", "entropy", "enthalpy", "ientropy", "ienthalpy", "parcel_dilute", "buoyan_dilute",
             "buoyan", "cldprp", "closure", "q1q2_pjr", "zm_convr", "zm_conv_evap", "momtran", "convtran"]
 
@@ -289,7 +293,7 @@ def run_geopotential():
     c = physconst()
     fx = {}
     for lr in (1, 0):
-        m = F.Module("/root/reference/physics/geopotential.F90",
+        m = F.Module(os.path.join(PHYSICS, "geopotential.F90"),
                      dict(pcols=pcols, pver=L, pverp=L + 1, dycore_is=(lambda s, lr=lr: s == "LR" if lr else s == "EUL")),
                      lenient=True)       # the MPAS/SE branch uses module data that is not in scope: kept as run-time stops
         m.load("geopotential_t")
@@ -330,7 +334,7 @@ def run_geopotential_gen():
     for lr in (0, 1):
         names = ("SE", "LR") if lr else ("SE",)
         sp = F.FArr((len(species),), data=species.astype(np.int64)) if hasattr(F, "FArr") else species
-        m = F.Module("/root/reference/physics/geopotential.F90",
+        m = F.Module(os.path.join(PHYSICS, "geopotential.F90"),
                      dict(pcols=pcols, pver=L, pverp=L + 1, dycore_is=(lambda s, names=names: s in names),
                           thermodynamic_active_species_num=len(species), thermodynamic_active_species_idx=sp),
                      lenient=True)
@@ -382,7 +386,7 @@ def run_convect_diagnostics():
     ns = dict(idx)
     ns.update(pcols=pcols, pver=L, pverp=L + 1, shallow_scheme="CLUBB_SGS", pbuf_get_field=pbuf_get_field,
               pbuf_set_field=pbuf_set_field, outfld=outfld, _OUTS={"pbuf_get_field": [2]})
-    m = F.Module("/root/reference/physics/convect_diagnostics.F90", ns, lenient=True)
+    m = F.Module(os.path.join(PHYSICS, "convect_diagnostics.F90"), ns, lenient=True)
     m.load("convect_diagnostics_calc")
     state = F.FStruct()
     state.lchnk, state.ncol = 1, ncol

@@ -1,5 +1,5 @@
-"""Randomised pin of the CPU oracle to the reference's own source text (CPU only; reads /root/reference, so it runs in
-the build container, not on the GPU box): random chunk widths, level counts, namelist values, zm_org / cam3 and
+"""Randomised pin of the CPU oracle to the reference's own source text (CPU only; reads the CAM-Nor source tree named by
+$CAM_NOR_SRC, which is not part of this repository): random chunk widths, level counts, namelist values, zm_org / cam3 and
 level-wise perturbed soundings go through the translated reference text (make_reference_fixtures.run_case) and through
 the glibc-libm oracle; every output of zm_convr, zm_conv_evap, momtran, convtran and the zm_conv_tend glue must agree
 bit for bit (the comparison is tests/test_oracle.py::test_oracle_equals_reference_source_text).

@@ -36,7 +36,8 @@ def test_library_is_built_from_the_sources_in_the_tree(built):
 def test_sm100a_code_is_embedded(built):
     import subprocess
     from cam_nor_physics_b200 import build
-    out = subprocess.run(["cuobjdump", "-lelf", build.LIB], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(os.path.realpath(build._nvcc())), "cuobjdump")   # nvcc's own toolkit
+    out = subprocess.run([cuobjdump, "-lelf", build.LIB], capture_output=True, text=True).stdout
     assert "sm_100a" in out
 
 

@@ -352,8 +352,9 @@ def test_oracle_equals_reference_source_text_sweep():
     assert not bad, bad
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/physics"),
-                    reason="executes the reference source text: build container only, never on the GPU box")
+@pytest.mark.skipif(not os.path.isfile(os.path.join(os.environ.get("CAM_NOR_SRC", "/nonexistent"), "physics",
+                                                    "zm_conv.F90")),
+                    reason="executes the reference source text: set CAM_NOR_SRC to a CAM-Nor source tree")
 def test_oracle_equals_reference_source_text_random_chunks():
     """A short run of tests/golden/reference_text_fuzz.py: random chunks / namelist values / zm_org / cam3 / perturbed
     soundings through the reference text and the glibc-libm oracle, bit for bit (the 300-case run of round 1 is
