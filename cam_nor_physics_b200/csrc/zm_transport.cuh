@@ -27,7 +27,9 @@ struct EvapArgs {
   double *ps = nullptr, *pq = nullptr;
 };
 
-template <bool FUSED>
+// HIST (fused step with history fields attached, zm_conv_tend_hist_fields): the fused kernel also stores its own
+// tend_s and the four diagnostics above, all five non-NULL (the caller substitutes scratch for unattached ones)
+template <bool FUSED, bool HIST = false>
 __global__ void __launch_bounds__(128)
 k_conv_evap(EvapArgs a) {
   const int pcols = P.pcols, pver = P.pver, pverp = P.pverp;
@@ -40,9 +42,10 @@ k_conv_evap(EvapArgs a) {
     for (int k = 0; k < pver; ++k) {
       const size_t e = cidx(c, k, i, pver);
       if (FUSED) { a.ps[e] = 0.0; a.pq[e] = 0.0; } else a.tend_s[e] = 0.0;
+      if (HIST) a.tend_s[e] = 0.0;
       a.tend_q[e] = 0.0;
       // tend_s_snwprd, tend_s_snwevmlt, ntprprd, ntsnprd are history diagnostics (zm_conv_intr.F90:779-794): all four
-      // NULL inside the fused zm_conv_tend step
+      // NULL inside the fused zm_conv_tend step unless zm_conv_tend_hist_fields attached them
       if (a.ntprprd) { a.tend_s_snwprd[e] = 0.0; a.tend_s_snwevmlt[e] = 0.0; a.ntprprd[e] = 0.0; a.ntsnprd[e] = 0.0; }
     }
     for (int k = 0; k < pverp; ++k) { a.flxprec[cidx(c, k, i, pverp)] = 0.0; a.flxsnow[cidx(c, k, i, pverp)] = 0.0; }
@@ -105,6 +108,7 @@ k_conv_evap(EvapArgs a) {
     a.flxsnow[cidx(c, k, i, pverp)] = flxsnow;
     const double tend_s = -evpprec * latvap + ntsnprd * latice;
     if (FUSED) { a.ps[e] = heat_k + tend_s; a.pq[e] = qtnd_k + evpprec; } else a.tend_s[e] = tend_s;
+    if (HIST) a.tend_s[e] = tend_s;
     a.tend_q[e] = evpprec;
   }
   a.prec[col] = div_z(flxprec, 1000.0);
@@ -202,6 +206,21 @@ __global__ void k_momtran_init(MomArgs a) {
     if (m < 2 && a.domom[m]) a.dqdt[e] = 0.0;
   }
   for (size_t e = tid; e < n2; e += nth) a.seten[e] = 0.0;
+}
+
+// momtran's in-cloud winds icwu / icwd of the fused step with split winds, when zm_conv_tend_hist_fields attached
+// them: the environment wind for i <= ncol (zm_conv.F90:2429-2443; state%u / state%v, component 1 = u), 0 in the
+// padding columns.  k_momtran_t then overwrites the convective columns.  (pguall / pgdall start as zero: k_zero_fill.)
+__global__ void k_icw_init(int nchunks, const int* ncol, const double* u, const double* v, double* icwu, double* icwd) {
+  const int pcols = P.pcols, pver = P.pver;
+  const size_t n2 = (size_t)nchunks * pcols * pver;
+  for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < 2 * n2; e += (size_t)gridDim.x * blockDim.x) {
+    // e -> (c, m, k, i) of the (pcols,pver,2) arrays
+    const size_t i = e % pcols, r = e / pcols;
+    const size_t m = (r / pver) & 1, c = r / ((size_t)pver * 2), src = (c * pver + r % pver) * pcols + i;
+    const double w = ((int)i < ncol[c]) ? (m ? v[src] : u[src]) : 0.0;
+    icwu[e] = w; icwd[e] = w;
+  }
 }
 
 // Warp per gathered (convective) column, lane = level.  Everything that is independent from level to level

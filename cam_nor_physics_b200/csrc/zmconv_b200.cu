@@ -128,6 +128,26 @@ struct Tran1Fields { int pcnst = 0; const double* q = nullptr; const double* fra
 thread_local Tran1Fields tls_tran1;
 struct Tran1Dev { int ncnst, nactive; const int* active; const int* is_dry; bool any_dry;
                   const double* q; const double* fracis; double* dqdt; };
+// zm_conv_tend's history fields (zm_conv_intr.F90:676-857), attached per call with zm_conv_tend_hist_fields (host or
+// device pointers like zm_org_fields): the outputs of zm_convr, zm_conv_evap and momtran inside the step.  NULL =
+// not materialised.  pguall, pgdall, icwu, icwd are (pcols,pver,2) per chunk, everything else (pcols,pver).
+enum { H_HEAT, H_QTND, H_EURT, H_DIF, H_DNLF, H_DNIF,                  // zm_convr
+       H_TEND_S, H_SNWPRD, H_SNWEVMLT, H_NTPRPRD, H_NTSNPRD,          // zm_conv_evap
+       H_SETEN, H_PGUALL, H_PGDALL, H_ICWU, H_ICWD,                   // momtran
+       H_N };
+struct HistFields {
+  double* p[H_N] = {};                   // argument order of zm_conv_tend_hist_fields
+  static bool is3d(int j) { return j >= H_PGUALL; }
+  bool any() const { for (int j = 0; j < H_N; ++j) if (p[j]) return true; return false; }
+  // the sub-batch that starts at chunk c0 (s2 = pcols*pver)
+  HistFields slice(size_t c0, size_t s2) const {
+    HistFields h = *this;
+    for (int j = 0; j < H_N; ++j)
+      if (h.p[j]) h.p[j] += c0 * s2 * (is3d(j) ? 2 : 1);
+    return h;
+  }
+};
+thread_local HistFields tls_hist;
 thread_local Workspace tls_work;     // kernel work arrays
 thread_local Workspace tls_stage;    // device staging of user arrays for the host-pointer API
 thread_local Workspace tls_stage2;   // staging for zm_conv_tend_2_batch
@@ -459,12 +479,21 @@ int convr_launch(Workspace& ws, cudaStream_t s, const ConvrIn& in, const ConvrOu
   FillList fl{};
   {
     const size_t n2 = ncolpad * pver, n2p = ncolpad * (pver + 1);
-    auto add = [&](double* p, size_t n) { if (p && fl.cnt < ZM_FILL_MAX) { fl.p[fl.cnt] = p; fl.n[fl.cnt] = n; ++fl.cnt; } };
+    bool full = false;
+    auto add = [&](double* p, size_t n) {
+      if (!p) return;
+      if (fl.cnt == ZM_FILL_MAX) { full = true; return; }
+      fl.p[fl.cnt] = p; fl.n[fl.cnt] = n; ++fl.cnt;
+    };
     for (double* p : {o.qtnd, o.heat, o.cme, o.dlf, o.zdu, o.rprd, o.mu, o.md, o.du, o.eu, o.ed, o.dp, o.ql}) add(p, n2);
-    // eurt, dif, dnlf, dnif are outputs of zm_convr that zm_conv_tend does not pass on: NULL inside the fused sequence
+    // eurt, dif, dnlf, dnif: NULL inside the fused sequence unless zm_conv_tend_hist_fields attached them
     for (double* p : {o.eurt, o.dif, o.dnlf, o.dnif}) add(p, n2);
     add(o.mcon, n2p); add(o.pflx, n2p);
     if (extra_fill) for (int a = 0; a < extra_fill->cnt; ++a) add(extra_fill->p[a], extra_fill->n[a]);
+    if (full) {      // an array left out would return stale arena contents
+      tls_err = "internal: zero-fill list of zm_convr exceeds ZM_FILL_MAX";
+      return -100;
+    }
   }
   // the work ordering of the first CAPE pass (latency-bound, inputs only) runs on the side stream beside the fill
   // (bandwidth-bound); ZM_ORDER_SIDE=0 keeps both on this stream
@@ -598,8 +627,9 @@ struct Stager {      // host-pointer API: bump-allocate device copies of user ar
 
 int evap_launch(cudaStream_t s, const EvapArgs& a) {
   const int ncolpad = a.nchunks * g_params.pcols;
-  if (a.heat) k_conv_evap<true><<<(ncolpad + 127) / 128, 128, 0, s>>>(a);
-  else        k_conv_evap<false><<<(ncolpad + 127) / 128, 128, 0, s>>>(a);
+  if (a.heat && a.tend_s) k_conv_evap<true, true><<<(ncolpad + 127) / 128, 128, 0, s>>>(a);
+  else if (a.heat)        k_conv_evap<true><<<(ncolpad + 127) / 128, 128, 0, s>>>(a);
+  else                    k_conv_evap<false><<<(ncolpad + 127) / 128, 128, 0, s>>>(a);
   ++tls_launches;
   CK(cudaGetLastError());
   return 0;
@@ -1375,23 +1405,35 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
                            double* md, double* du, double* eu, double* ed, double* dp, double* dsubcld,
                            int* jt, int* maxg, int* ideep, int* lengath, double* cape, void* stream,
                            const TendHooks* hooks, const double* org = nullptr, double* orgt = nullptr,
-                           double* org2d = nullptr, const Tran1Dev* tr1 = nullptr) {
+                           double* org2d = nullptr, const Tran1Dev* tr1 = nullptr, const HistFields* hist = nullptr) {
   NEED_INIT();
   if (nchunks <= 0) return 0;
   const size_t pc = g_params.pcols, L = g_params.pver, nc = (size_t)nchunks * pc;
   const size_t n2 = nc * L, n2p = nc * (L + 1);
-  if (ws.ensure(convr_work_bytes(nc, (int)L) + 19 * al(n2, 8) + 6 * al(2 * n2, 8) + chunk_bounds_bytes(nchunks, (int)nc) + 8192))
+  const HistFields H = hist ? *hist : HistFields{};
+  if (ws.ensure(convr_work_bytes(nc, (int)L) + 19 * al(n2, 8) + 6 * al(2 * n2, 8) + chunk_bounds_bytes(nchunks, (int)nc) + 8192 +
+                (H.any() ? 4 * al(n2, 8) + 4 * al(2 * n2, 8) : 0)))
     return -100;
   cudaStream_t s = (cudaStream_t)stream;      // NULL = the CUDA default stream
-  // eurt, dif, dnlf, dnif of zm_convr (history diagnostics EURT / DIFZM and the microphysics number tendencies) are
-  // not among zm_conv_tend's outputs: not materialised here (all four NULL together)
-  double *heat = ws.take<double>(n2), *qtnd = ws.take<double>(n2), *eurt = nullptr, *dif = nullptr, *dnlf = nullptr,
-         *dnif = nullptr, *t1 = ws.take<double>(n2), *q1 = ws.take<double>(n2), *ev_s = ws.take<double>(n2),
-         *ev_q_scratch = ws.take<double>(n2), *snwprd = nullptr, *snwevmlt = nullptr, *ntprprd = nullptr, *ntsnprd = nullptr,
-         *seten = ws.take<double>(n2);     // zm_conv_evap's four history diagnostics are not materialised either
-  // momtran's pguall / pgdall / icwu / icwd are history diagnostics the step does not return: not materialised
+  // History fields (zm_conv_tend_hist_fields): an attached field is written where it is computed; heat, qtnd, tend_s
+  // and seten are needed anyway and live in scratch otherwise.  eurt, dif, dnlf, dnif of zm_convr, zm_conv_evap's four
+  // diagnostics and momtran's pguall / pgdall / icwu / icwd are not materialised unless attached; the kernels store
+  // the last two groups as a whole, so an attached group gets scratch for its unattached members.
+  auto own = [&](int j, size_t n) { return H.p[j] ? H.p[j] : ws.take<double>(n); };
+  const bool hist_evap = H.p[H_TEND_S] || H.p[H_SNWPRD] || H.p[H_SNWEVMLT] || H.p[H_NTPRPRD] || H.p[H_NTSNPRD];
+  const bool hist_mom = H.p[H_PGUALL] || H.p[H_PGDALL] || H.p[H_ICWU] || H.p[H_ICWD];
+  double *heat = own(H_HEAT, n2), *qtnd = own(H_QTND, n2), *eurt = H.p[H_EURT], *dif = H.p[H_DIF],
+         *dnlf = H.p[H_DNLF], *dnif = H.p[H_DNIF], *t1 = ws.take<double>(n2), *q1 = ws.take<double>(n2),
+         *ev_s = own(H_TEND_S, n2), *ev_q_scratch = ws.take<double>(n2), *snwprd = nullptr, *snwevmlt = nullptr,
+         *ntprprd = nullptr, *ntsnprd = nullptr, *seten = own(H_SETEN, n2);
   double *winds = ws.take<double>(2 * n2), *wtend = ws.take<double>(2 * n2), *pgu = nullptr, *pgd = nullptr,
          *icwu = nullptr, *icwd = nullptr;
+  if (hist_evap) {
+    snwprd = own(H_SNWPRD, n2); snwevmlt = own(H_SNWEVMLT, n2); ntprprd = own(H_NTPRPRD, n2); ntsnprd = own(H_NTSNPRD, n2);
+  }
+  if (hist_mom) {
+    pgu = own(H_PGUALL, 2 * n2); pgd = own(H_PGDALL, 2 * n2); icwu = own(H_ICWU, 2 * n2); icwd = own(H_ICWD, 2 * n2);
+  }
   // zm_conv_evap's tend_q IS evapcdp (zm_conv_intr.F90:764-769 passes ptend_loc%q(:,:,1), :796 outputs it): written in place
   double* ev_q = evapcdp ? evapcdp : ev_q_scratch;
   const bool do_mom = !g_params.cam3;          // zm_conv_intr.F90:808: momentum transport is non-cam3 physics
@@ -1407,8 +1449,16 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
   // split winds: ptend_u / ptend_v / seten are zero outside the convective columns momtran writes -- filled with
   // zm_convr's own outputs at the start of the step
   FillList xf{};
-  if (split) { xf.p[0] = ptend_u; xf.p[1] = ptend_v; xf.p[2] = seten; xf.n[0] = xf.n[1] = xf.n[2] = n2; xf.cnt = 3; }
-  int rc = convr_launch(ws, s, in, o, false, orgt, org2d, split ? &xf : nullptr);
+  auto xadd = [&](double* p, size_t n) { xf.p[xf.cnt] = p; xf.n[xf.cnt] = n; ++xf.cnt; };
+  if (split) { xadd(ptend_u, n2); xadd(ptend_v, n2); xadd(seten, n2); }
+  // momtran's diagnostics: pguall / pgdall are zero outside the convective columns; with cam3 (no momtran,
+  // zm_conv_intr.F90:808) all five momtran fields return 0
+  if (hist_mom) { xadd(pgu, 2 * n2); xadd(pgd, 2 * n2); }
+  if (!do_mom) {
+    if (H.p[H_SETEN]) xadd(seten, n2);
+    if (hist_mom) { xadd(icwu, 2 * n2); xadd(icwd, 2 * n2); }
+  }
+  int rc = convr_launch(ws, s, in, o, false, orgt, org2d, xf.cnt ? &xf : nullptr);
   if (rc) return rc;
   if (hooks) {
     CK(cudaEventRecord(hooks->convr_done, s));            // zm_convr outputs are final from here on
@@ -1426,8 +1476,9 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
   // left for the end of the step is ptend_s += seten.  ZM_TEND_FUSE_EVAP=0: separate state update and final sum.
   const bool fuse_evap = split && o.mcon_kgm2s && (((uintptr_t)ptend_s) & 15) == 0 &&
                          !(getenv("ZM_TEND_FUSE_EVAP") && atoi(getenv("ZM_TEND_FUSE_EVAP")) == 0);
-  if (fuse_evap) {
-    ea.t = t; ea.q = q; ea.heat = heat; ea.qtnd = qtnd; ea.ps = ptend_s; ea.pq = ptend_q; ea.tend_s = nullptr;
+  if (fuse_evap) {     // tend_s stays: k_conv_evap<true, true> also stores it and the four snow diagnostics
+    ea.t = t; ea.q = q; ea.heat = heat; ea.qtnd = qtnd; ea.ps = ptend_s; ea.pq = ptend_q;
+    if (!hist_evap) ea.tend_s = nullptr;
   }
   if (fork) {
     if (ws.ensure_side()) return -100;
@@ -1476,6 +1527,7 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
     ma.dqdt = wtend; ma.pguall = pgu; ma.pgdall = pgd; ma.icwu = icwu; ma.icwd = icwd; ma.seten = seten;
     ma.dt = ztodt;
     if (split) { ma.q_u = u; ma.q_v = v; ma.dq_u = ptend_u; ma.dq_v = ptend_v; }
+    if (hist_mom) { k_icw_init<<<1184, 256, 0, s>>>(nchunks, ncol, u, v, icwu, icwd); ++tls_launches; }
     rc = momtran_launch(ws, s, ma, false, &cb);
     if (rc) return rc;
   }
@@ -1537,6 +1589,8 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
   tp.dev_nb = 0;
   const OrgFields of = tls_org; tls_org = OrgFields{};       // one-shot
   const Tran1Fields tf = tls_tran1; tls_tran1 = Tran1Fields{};   // one-shot
+  const HistFields hf = tls_hist; tls_hist = HistFields{};       // one-shot
+  const HistFields* hfp = hf.any() ? &hf : nullptr;
   Tran1Dev td{};
   const Tran1Dev* tdp = nullptr;
   if (tf.pcnst > 0) {
@@ -1550,7 +1604,7 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
       return conv_tend_impl(ws, nchunks, ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, tpert, landfrac,
                             cld, ztodt, ptend_s, ptend_q, ptend_u, ptend_v, mcon, cme, pflx, zdu, rliq, rice, jctop,
                             jcbot, prec, snow, ql, rprd, evapcdp, flxprec, flxsnow, dlf, mu, md, du, eu, ed, dp,
-                            dsubcld, jt, maxg, ideep, lengath, cape, on, nullptr, of.org, of.orgt, of.org2d, tdp);
+                            dsubcld, jt, maxg, ideep, lengath, cape, on, nullptr, of.org, of.orgt, of.org2d, tdp, hfp);
     };
     static const bool use_graph = !(getenv("ZM_DEV_GRAPH") && atoi(getenv("ZM_DEV_GRAPH")) == 0);
     if (g_profile || !use_graph) { tls_graph.clear(); return direct(tls_work, stream); }
@@ -1562,8 +1616,10 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
         evapcdp, flxprec, flxsnow, dlf, mu, md, du, eu, ed, dp, dsubcld, jt, maxg, ideep, lengath, cape,
         of.org, of.orgt, of.org2d, ztbits, (const void*)(size_t)nchunks, (const void*)(size_t)g_epoch,
         tf.q, tf.fracis, tf.ptend_q, (const void*)(size_t)tf.pcnst, (const void*)tls_tmeta1.d,
-        (const void*)(size_t)(tdp ? tls_tmeta1.version : 0),
-        (const void*)ws.dbuf, (const void*)ws.dcap};
+        (const void*)(size_t)(tdp ? tls_tmeta1.version : 0)};
+    // attached history fields: a replay must write where this call asked, and attaching or detaching recaptures
+    key.insert(key.end(), hf.p, hf.p + H_N);
+    key.push_back((const void*)ws.dbuf); key.push_back((const void*)ws.dcap);
     cudaStream_t s = (cudaStream_t)stream;
     if (key == G.key) {
       if (!G.exec) {                                   // second identical call: capture on the library's own stream
@@ -1607,6 +1663,7 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
       const size_t o3 = (size_t)c0 * s2 * td.ncnst;
       tb.q = td.q + o3; tb.fracis = td.fracis + o3; tb.dqdt = td.dqdt + o3;
     }
+    const HistFields hb = hf.slice(c0, s2);
 #define O2(x)  ((x) + (size_t)c0 * s2)
 #define O2P(x) ((x) + (size_t)c0 * s2p)
 #define O1(x)  ((x) + (size_t)c0 * s1)
@@ -1617,7 +1674,7 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
                             O2P(flxprec), O2P(flxsnow), O2(dlf), O2(mu), O2(md), O2(du), O2(eu), O2(ed), O2(dp),
                             O1(dsubcld), O1(jt), O1(maxg), O1(ideep), lengath + c0, O1(cape), (void*)ws.stream, nullptr,
                             of.org ? O2(of.org) : nullptr, of.orgt ? O2(of.orgt) : nullptr,
-                            of.org2d ? O2(of.org2d) : nullptr, tdp ? &tb : nullptr);
+                            of.org2d ? O2(of.org2d) : nullptr, tdp ? &tb : nullptr, hfp ? &hb : nullptr);
 #undef O2
 #undef O2P
 #undef O1
@@ -1645,8 +1702,12 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
   const size_t n2 = nc * L, n2p = nc * (L + 1);
   Workspace& st = tls_stage;
   tls_mirror = PbufMirror{};                 // whatever happens below, the previous step's mirror is gone
+  const HistFields hf = tls_hist; tls_hist = HistFields{};       // one-shot
+  size_t hist_bytes = 0;                     // staging of the attached history fields
+  for (int j = 0; j < H_N; ++j)
+    if (hf.p[j]) hist_bytes += al(HistFields::is3d(j) ? 2 * n2 : n2, 8);
   if (st.ensure(al(nchunks, 4) + 27 * al(n2, 8) + 6 * al(n2p, 8) + 14 * al(nc, 8) + 4 * al(nc, 4) + 8192 +
-                al(nc * (20 * L + 4), 8) + al((size_t)nchunks + 16, 4)))
+                al(nc * (20 * L + 4), 8) + al((size_t)nchunks + 16, 4) + hist_bytes))
     return -100;
   Workspace& mw = tls_mirror_ws;
   if (mw.ensure(6 * al(n2, 8) + al(nc, 8) + 3 * al(nc, 4) + al(nchunks, 4) + 4096)) return -100;
@@ -1726,6 +1787,12 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
     }
     d_org = DIN(of.org, s2); d_org2d = DOUTE(of.org2d, s2); d_orgt = DOUTF(of.orgt, s2);
   }
+  // history fields travel whole, also under ZM_TEND_RETURN=sparse: zm_convr's as soon as the plume kernel is done,
+  // zm_conv_evap's and momtran's at the end of the sub-batch
+  HistFields dh;
+  for (int j = 0; j < H_N; ++j)
+    if (hf.p[j]) dh.p[j] = (double*)dev(hf.p[j], HistFields::is3d(j) ? 2 * s2 : s2, 8, j <= H_DNIF ? 2 : 3);
+  const bool hist_on = hf.any();
 #undef DIN
 #undef DLATE
 #undef DOUTE
@@ -1858,6 +1925,7 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
       const size_t o3 = (size_t)c0 * s2 * td.ncnst;
       tb.q = td.q + o3; tb.fracis = td.fracis + o3; tb.dqdt = td.dqdt + o3;
     }
+    const HistFields hb = dh.slice(c0, s2);
 #define O2(x)  ((x) + (size_t)c0 * s2)
 #define O2P(x) ((x) + (size_t)c0 * s2p)
 #define O1(x)  ((x) + (size_t)c0 * s1)
@@ -1868,7 +1936,8 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
                         O2(d_rprd), O2(d_evap), O2P(d_fp), O2P(d_fs), O2(d_dlf), O2(d_mu), O2(d_md), O2(d_du),
                         O2(d_eu), O2(d_ed), O2(d_dp), O1(d_dsub), O1(d_jt), O1(d_maxg), O1(d_ideep), d_len + c0,
                         O1(d_cape), (void*)ws.stream, &hooks, d_org ? O2(d_org) : nullptr,
-                        d_orgt ? O2(d_orgt) : nullptr, d_org2d ? O2(d_org2d) : nullptr, tdp ? &tb : nullptr);
+                        d_orgt ? O2(d_orgt) : nullptr, d_org2d ? O2(d_org2d) : nullptr, tdp ? &tb : nullptr,
+                        hist_on ? &hb : nullptr);
 #undef O2
 #undef O2P
 #undef O1
@@ -2023,6 +2092,20 @@ int zm_tend_transfer_bytes(long long* h2d, long long* d2h) {
 // for *_dev).  Replaces the pointer dummies org/orgt/org2d of zm_convr (zm_conv.F90:242, 421-423).
 int zm_org_fields(const double* org, double* orgt, double* org2d) {
   tls_org = OrgFields{org, orgt, org2d};
+  return 0;
+}
+
+// zm_conv_tend's history fields (zm_conv_intr.F90:676-857) for the NEXT zm_conv_tend_batch[_dev] call of this
+// thread; any pointer may be NULL (not materialised, not copied)
+int zm_conv_tend_hist_fields(double* heat, double* qtnd, double* eurt, double* dif, double* dnlf, double* dnif,
+                             double* tend_s, double* tend_s_snwprd, double* tend_s_snwevmlt,
+                             double* ntprprd, double* ntsnprd,
+                             double* seten, double* pguall, double* pgdall, double* icwu, double* icwd) {
+  HistFields h;
+  double* const a[H_N] = {heat, qtnd, eurt, dif, dnlf, dnif, tend_s, tend_s_snwprd, tend_s_snwevmlt, ntprprd, ntsnprd,
+                          seten, pguall, pgdall, icwu, icwd};
+  std::copy(a, a + H_N, h.p);
+  tls_hist = h;
   return 0;
 }
 

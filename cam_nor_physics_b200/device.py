@@ -15,10 +15,12 @@ def _ptr(t: torch.Tensor):
 class DeviceTend:
     """Holds one rank's chunk set on the GPU and runs zm_conv_tend on it."""
 
-    def __init__(self, ch, device="cuda", ncnst=0):
+    def __init__(self, ch, device="cuda", ncnst=0, hist=None):
         """ncnst > 0 adds the constituent arrays of BASELINE config 4 (convtran over the tracer set as zm_conv_intr
         runs it from tphysbc): constituents 2,3 (cloud liquid / ice) are transported by convtran1 inside zm_conv_tend
-        (zm_conv_intr.F90:865-880), 4..ncnst by convtran2 in zm_conv_tend_2 (:955-1028), every third of those 'dry'."""
+        (zm_conv_intr.F90:865-880), 4..ncnst by convtran2 in zm_conv_tend_2 (:955-1028), every third of those 'dry'.
+        hist = True or an iterable of zm_conv.HIST_FIELDS names: every step also writes those history fields into the
+        device tensors self.hist[name] (zm_conv_tend_hist_fields)."""
         p = Z._params
         if p is None:
             raise Z.ZmError("zm_init has not been called")
@@ -44,6 +46,7 @@ class DeviceTend:
         for k in Z.TEND_OUT_INT:
             self.out[k] = torch.zeros((nch, pc), **i32)
         self.out["lengath"] = torch.zeros(nch, **i32)
+        self.hist = {k: torch.zeros(Z.hist_shape(k, nch, L, pc), **f64) for k in Z.hist_names(hist)}
         self.in_bytes = sum(v.numel() * v.element_size() for v in self.host_in.values()) + self.host_ncol.numel() * 4
         self.ncnst = int(ncnst)
         if self.ncnst:
@@ -71,6 +74,8 @@ class DeviceTend:
             Z.lib().zm_convtran1_fields(C.c_int(self.ncnst), self.do1.ctypes.data_as(Z.c_ip),
                                         self.dry.ctypes.data_as(Z.c_ip), _ptr(self.tr["q"]), _ptr(self.tr["fracis"]),
                                         _ptr(self.ptend_qc))
+        if self.hist:
+            Z.lib().zm_conv_tend_hist_fields(*[(_ptr(self.hist[k]) if k in self.hist else None) for k in Z.HIST_FIELDS])
         args = [C.c_int(self.nch), _ptr(self.ncol)] + [_ptr(self.inp[k]) for k in Z.TEND_IN_ORDER]
         args += [C.c_double(self.ztodt)] + [_ptr(self.out[k]) for k in Z.TEND_ARG_ORDER] + [C.c_void_p(s)]
         rc = Z.lib().zm_conv_tend_batch_dev(*args)

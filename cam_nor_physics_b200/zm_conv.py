@@ -78,7 +78,7 @@ EXPORTS = [
     "zm_math_eval_dev", "zm_math_eval_host", "zm_thermo_eval_dev", "zm_fp64_peak_flops",
     "zm_set_profiling", "zm_get_kernel_times", "zm_launch_count",
     "zm_convtran1_fields", "zm_conv_tend_diag_batch", "zm_conv_tend_diag_batch_dev", "zm_get_timers",
-    "zm_conv_tend_2_batch_dev", "zm_tend_transfer_bytes", "zm_build_info",
+    "zm_conv_tend_2_batch_dev", "zm_tend_transfer_bytes", "zm_build_info", "zm_conv_tend_hist_fields",
 ]
 
 
@@ -258,6 +258,28 @@ TEND_ARG_ORDER = ["ptend_s", "ptend_q", "ptend_u", "ptend_v", "mcon", "cme", "pf
                   "mu", "md", "du", "eu", "ed", "dp", "dsubcld", "jt", "maxg", "ideep", "lengath", "cape"]
 TEND_IN_ORDER = ["t", "q", "u", "v", "pmid", "pint", "pdel", "zm", "zi", "phis", "pblh", "tpert",
                  "landfrac", "cld"]
+# zm_conv_tend's history fields, in the argument order of zm_conv_tend_hist_fields: zm_convr's, zm_conv_evap's and
+# momtran's own outputs inside the step (zm_conv_intr.F90:676-857)
+HIST_FIELDS = ["heat", "qtnd", "eurt", "dif", "dnlf", "dnif", "tend_s", "tend_s_snwprd", "tend_s_snwevmlt",
+               "ntprprd", "ntsnprd", "seten", "pguall", "pgdall", "icwu", "icwd"]
+HIST_3D = ("pguall", "pgdall", "icwu", "icwd")          # (pcols,pver,2) per chunk: component 1 = u, 2 = v
+
+
+def hist_names(hist) -> list:
+    """The history fields selected by `hist`: True = all, False/None = none, else an iterable of names."""
+    if hist is None or hist is False:
+        return []
+    if hist is True:
+        return list(HIST_FIELDS)
+    names = list(hist)
+    bad = [k for k in names if k not in HIST_FIELDS]
+    if bad:
+        raise ZmError(f"unknown history fields {bad}; known: {HIST_FIELDS}")
+    return [k for k in HIST_FIELDS if k in names]
+
+
+def hist_shape(name: str, nch: int, L: int, pc: int) -> tuple:
+    return (nch, 2, L, pc) if name in HIST_3D else (nch, L, pc)
 
 
 def zm_conv_tend_2(doconvtran, q, pdeldry, fracis, ztodt, cnst_is_dry, ptend_q=None):
@@ -273,13 +295,16 @@ def zm_conv_tend_2(doconvtran, q, pdeldry, fracis, ztodt, cnst_is_dry, ptend_q=N
 
 
 def zm_conv_tend(ncol, state: dict, ztodt: float, out: dict | None = None, keep_pbuf_on_device: bool = False,
-                 convtran1: dict | None = None):
+                 convtran1: dict | None = None, hist=None):
     """zm_conv_tend (zm_conv_intr.F90:390) over host arrays: zm_convr -> physics_update ->
     zm_conv_evap -> momtran [-> convtran1] with everything resident on the device in between.
     `state` holds t,q,u,v,pmid,pint,pdel,zm,zi,phis,pblh,tpert,landfrac,cld in chunk layout.
     convtran1 = dict(doconvtran=cnst_is_convtran1 flags [pcnst], cnst_is_dry=[pcnst] or None,
     q=state%q [nchunks,pcnst,pver,pcols], fracis=same shape[, ptend_q=initial ptend_all%q]) adds the transport of
-    cloud liquid / ice (zm_conv_intr.F90:865-880); the result comes back as out["ptend_qc"]."""
+    cloud liquid / ice (zm_conv_intr.F90:865-880); the result comes back as out["ptend_qc"].
+    hist = True (all) or an iterable of HIST_FIELDS names returns those history fields in `out` under their names
+    (zm_conv_tend_hist_fields): [nchunks, pver, pcols], or [nchunks, 2, pver, pcols] for pguall, pgdall, icwu, icwd.
+    Arrays already in `out` under those names are written in place."""
     pc, L = _grid()
     ncol = _i(ncol)
     nch = ncol.shape[0]
@@ -309,6 +334,14 @@ def zm_conv_tend(ncol, state: dict, ztodt: float, out: dict | None = None, keep_
         keep = (q3, f3)                                                    # noqa: F841 (alive during the call)
         lib().zm_convtran1_fields(C.c_int(pcnst), _ip(_i(convtran1["doconvtran"])),
                                   _ip(_i(dry)) if dry is not None else None, _dp(q3), _dp(f3), _dp(out["ptend_qc"]))
+    names = hist_names(hist)
+    for k in names:
+        shape = hist_shape(k, nch, L, pc)
+        if k not in out:
+            out[k] = np.zeros(shape)
+        a = out[k]
+        if a.shape != shape or a.dtype != np.float64 or not a.flags.c_contiguous:
+            raise ZmError(f"out[{k!r}] must be a C-contiguous float64 array of shape {shape}")
     mirror_only = {"mu", "md", "du", "eu", "ed", "dp", "dsubcld", "jt", "maxg"} if keep_pbuf_on_device else set()
     for k in TEND_ARG_ORDER:
         a = out[k]
@@ -316,6 +349,8 @@ def zm_conv_tend(ncol, state: dict, ztodt: float, out: dict | None = None, keep_
             args.append(None)       # stays in the device mirror for zm_conv_tend_2 (no D2H)
         else:
             args.append(_ip(a) if a.dtype == np.int32 else _dp(a))
+    if names:       # attached last: nothing above may fail and leave the attachment to a later call
+        lib().zm_conv_tend_hist_fields(*[(_dp(out[k]) if k in names else None) for k in HIST_FIELDS])
     rc = lib().zm_conv_tend_batch(*args)
     _check(rc, "zm_conv_tend")
     return out

@@ -31,6 +31,7 @@ module zm_conv_intr_batched
   use cam_logfile,     only: iulog
   use cam_history,     only: outfld
   use perf_mod,        only: t_startf, t_stopf
+  use phys_control,    only: cam_physpkg_is
 
   implicit none
   save
@@ -56,6 +57,15 @@ module zm_conv_intr_batched
   real(c_double), allocatable, dimension(:,:,:,:) :: q3_b, fracis_b, ptend_q3_b                            ! (pcols,pver,pcnst,nchunks)
   real(c_double), allocatable, dimension(:,:,:) :: pdeldry_b
   integer(c_int) :: doconvtran1(pcnst), doconvtran2(pcnst), cnst_is_dry(pcnst)
+  ! history fields of zm_conv_tend (zm_conv_intr.F90:676-857): zm_convr's, zm_conv_evap's and momtran's own outputs,
+  ! attached with zm_conv_tend_hist_fields; the momtran arrays are (pcols,pver,2,nchunks), component 1 = u, 2 = v
+  real(c_double), allocatable, dimension(:,:,:) :: heat_b, qtnd_b, eurt_b, dif_b, dnlf_b, dnif_b, tend_s_b, &
+                                                    snwprd_b, snwevmlt_b, ntprprd_b, ntsnprd_b, seten_b
+  real(c_double), allocatable, dimension(:,:,:,:) :: pguall_b, pgdall_b, icwu_b, icwd_b
+  ! zmconv_org: the organisation tracer state%q(:,:,ixorg) in, its tendency and column mean out (zm_conv.F90:421-423)
+  logical :: org_on = .false.
+  integer :: ixorg = -1
+  real(c_double), allocatable, dimension(:,:,:) :: org_b, orgt_b, org2d_b
 
   interface
      integer(c_int) function zm_conv_tend_batch(nchunks, ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, &
@@ -104,6 +114,14 @@ module zm_conv_intr_batched
        real(c_double), intent(out) :: orgt(*), org2d(*)
      end function zm_org_fields
 
+     integer(c_int) function zm_conv_tend_hist_fields(heat, qtnd, eurt, dif, dnlf, dnif, tend_s, tend_s_snwprd, &
+          tend_s_snwevmlt, ntprprd, ntsnprd, seten, pguall, pgdall, icwu, icwd) bind(C, name='zm_conv_tend_hist_fields')
+       import :: c_int, c_double
+       real(c_double), intent(out) :: heat(*), qtnd(*), eurt(*), dif(*), dnlf(*), dnif(*), tend_s(*), &
+                                      tend_s_snwprd(*), tend_s_snwevmlt(*), ntprprd(*), ntsnprd(*), seten(*), &
+                                      pguall(*), pgdall(*), icwu(*), icwd(*)
+     end function zm_conv_tend_hist_fields
+
      integer(c_int) function zm_conv_tend_diag_batch(nchunks, ncol, ps, pmid, mu, md, jt, maxg, ideep, lengath, &
           freqzm, mu_out, md_out, pcont, pconb) bind(C, name='zm_conv_tend_diag_batch')
        import :: c_int, c_double
@@ -136,9 +154,11 @@ module zm_conv_intr_batched
 contains
 
   !-------------------------------------------------------------------------------
-  subroutine zm_batch_init(nchunks)
-    ! once, after zm_conv_init (zm_convi -> zm_init is done by the shim's zm_convi, zm_conv_intr.F90:376-379)
+  subroutine zm_batch_init(nchunks, zmconv_org)
+    ! once, after zm_conv_init (zm_convi -> zm_init is done by the shim's zm_convi, zm_conv_intr.F90:376-379);
+    ! zmconv_org: the namelist switch zm_convi received (organisation tracer 'ZM_ORG')
     integer, intent(in) :: nchunks
+    logical, intent(in), optional :: zmconv_org
     integer :: m
     nchunks_b = nchunks
     allocate(ncol_b(nchunks), lengath_b(nchunks))
@@ -159,6 +179,18 @@ contains
     allocate(jt_b(pcols,nchunks), maxg_b(pcols,nchunks), ideep_b(pcols,nchunks))
     allocate(q3_b(pcols,pver,pcnst,nchunks), fracis_b(pcols,pver,pcnst,nchunks), ptend_q3_b(pcols,pver,pcnst,nchunks), &
              pdeldry_b(pcols,pver,nchunks))
+    allocate(heat_b(pcols,pver,nchunks), qtnd_b(pcols,pver,nchunks), eurt_b(pcols,pver,nchunks), dif_b(pcols,pver,nchunks), &
+             dnlf_b(pcols,pver,nchunks), dnif_b(pcols,pver,nchunks), tend_s_b(pcols,pver,nchunks), &
+             snwprd_b(pcols,pver,nchunks), snwevmlt_b(pcols,pver,nchunks), ntprprd_b(pcols,pver,nchunks), &
+             ntsnprd_b(pcols,pver,nchunks), seten_b(pcols,pver,nchunks))
+    allocate(pguall_b(pcols,pver,2,nchunks), pgdall_b(pcols,pver,2,nchunks), icwu_b(pcols,pver,2,nchunks), &
+             icwd_b(pcols,pver,2,nchunks))
+    org_on = .false.
+    if (present(zmconv_org)) org_on = zmconv_org
+    if (org_on) then
+       call cnst_get_ind('ZM_ORG', ixorg)
+       allocate(org_b(pcols,pver,nchunks), orgt_b(pcols,pver,nchunks), org2d_b(pcols,pver,nchunks))
+    end if
     ! constituent flags: lq(2:) = cnst_is_convtran1(2:) (zm_conv_intr.F90:868), cnst_is_convtran2 (:1009-1010),
     ! cnst_get_type_byind(m) == 'dry' (zm_conv.F90:2087)
     doconvtran1 = 0; doconvtran2 = 0; cnst_is_dry = 0
@@ -184,6 +216,7 @@ contains
     phis_b(:,ic) = state%phis;   ps_b(:,ic) = state%ps
     pblh_b(:,ic) = pblh; tpert_b(:,ic) = tpert; landfrac_b(:,ic) = landfrac; cld_b(:,:,ic) = cld
     q3_b(:,:,:,ic) = state%q;    fracis_b(:,:,:,ic) = fracis
+    if (org_on) org_b(:,:,ic) = state%q(:,:,ixorg)
   end subroutine zm_batch_gather
 
   !-------------------------------------------------------------------------------
@@ -194,6 +227,9 @@ contains
     call t_startf('zm_conv_tend_batch')
     ptend_q3_b = 0._r8                        ! physics_ptend_init(ptend_loc, ..., lq=lq) zeroes the flagged slices
     rc = zm_convtran1_fields(int(pcnst, c_int), doconvtran1, cnst_is_dry, q3_b, fracis_b, ptend_q3_b)
+    if (org_on) rc = zm_org_fields(org_b, orgt_b, org2d_b)       ! zm_conv_intr.F90:656-659
+    rc = zm_conv_tend_hist_fields(heat_b, qtnd_b, eurt_b, dif_b, dnlf_b, dnif_b, tend_s_b, snwprd_b, snwevmlt_b, &
+         ntprprd_b, ntsnprd_b, seten_b, pguall_b, pgdall_b, icwu_b, icwd_b)
     rc = zm_conv_tend_batch(int(nchunks_b, c_int), ncol_b, t_b, q_b, u_b, v_b, pmid_b, pint_b, pdel_b, zm_b, zi_b, &
          phis_b, pblh_b, tpert_b, landfrac_b, cld_b, real(ztodt, c_double), ptend_s_b, ptend_q_b, ptend_u_b, ptend_v_b, &
          mcon_b, cme_b, pflx_b, zdu_b, rliq_b, rice_b, jctop_b, jcbot_b, prec_b, snow_b, ql_b, rprd_b, evapcdp_b, &
@@ -208,10 +244,12 @@ contains
   !-------------------------------------------------------------------------------
   subroutine zm_batch_scatter(ic, lchnk, ptend_all, mcon, cme, pflx, zdu, rliq, rice, jctop, jcbot, &
                               prec, snow, ql, rprd, evapcdp, flxprec, flxsnow, dlf, mconzm, &
-                              mu, md, du, eu, ed, dp, dsubcld, jt, maxg, ideep, lengath)
-    ! loop 2 of the split chunk loop: chunk ic's outputs of zm_conv_tend -- ptend_all (lq(1), ls, lu, lv and the
-    ! convtran1 constituents), the dummy outputs (zm_conv_intr.F90:390-394), the pbuf fields (:591-621) -- and the
-    ! history output of :676-729, 796-857, 882-883
+                              mu, md, du, eu, ed, dp, dsubcld, jt, maxg, ideep, lengath, &
+                              difzm, dnlfzm, dnifzm, dp_cldliq, dp_cldice, org2d)
+    ! loop 2 of the split chunk loop: chunk ic's outputs of zm_conv_tend -- ptend_all (lq(1), ls, lu, lv, the
+    ! convtran1 constituents and, under zmconv_org, the organisation tracer), the dummy outputs
+    ! (zm_conv_intr.F90:390-394), the pbuf fields (:591-621; DIFZM, DNLFZM, DNIFZM, DP_CLDLIQ, DP_CLDICE and
+    ! ZM_ORG2D are optional) -- and the history output of :676-857, 882-883
     use physics_types, only: physics_ptend, physics_ptend_init
     integer, intent(in) :: ic, lchnk
     type(physics_ptend), intent(out) :: ptend_all
@@ -222,6 +260,8 @@ contains
     real(r8), intent(out) :: mu(pcols,pver), md(pcols,pver), du(pcols,pver), eu(pcols,pver), ed(pcols,pver), &
                              dp(pcols,pver), dsubcld(pcols)
     integer,  intent(out) :: jt(pcols), maxg(pcols), ideep(pcols), lengath
+    real(r8), intent(out), optional :: difzm(pcols,pver), dnlfzm(pcols,pver), dnifzm(pcols,pver), &
+                                       dp_cldliq(pcols,pver), dp_cldice(pcols,pver), org2d(pcols,pver)
     logical  :: lq(pcnst)
     real(r8) :: ftem(pcols,pver)
     integer  :: m, ncol, ixcldliq, ixcldice
@@ -230,14 +270,26 @@ contains
     do m = 2, pcnst
        lq(m) = doconvtran1(m) /= 0
     end do
+    if (org_on) lq(ixorg) = .true.
     call physics_ptend_init(ptend_all, pcols, 'zm_conv_tend', ls=.true., lu=.true., lv=.true., lq=lq)
     ptend_all%s(:ncol,:) = ptend_s_b(:ncol,:,ic)
     ptend_all%u(:ncol,:) = ptend_u_b(:ncol,:,ic)
     ptend_all%v(:ncol,:) = ptend_v_b(:ncol,:,ic)
     ptend_all%q(:ncol,:,1) = ptend_q_b(:ncol,:,ic)
     do m = 2, pcnst
-       if (lq(m)) ptend_all%q(:ncol,:,m) = ptend_q3_b(:ncol,:,m,ic)
+       if (lq(m) .and. doconvtran1(m) /= 0) ptend_all%q(:ncol,:,m) = ptend_q3_b(:ncol,:,m,ic)
     end do
+    if (org_on) then
+       ptend_all%q(:ncol,:,ixorg) = orgt_b(:ncol,:,ic)
+       if (present(org2d)) org2d = org2d_b(:,:,ic)
+    end if
+    ! pbuf fields filled from zm_convr's dif / dnlf / dnif; without zmconv_microp the convective cloud water and ice
+    ! are 0 (zm_conv_intr.F90:591-621)
+    if (present(difzm))     difzm  = dif_b(:,:,ic)
+    if (present(dnlfzm))    dnlfzm = dnlf_b(:,:,ic)
+    if (present(dnifzm))    dnifzm = dnif_b(:,:,ic)
+    if (present(dp_cldliq)) dp_cldliq = 0._r8
+    if (present(dp_cldice)) dp_cldice = 0._r8
     mcon = mcon_b(:,:,ic); cme = cme_b(:,:,ic); pflx = pflx_b(:,:,ic); zdu = zdu_b(:,:,ic)
     rliq = rliq_b(:,ic); rice = rice_b(:,ic); jctop = jctop_b(:,ic); jcbot = jcbot_b(:,ic)
     prec = prec_b(:,ic); snow = snow_b(:,ic); ql = ql_b(:,:,ic); rprd = rprd_b(:,:,ic); evapcdp = evapcdp_b(:,:,ic)
@@ -263,6 +315,39 @@ contains
     call cnst_get_ind('CLDICE', ixcldice)
     call outfld('ZMDICE ', ptend_q3_b(:,:,ixcldice,ic), pcols, lchnk)
     call outfld('ZMDLIQ ', ptend_q3_b(:,:,ixcldliq,ic), pcols, lchnk)
+    ! history of zm_convr's, zm_conv_evap's and momtran's intermediates (zm_conv_intr.F90:676-857).  The field names
+    ! and the /cpair of each follow the list of the fields this binding used to drop; confirm them against
+    ! zm_conv_intr.F90:285-330 (addfld) when the reference source is at hand -- the library returns the procedures'
+    ! own quantities, so only this file would change.
+    ftem = 0._r8
+    ftem(:ncol,:) = heat_b(:ncol,:,ic) / cpair
+    call outfld('ZMDT    ', ftem,                 pcols, lchnk)
+    call outfld('ZMDQ    ', qtnd_b(:,:,ic),       pcols, lchnk)
+    call outfld('EURT    ', eurt_b(:,:,ic),       pcols, lchnk)
+    call outfld('DIFZM   ', dif_b(:,:,ic),        pcols, lchnk)
+    ftem(:ncol,:) = tend_s_b(:ncol,:,ic) / cpair
+    call outfld('EVAPTZM ', ftem,                 pcols, lchnk)
+    call outfld('ZMEIHEAT', tend_s_b(:,:,ic),     pcols, lchnk)
+    ftem(:ncol,:) = snwprd_b(:ncol,:,ic) / cpair
+    call outfld('FZSNTZM ', ftem,                 pcols, lchnk)
+    ftem(:ncol,:) = snwevmlt_b(:ncol,:,ic) / cpair
+    call outfld('EVSNTZM ', ftem,                 pcols, lchnk)
+    call outfld('ZMNTPRPD', ntprprd_b(:,:,ic),    pcols, lchnk)
+    call outfld('ZMNTSNPD', ntsnprd_b(:,:,ic),    pcols, lchnk)
+    call outfld('ZMFLXPRC', flxprec,              pcols, lchnk)
+    call outfld('ZMFLXSNW', flxsnow,              pcols, lchnk)
+    if (.not. cam_physpkg_is('cam3')) then       ! momtran is skipped under cam3 (zm_conv_intr.F90:808)
+       ftem(:ncol,:) = seten_b(:ncol,:,ic) / cpair
+       call outfld('ZMMTT   ', ftem,                 pcols, lchnk)
+       call outfld('ZMUPGU  ', pguall_b(:,:,1,ic),   pcols, lchnk)
+       call outfld('ZMUPGD  ', pgdall_b(:,:,1,ic),   pcols, lchnk)
+       call outfld('ZMVPGU  ', pguall_b(:,:,2,ic),   pcols, lchnk)
+       call outfld('ZMVPGD  ', pgdall_b(:,:,2,ic),   pcols, lchnk)
+       call outfld('ZMICUU  ', icwu_b(:,:,1,ic),     pcols, lchnk)
+       call outfld('ZMICUD  ', icwd_b(:,:,1,ic),     pcols, lchnk)
+       call outfld('ZMICVU  ', icwu_b(:,:,2,ic),     pcols, lchnk)
+       call outfld('ZMICVD  ', icwd_b(:,:,2,ic),     pcols, lchnk)
+    end if
   end subroutine zm_batch_scatter
 
   !-------------------------------------------------------------------------------

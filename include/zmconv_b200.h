@@ -261,6 +261,22 @@ int zm_org_fields(const double* org, double* orgt, double* org2d);
 int zm_convtran1_fields(int pcnst, const int* doconvtran, const int* cnst_is_dry, const double* q,
                         const double* fracis, double* ptend_q);
 
+/* zm_conv_tend's history fields (zm_conv_intr.F90:676-857): attach for the NEXT zm_conv_tend_batch[_dev] call of the
+ * calling thread (host pointers for the host-pointer entry point, device pointers for _dev) the intermediate results
+ * the step otherwise keeps to itself -- zm_convr's heat (ptend_loc%s), qtnd (ptend_loc%q(:,:,1)), eurt, dif, dnlf, dnif;
+ * zm_conv_evap's (on state1) tend_s, tend_s_snwprd, tend_s_snwevmlt, ntprprd, ntsnprd; momtran's (on state1%u/v) seten,
+ * pguall, pgdall, icwu, icwd.  The procedures' own quantities: no /cpair, no unit change (ZMDT = heat/cpair etc. stay
+ * with the caller's outfld calls).  pguall, pgdall, icwu, icwd are (pcols,pver,2) per chunk, component 1 = u and 2 = v
+ * as momtran returns them; all others (pcols,pver) per chunk.  Any pointer may be NULL: that field is neither
+ * materialised nor copied.  Every element of an attached field is defined on return; padding columns (i > ncol) are 0,
+ * and with cam3 = 1 (no momtran, zm_conv_intr.F90:808) the five momtran fields are 0.  The regular outputs do not
+ * depend on what is attached.  The host-pointer variant copies the attached fields whole, also under
+ * ZM_TEND_RETURN=sparse, and zm_tend_transfer_bytes counts them. */
+int zm_conv_tend_hist_fields(double* heat, double* qtnd, double* eurt, double* dif, double* dnlf, double* dnif,
+                             double* tend_s, double* tend_s_snwprd, double* tend_s_snwevmlt,
+                             double* ntprprd, double* ntsnprd,
+                             double* seten, double* pguall, double* pgdall, double* icwu, double* icwd);
+
 /* zm_conv_tend's history diagnostics that involve arithmetic (zm_conv_intr.F90): freqzm (:685-688, 1 where the
  * column convects), mu_out / md_out (:575-576, 700-706: ungathered mass fluxes in kg/m2/s), pcont / pconb (:721-729:
  * pressure at cloud top / base, ps elsewhere).  ps, freqzm, pcont, pconb are (pcols); pmid, mu, md, mu_out, md_out
