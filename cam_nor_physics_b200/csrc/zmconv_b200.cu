@@ -218,6 +218,11 @@ struct SparseFields {
   int off[SF_N];             // offset of the field inside a record (doubles), -1 = absent
   int rec_len;               // doubles per record
 };
+// zm_conv_tend_batch_gathered: the same records go straight to the caller, who scatters them in its own chunk loop
+struct GatheredOut {
+  double* rec;               // caller's record buffer (capacity checked by the entry point)
+  bool pbuf;                 // the slot-indexed pbuf fields mu..dp are part of the records
+};
 // exclusive prefix of lengath over the chunks of a sub-batch (one block): base[c], total in base[nchunks]
 __global__ void k_lengath_scan(int nchunks, const int* lengath, int* base) {
   __shared__ int part[1024];
@@ -1686,18 +1691,19 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
   return 0;
 }
 
-int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const double* q, const double* u,
-                       const double* v, const double* pmid, const double* pint, const double* pdel,
-                       const double* zm, const double* zi, const double* phis, const double* pblh,
-                       const double* tpert, const double* landfrac, const double* cld, double ztodt,
-                       double* ptend_s, double* ptend_q, double* ptend_u, double* ptend_v, double* mcon,
-                       double* cme, double* pflx, double* zdu, double* rliq, double* rice, double* jctop,
-                       double* jcbot, double* prec, double* snow, double* ql, double* rprd, double* evapcdp,
-                       double* flxprec, double* flxsnow, double* dlf, double* mu, double* md, double* du,
-                       double* eu, double* ed, double* dp, double* dsubcld, int* jt, int* maxg, int* ideep,
-                       int* lengath, double* cape) {
-  NEED_INIT();
-  if (nchunks <= 0) return 0;
+// The host-pointer step behind zm_conv_tend_batch (g == NULL) and zm_conv_tend_batch_gathered (g != NULL: the
+// (pcols,pver[p]) outputs are packed into records that go to g->rec instead of being copied back whole; their
+// pointers are NULL here).
+static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const double* q, const double* u,
+                           const double* v, const double* pmid, const double* pint, const double* pdel,
+                           const double* zm, const double* zi, const double* phis, const double* pblh,
+                           const double* tpert, const double* landfrac, const double* cld, double ztodt,
+                           double* ptend_s, double* ptend_q, double* ptend_u, double* ptend_v, double* mcon,
+                           double* cme, double* pflx, double* zdu, double* rliq, double* rice, double* jctop,
+                           double* jcbot, double* prec, double* snow, double* ql, double* rprd, double* evapcdp,
+                           double* flxprec, double* flxsnow, double* dlf, double* mu, double* md, double* du,
+                           double* eu, double* ed, double* dp, double* dsubcld, int* jt, int* maxg, int* ideep,
+                           int* lengath, double* cape, const GatheredOut* g) {
   const size_t pc = g_params.pcols, L = g_params.pver, nc = (size_t)nchunks * pc;
   const size_t n2 = nc * L, n2p = nc * (L + 1);
   Workspace& st = tls_stage;
@@ -1734,9 +1740,9 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
   // parallel memset against 56 GB/s D2H) that costs more than it saves -- measured 11.7 against 8.2 ms per f09 step
   // (DESIGN.md section 5) -- so it is opt-in, for hosts with memory bandwidth to spare.
   // ZM_TEND_OUTPUTS_PREZEROED=1: the caller's arrays are all-zero on entry (as after physics_ptend_init), the
-  // zero-fill is skipped.
+  // zero-fill is skipped.  The gathered entry point ignores ZM_TEND_RETURN: its records are its return path.
   const char* ret_env = getenv("ZM_TEND_RETURN");
-  const bool sparse = ret_env && !strcmp(ret_env, "sparse");
+  const bool sparse = !g && ret_env && !strcmp(ret_env, "sparse");
   const bool prezeroed = getenv("ZM_TEND_OUTPUTS_PREZEROED") && atoi(getenv("ZM_TEND_OUTPUTS_PREZEROED")) != 0;
   double* sf_host[SF_N] = {};               // caller's arrays of the sparse fields (NULL: not wanted)
   double* sf_dev[SF_N] = {};
@@ -1767,8 +1773,9 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
   to_mirror = true;
   double *d_mu = SPE(SF_MU, mu, s2), *d_md = SPE(SF_MD, md, s2), *d_du = SPE(SF_DU, du, s2), *d_eu = SPE(SF_EU, eu, s2),
          *d_ed = SPE(SF_ED, ed, s2), *d_dp = SPE(SF_DP, dp, s2), *d_dsub = DOUTE(dsubcld, s1);
+  // gathered: lengath returns per sub-batch, ahead of that sub-batch's records (below), not with the batch's end
   int *d_jt = (int*)dev(jt, s1, 4, 2), *d_maxg = (int*)dev(maxg, s1, 4, 2), *d_ideep = (int*)dev(ideep, s1, 4, 2),
-      *d_len = (int*)dev(lengath, 1, 4, 2);
+      *d_len = (int*)dev(g ? nullptr : lengath, 1, 4, 2);
   to_mirror = false;
   const PbufMirror new_mirror{nchunks, d_mu, d_md, d_du, d_eu, d_ed, d_dp, d_dsub, d_jt, d_maxg, d_ideep, d_len};
   double *d_ps = SPF(SF_PS, ptend_s, s2), *d_pq = SPF(SF_PQ, ptend_q, s2), *d_pu = SPF(SF_PU, ptend_u, s2),
@@ -1800,17 +1807,19 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
 #undef SPE
 #undef SPF
   // sparse return: record layout (fields the caller asked for), device record buffer sized for the worst case so
-  // that a sub-batch's region does not depend on the counts of the others
+  // that a sub-batch's region does not depend on the counts of the others.  gathered: the 14 column-indexed fields,
+  // then the pbuf fields if asked for.
   int sf_off[SF_N], rec_len = 0;
   for (int qf = 0; qf < SF_N; ++qf) {
     const int nlev = (qf >= SF_MCON && qf <= SF_FS) ? (int)L + 1 : (int)L;
-    if (sparse && sf_host[qf]) { sf_off[qf] = rec_len; rec_len += nlev; } else sf_off[qf] = -1;
+    const bool packed = sparse ? sf_host[qf] != nullptr : (g && (qf < SF_MU || g->pbuf));
+    if (packed) { sf_off[qf] = rec_len; rec_len += nlev; } else sf_off[qf] = -1;
   }
   double* d_rec = nullptr; int* d_base = nullptr;
-  if (sparse && rec_len > 0) {
+  if (rec_len > 0) {
     d_rec = st.take<double>(nc * rec_len);
     d_base = st.take<int>((size_t)nchunks + TendPipe::MAXB + 1);
-    if (tp.ensure_pinned(0, 2 * (nc + nchunks + 2 * TendPipe::MAXB))) return -100;
+    if (sparse && tp.ensure_pinned(0, 2 * (nc + nchunks + 2 * TendPipe::MAXB))) return -100;
   }
   // convtran1 (zm_conv_intr.F90:865-880): only the slices of the transported constituents travel; on the device
   // they are stored compactly, (pcols,pver,nactive) per chunk
@@ -1943,7 +1952,7 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
 #undef O1
     if (rc) break;
     const double w_k = wall_ms();
-    if (pool) {         // the convective columns' records of this sub-batch
+    if (rec_len > 0) {  // the convective columns' records of this sub-batch
       SparseFields sf;
       sf.rec_len = rec_len;
       for (int qf = 0; qf < SF_N; ++qf) {
@@ -2044,6 +2053,33 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
       else scatter(NB - 1);
     }
   }
+  if (rc == 0 && g) {
+    // gathered: a sub-batch's lengath comes back as soon as its kernels are done, into the caller's array; its sum is
+    // the sub-batch's record count, and exactly that many records go to their final place in the caller's buffer
+    // (chunk after chunk, so the running sum is the exclusive prefix of lengath).  The host waits here only after
+    // every sub-batch has been enqueued.  Lengath and records share d2h_final, which has waited for no later
+    // sub-batch yet, so sub-batch b's records move while the sub-batches after it compute; d2h_early, behind every
+    // sub-batch's wait, keeps the attachments and the per-column outputs.
+    size_t hoff = 0;                       // doubles into g->rec
+    for (int b = 0; b < NB && rc == 0; ++b) {
+      const int c0 = tp.sched_first[b], nb = tp.sched_first[b + 1] - c0;
+      if (cudaStreamWaitEvent(tp.d2h_final, tp.done[b], 0) != cudaSuccess ||
+          cudaMemcpyAsync(lengath + c0, d_len + c0, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost,
+                          tp.d2h_final) != cudaSuccess ||
+          cudaEventRecord(tp.small_back[b], tp.d2h_final) != cudaSuccess ||
+          cudaEventSynchronize(tp.small_back[b]) != cudaSuccess) { rc = -100; break; }
+      moved_d2h += (long long)nb * sizeof(int);
+      size_t cnt = 0;
+      for (int c = c0; c < c0 + nb; ++c) cnt += (size_t)lengath[c];
+      const size_t n = cnt * rec_len;
+      if (n && cudaMemcpyAsync(g->rec + hoff, d_rec + (size_t)c0 * pc * rec_len, n * sizeof(double),
+                               cudaMemcpyDeviceToHost, tp.d2h_final) != cudaSuccess) rc = -100;
+      // zm_tend_trace's "remaining outputs on host" of this sub-batch: its records
+      if (cudaEventRecord(tp.final_back[b], tp.d2h_final) != cudaSuccess) rc = -100;
+      moved_d2h += (long long)n * 8;
+      hoff += n;
+    }
+  }
   if (rc == 0) copy_kind(5, 0, nchunks, tp.d2h_early);
   // the Brent failure counters of all sub-batches ride back on the return stream (it has waited for every
   // sub-batch): one synchronisation instead of one per sub-batch
@@ -2078,6 +2114,52 @@ int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const doub
   tp.last_h2d = moved_h2d; tp.last_d2h = moved_d2h;
   return fails;
 #undef CKP
+}
+
+int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const double* q, const double* u,
+                       const double* v, const double* pmid, const double* pint, const double* pdel,
+                       const double* zm, const double* zi, const double* phis, const double* pblh,
+                       const double* tpert, const double* landfrac, const double* cld, double ztodt,
+                       double* ptend_s, double* ptend_q, double* ptend_u, double* ptend_v, double* mcon,
+                       double* cme, double* pflx, double* zdu, double* rliq, double* rice, double* jctop,
+                       double* jcbot, double* prec, double* snow, double* ql, double* rprd, double* evapcdp,
+                       double* flxprec, double* flxsnow, double* dlf, double* mu, double* md, double* du,
+                       double* eu, double* ed, double* dp, double* dsubcld, int* jt, int* maxg, int* ideep,
+                       int* lengath, double* cape) {
+  NEED_INIT();
+  if (nchunks <= 0) return 0;
+  return conv_tend_batch(nchunks, ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, tpert, landfrac, cld, ztodt,
+                         ptend_s, ptend_q, ptend_u, ptend_v, mcon, cme, pflx, zdu, rliq, rice, jctop, jcbot, prec, snow,
+                         ql, rprd, evapcdp, flxprec, flxsnow, dlf, mu, md, du, eu, ed, dp, dsubcld, jt, maxg, ideep,
+                         lengath, cape, nullptr);
+}
+
+int zm_conv_tend_batch_gathered(int nchunks, const int* ncol, const double* t, const double* q, const double* u,
+                                const double* v, const double* pmid, const double* pint, const double* pdel,
+                                const double* zm, const double* zi, const double* phis, const double* pblh,
+                                const double* tpert, const double* landfrac, const double* cld, double ztodt,
+                                double* rliq, double* rice, double* jctop, double* jcbot, double* prec, double* snow,
+                                double* cape, double* dsubcld, int* jt, int* maxg, int* ideep, int* lengath,
+                                int pbuf_in_records, double* rec, long long rec_cap) {
+  NEED_INIT();
+  if (nchunks <= 0) return 0;
+  // argument checks come before anything else: a refused call writes nothing and leaves attachments and mirror alone
+  if (!ideep || !lengath || !rec) {
+    tls_err = "zm_conv_tend_batch_gathered: ideep, lengath and rec are required (non-NULL)";
+    return -9;
+  }
+  const long long L = g_params.pver, rec_len = (pbuf_in_records ? 20 : 14) * L + 4;
+  const long long need = (long long)nchunks * g_params.pcols * rec_len;
+  if (rec_cap < need) {
+    tls_err = "zm_conv_tend_batch_gathered: rec_cap = " + std::to_string(rec_cap) + " doubles, need nchunks*pcols*rec_len = " +
+              std::to_string(need) + " (rec_len = " + std::to_string(rec_len) + ")";
+    return -9;
+  }
+  const GatheredOut g{rec, pbuf_in_records != 0};
+  return conv_tend_batch(nchunks, ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, tpert, landfrac, cld, ztodt,
+                         nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, rliq, rice, jctop, jcbot,
+                         prec, snow, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+                         nullptr, nullptr, nullptr, dsubcld, jt, maxg, ideep, lengath, cape, &g);
 }
 
 // bytes the calling thread's last zm_conv_tend_batch moved over PCIe (host->device, device->host)

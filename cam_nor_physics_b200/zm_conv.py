@@ -79,6 +79,7 @@ EXPORTS = [
     "zm_set_profiling", "zm_get_kernel_times", "zm_launch_count",
     "zm_convtran1_fields", "zm_conv_tend_diag_batch", "zm_conv_tend_diag_batch_dev", "zm_get_timers",
     "zm_conv_tend_2_batch_dev", "zm_tend_transfer_bytes", "zm_build_info", "zm_conv_tend_hist_fields",
+    "zm_conv_tend_batch_gathered",
 ]
 
 
@@ -319,19 +320,42 @@ def zm_conv_tend(ncol, state: dict, ztodt: float, out: dict | None = None, keep_
         for k in TEND_OUT_INT:
             out[k] = np.zeros((nch, pc), np.int32)
         out["lengath"] = np.zeros(nch, np.int32)
+    args, names, alive = _tend_inputs(ncol, state, ztodt, out, convtran1, hist)
+    mirror_only = {"mu", "md", "du", "eu", "ed", "dp", "dsubcld", "jt", "maxg"} if keep_pbuf_on_device else set()
+    for k in TEND_ARG_ORDER:
+        a = out[k]
+        if k in mirror_only:
+            args.append(None)       # stays in the device mirror for zm_conv_tend_2 (no D2H)
+        else:
+            args.append(_ip(a) if a.dtype == np.int32 else _dp(a))
+    _attach_hist(out, names)
+    rc = lib().zm_conv_tend_batch(*args)
+    del alive                   # the attached org / convtran1 arrays had to outlive the step
+    _check(rc, "zm_conv_tend")
+    return out
+
+
+def _tend_inputs(ncol, state, ztodt, out, convtran1, hist):
+    """Marshalling shared by zm_conv_tend and zm_conv_tend_gathered: the input arguments, the org / convtran1
+    attachments, the history arrays in `out` (created or checked).  Returns (argument list, history names, arrays the
+    library holds raw pointers to: the caller keeps them alive until the step has returned)."""
+    pc, L = _grid()
+    nch = ncol.shape[0]
     ins = [_f(state[k]) for k in TEND_IN_ORDER]
     args = [C.c_int(nch), _ip(ncol)] + [_dp(a) for a in ins] + [C.c_double(ztodt)]
+    alive = []                              # attached arrays: _f may have made a copy that nothing else references
     if "org" in state:                      # zmconv_org: organisation tracer in, its tendency and column mean out
         org = _f(state["org"])
         if "orgt" not in out:
             out["orgt"], out["org2d"] = np.zeros_like(org), np.zeros_like(org)
         zm_org_fields(org, out["orgt"], out["org2d"])
+        alive.append(org)
     if convtran1 is not None:
         q3, f3 = _f(convtran1["q"]), _f(convtran1["fracis"])
         pcnst = q3.shape[1]
         out["ptend_qc"] = np.zeros_like(q3) if convtran1.get("ptend_q") is None else _f(convtran1["ptend_q"]).copy()
         dry = convtran1.get("cnst_is_dry")
-        keep = (q3, f3)                                                    # noqa: F841 (alive during the call)
+        alive += [q3, f3]
         lib().zm_convtran1_fields(C.c_int(pcnst), _ip(_i(convtran1["doconvtran"])),
                                   _ip(_i(dry)) if dry is not None else None, _dp(q3), _dp(f3), _dp(out["ptend_qc"]))
     names = hist_names(hist)
@@ -342,17 +366,95 @@ def zm_conv_tend(ncol, state: dict, ztodt: float, out: dict | None = None, keep_
         a = out[k]
         if a.shape != shape or a.dtype != np.float64 or not a.flags.c_contiguous:
             raise ZmError(f"out[{k!r}] must be a C-contiguous float64 array of shape {shape}")
-    mirror_only = {"mu", "md", "du", "eu", "ed", "dp", "dsubcld", "jt", "maxg"} if keep_pbuf_on_device else set()
-    for k in TEND_ARG_ORDER:
-        a = out[k]
-        if k in mirror_only:
-            args.append(None)       # stays in the device mirror for zm_conv_tend_2 (no D2H)
-        else:
-            args.append(_ip(a) if a.dtype == np.int32 else _dp(a))
-    if names:       # attached last: nothing above may fail and leave the attachment to a later call
+    return args, names, alive
+
+
+def _attach_hist(out, names):
+    if names:       # attached last, right before the step: nothing may fail and leave the attachment to a later call
         lib().zm_conv_tend_hist_fields(*[(_dp(out[k]) if k in names else None) for k in HIST_FIELDS])
-    rc = lib().zm_conv_tend_batch(*args)
-    _check(rc, "zm_conv_tend")
+
+
+# Record of one convective column in zm_conv_tend_batch_gathered (include/zmconv_b200.h): the fields indexed by the
+# column ideep(slot), then -- with the pbuf fields in the records -- the slot-indexed pbuf fields.
+GATHERED_FIELDS = ["ptend_s", "ptend_q", "ptend_u", "ptend_v", "cme", "zdu", "ql", "rprd", "evapcdp", "dlf",
+                   "mcon", "pflx", "flxprec", "flxsnow"]
+GATHERED_PBUF = ["mu", "md", "du", "eu", "ed", "dp"]
+GATHERED_COL_OUT = ["rliq", "rice", "jctop", "jcbot", "prec", "snow", "cape", "dsubcld"]
+
+
+def gathered_layout(pver: int, with_pbuf: bool):
+    """({field: (offset, nlev)} in doubles, rec_len) of a zm_conv_tend_batch_gathered record."""
+    lay, off = {}, 0
+    for k in GATHERED_FIELDS + (GATHERED_PBUF if with_pbuf else []):
+        n = pver + 1 if k in TEND_OUT_2DP else pver
+        lay[k] = (off, n)
+        off += n
+    return lay, off
+
+
+def zm_conv_tend_gathered(ncol, state: dict, ztodt: float, keep_pbuf_on_device: bool = False,
+                          convtran1: dict | None = None, hist=None, out: dict | None = None):
+    """zm_conv_tend with the (pcols,pver[p]) outputs returned as one record per convective column
+    (zm_conv_tend_batch_gathered).  Returns the per-column outputs (rliq, rice, jctop, jcbot, prec, snow, cape,
+    dsubcld, jt, maxg, ideep, lengath), `pbuf_in_records` and `rec`, a [sum(lengath), rec_len] view, chunk after
+    chunk in gathered order; gathered_layout gives the fields' offsets, scatter_gathered the dense arrays of zm_conv_tend.
+    keep_pbuf_on_device: mu..dp stay out of the records and, with dsubcld, jt, maxg, in the device mirror only (those
+    three are then left as found).  convtran1 / hist as in zm_conv_tend (their arrays travel whole).  Arrays already in
+    `out` are written in place; out["rec_buf"] may be a 1-D float64 buffer of at least nchunks*pcols*rec_len doubles that
+    the records are written into (e.g. page-locked once and reused)."""
+    pc, L = _grid()
+    ncol = _i(ncol)
+    nch = ncol.shape[0]
+    _, rec_len = gathered_layout(L, not keep_pbuf_on_device)
+    out = {} if out is None else out
+    for k in GATHERED_COL_OUT:
+        out.setdefault(k, np.zeros((nch, pc)))
+    for k in ("jt", "maxg", "ideep"):
+        out.setdefault(k, np.zeros((nch, pc), np.int32))
+    out.setdefault("lengath", np.zeros(nch, np.int32))
+    buf = out.get("rec_buf")
+    if buf is None:
+        buf = out["rec_buf"] = np.empty(nch * pc * rec_len)
+    if buf.dtype != np.float64 or buf.ndim != 1 or not buf.flags.c_contiguous:
+        raise ZmError("out['rec_buf'] must be a 1-D C-contiguous float64 array")
+    args, names, alive = _tend_inputs(ncol, state, ztodt, out, convtran1, hist)
+    mirror_only = {"dsubcld", "jt", "maxg"} if keep_pbuf_on_device else set()
+    for k in GATHERED_COL_OUT + ["jt", "maxg", "ideep", "lengath"]:
+        a = out[k]
+        args.append(None if k in mirror_only else (_ip(a) if a.dtype == np.int32 else _dp(a)))
+    args += [C.c_int(0 if keep_pbuf_on_device else 1), _dp(buf), C.c_longlong(buf.size)]
+    _attach_hist(out, names)
+    rc = lib().zm_conv_tend_batch_gathered(*args)
+    del alive                   # the attached org / convtran1 arrays had to outlive the step
+    _check(rc, "zm_conv_tend_gathered")
+    n = int(out["lengath"].sum())
+    out["rec"] = buf[:n * rec_len].reshape(n, rec_len)
+    out["pbuf_in_records"] = int(not keep_pbuf_on_device)
+    return out
+
+
+def scatter_gathered(res: dict) -> dict:
+    """zm_conv_tend's dense output dict rebuilt from a zm_conv_tend_gathered result: zeros, then every record's fields
+    into column ideep(slot) (slot row for the pbuf fields) of its chunk.  Without the pbuf fields in the records,
+    mu..dp are 0, as zm_conv_tend returns them with keep_pbuf_on_device."""
+    lengath, ideep, rec = res["lengath"], res["ideep"], res["rec"]
+    nch, pc = ideep.shape
+    with_pbuf = bool(res["pbuf_in_records"])
+    L = (rec.shape[1] - 4) // (20 if with_pbuf else 14)
+    lay, rec_len = gathered_layout(L, with_pbuf)
+    assert rec.shape == (int(lengath.sum()), rec_len), rec.shape
+    chunk = np.repeat(np.arange(nch), lengath)
+    slot = np.arange(rec.shape[0]) - np.repeat(np.cumsum(lengath) - lengath, lengath)
+    col = ideep[chunk, slot] - 1
+    out = {}
+    for k in TEND_OUT_2D + TEND_OUT_2DP:
+        n = L + 1 if k in TEND_OUT_2DP else L
+        out[k] = np.zeros((nch, n, pc))
+        if k in lay:
+            o, _ = lay[k]
+            out[k][chunk, :, slot if k in GATHERED_PBUF else col] = rec[:, o:o + n]
+    for k in GATHERED_COL_OUT + ["jt", "maxg", "ideep", "lengath"]:
+        out[k] = res[k]
     return out
 
 

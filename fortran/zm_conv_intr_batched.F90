@@ -12,6 +12,12 @@ module zm_conv_intr_batched
 ! pbuf fields, the history diagnostics) and carries on with physics_update / check_energy_chng.
 ! zm_conv_tend_2_batched does the same for zm_conv_tend_2 (called from tphysac).
 !
+! Gathered mode (zm_batch_init(..., gathered=.true.)): the step returns the twenty (pcols,pver[p]) outputs as one
+! record per convective column (zm_conv_tend_batch_gathered) instead of twenty dense rank-level arrays, and
+! zm_batch_scatter writes each chunk's records into ptend_all (zeroed by physics_ptend_init) and into the dummy
+! outputs and pbuf fields, which it zeroes first.  The outputs are the same; about a third of the bytes cross PCIe
+! and host memory (INTEGRATION.md section 2).
+!
 ! The five GPTL timers of the reference (t_startf/t_stopf 'zm_convr', 'zm_conv_evap', 'momtran', 'convtran1',
 ! zm_conv_intr.F90:654-880, and 'convtran2', :1019-1025) cannot bracket host code any more -- the phases run
 ! back to back on the device -- so zm_batch_report_timers reads the device times of the phases back with
@@ -66,6 +72,12 @@ module zm_conv_intr_batched
   logical :: org_on = .false.
   integer :: ixorg = -1
   real(c_double), allocatable, dimension(:,:,:) :: org_b, orgt_b, org2d_b
+  ! gathered mode: the records of the convective columns, chunk after chunk (layout: include/zmconv_b200.h,
+  ! zm_conv_tend_batch_gathered); rec_base_b(c) = sum(lengath_b(1:c-1)) is chunk c's first record
+  logical :: gathered_on = .false.
+  integer :: rec_len_b = 0
+  real(c_double), allocatable :: rec_b(:)
+  integer(c_long_long), allocatable :: rec_base_b(:)
 
   interface
      integer(c_int) function zm_conv_tend_batch(nchunks, ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, &
@@ -85,6 +97,22 @@ module zm_conv_intr_batched
        integer(c_int), intent(out) :: jt(*), maxg(*), ideep(*), lengath(*)
        real(c_double), intent(out) :: cape(*)
      end function zm_conv_tend_batch
+
+     integer(c_int) function zm_conv_tend_batch_gathered(nchunks, ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, &
+          pblh, tpert, landfrac, cld, ztodt, rliq, rice, jctop, jcbot, prec, snow, cape, dsubcld, jt, maxg, ideep, &
+          lengath, pbuf_in_records, rec, rec_cap) bind(C, name='zm_conv_tend_batch_gathered')
+       import :: c_int, c_double, c_long_long
+       integer(c_int), value :: nchunks
+       integer(c_int), intent(in) :: ncol(*)
+       real(c_double), intent(in) :: t(*), q(*), u(*), v(*), pmid(*), pint(*), pdel(*), zm(*), zi(*), phis(*), &
+                                     pblh(*), tpert(*), landfrac(*), cld(*)
+       real(c_double), value :: ztodt
+       real(c_double), intent(out) :: rliq(*), rice(*), jctop(*), jcbot(*), prec(*), snow(*), cape(*), dsubcld(*)
+       integer(c_int), intent(out) :: jt(*), maxg(*), ideep(*), lengath(*)
+       integer(c_int), value :: pbuf_in_records
+       real(c_double), intent(out) :: rec(*)
+       integer(c_long_long), value :: rec_cap
+     end function zm_conv_tend_batch_gathered
 
      integer(c_int) function zm_conv_tend_2_batch(nchunks, doconvtran, q, pcnst, pdeldry, fracis, ptend_q, ztodt, &
           cnst_is_dry) bind(C, name='zm_conv_tend_2_batch')
@@ -127,8 +155,10 @@ module zm_conv_intr_batched
        import :: c_int, c_double
        integer(c_int), value :: nchunks
        integer(c_int), intent(in) :: ncol(*)
-       real(c_double), intent(in) :: ps(*), pmid(*), mu(*), md(*)
-       integer(c_int), intent(in) :: jt(*), maxg(*), ideep(*), lengath(*)
+       real(c_double), intent(in) :: ps(*), pmid(*)
+       ! absent (NULL): taken from the library's device mirror of the last step (gathered mode)
+       real(c_double), intent(in), optional :: mu(*), md(*)
+       integer(c_int), intent(in), optional :: jt(*), maxg(*), ideep(*), lengath(*)
        real(c_double), intent(out) :: freqzm(*), mu_out(*), md_out(*), pcont(*), pconb(*)
      end function zm_conv_tend_diag_batch
 
@@ -154,25 +184,35 @@ module zm_conv_intr_batched
 contains
 
   !-------------------------------------------------------------------------------
-  subroutine zm_batch_init(nchunks, zmconv_org)
+  subroutine zm_batch_init(nchunks, zmconv_org, gathered)
     ! once, after zm_conv_init (zm_convi -> zm_init is done by the shim's zm_convi, zm_conv_intr.F90:376-379);
-    ! zmconv_org: the namelist switch zm_convi received (organisation tracer 'ZM_ORG')
+    ! zmconv_org: the namelist switch zm_convi received (organisation tracer 'ZM_ORG'); gathered: the step returns
+    ! the convective columns' records instead of the dense (pcols,pver[p]) arrays (fewer bytes through PCIe and host
+    ! memory; INTEGRATION.md section 2 says when to pick it)
     integer, intent(in) :: nchunks
-    logical, intent(in), optional :: zmconv_org
+    logical, intent(in), optional :: zmconv_org, gathered
     integer :: m
     nchunks_b = nchunks
+    gathered_on = .false.
+    if (present(gathered)) gathered_on = gathered
     allocate(ncol_b(nchunks), lengath_b(nchunks))
     allocate(t_b(pcols,pver,nchunks), q_b(pcols,pver,nchunks), u_b(pcols,pver,nchunks), v_b(pcols,pver,nchunks), &
              pmid_b(pcols,pver,nchunks), pdel_b(pcols,pver,nchunks), zm_b(pcols,pver,nchunks), cld_b(pcols,pver,nchunks), &
              pint_b(pcols,pverp,nchunks), zi_b(pcols,pverp,nchunks), phis_b(pcols,nchunks), pblh_b(pcols,nchunks), &
              tpert_b(pcols,nchunks), landfrac_b(pcols,nchunks), ps_b(pcols,nchunks))
-    allocate(ptend_s_b(pcols,pver,nchunks), ptend_q_b(pcols,pver,nchunks), ptend_u_b(pcols,pver,nchunks), &
-             ptend_v_b(pcols,pver,nchunks), cme_b(pcols,pver,nchunks), zdu_b(pcols,pver,nchunks), ql_b(pcols,pver,nchunks), &
-             rprd_b(pcols,pver,nchunks), evapcdp_b(pcols,pver,nchunks), dlf_b(pcols,pver,nchunks), mu_b(pcols,pver,nchunks), &
-             md_b(pcols,pver,nchunks), du_b(pcols,pver,nchunks), eu_b(pcols,pver,nchunks), ed_b(pcols,pver,nchunks), &
-             dp_b(pcols,pver,nchunks), mu_out_b(pcols,pver,nchunks), md_out_b(pcols,pver,nchunks))
-    allocate(mcon_b(pcols,pverp,nchunks), pflx_b(pcols,pverp,nchunks), flxprec_b(pcols,pverp,nchunks), &
-             flxsnow_b(pcols,pverp,nchunks))
+    if (gathered_on) then
+       rec_len_b = 20*pver + 4                 ! the pbuf fields mu..dp are in the records (pbuf_in_records = 1)
+       allocate(rec_b(int(rec_len_b, c_long_long)*pcols*nchunks), rec_base_b(nchunks))
+    else
+       allocate(ptend_s_b(pcols,pver,nchunks), ptend_q_b(pcols,pver,nchunks), ptend_u_b(pcols,pver,nchunks), &
+                ptend_v_b(pcols,pver,nchunks), cme_b(pcols,pver,nchunks), zdu_b(pcols,pver,nchunks), &
+                ql_b(pcols,pver,nchunks), rprd_b(pcols,pver,nchunks), evapcdp_b(pcols,pver,nchunks), &
+                dlf_b(pcols,pver,nchunks), mu_b(pcols,pver,nchunks), md_b(pcols,pver,nchunks), du_b(pcols,pver,nchunks), &
+                eu_b(pcols,pver,nchunks), ed_b(pcols,pver,nchunks), dp_b(pcols,pver,nchunks))
+       allocate(mcon_b(pcols,pverp,nchunks), pflx_b(pcols,pverp,nchunks), flxprec_b(pcols,pverp,nchunks), &
+                flxsnow_b(pcols,pverp,nchunks))
+    end if
+    allocate(mu_out_b(pcols,pver,nchunks), md_out_b(pcols,pver,nchunks))
     allocate(rliq_b(pcols,nchunks), rice_b(pcols,nchunks), jctop_b(pcols,nchunks), jcbot_b(pcols,nchunks), &
              prec_b(pcols,nchunks), snow_b(pcols,nchunks), dsubcld_b(pcols,nchunks), cape_b(pcols,nchunks), &
              freqzm_b(pcols,nchunks), pcont_b(pcols,nchunks), pconb_b(pcols,nchunks))
@@ -224,19 +264,36 @@ contains
     ! zm_conv_tend for every chunk of the rank (zm_conv_intr.F90:662-886) + its history arithmetic (:685-729)
     real(r8), intent(in) :: ztodt
     integer(c_int) :: rc
+    integer :: c
     call t_startf('zm_conv_tend_batch')
     ptend_q3_b = 0._r8                        ! physics_ptend_init(ptend_loc, ..., lq=lq) zeroes the flagged slices
     rc = zm_convtran1_fields(int(pcnst, c_int), doconvtran1, cnst_is_dry, q3_b, fracis_b, ptend_q3_b)
     if (org_on) rc = zm_org_fields(org_b, orgt_b, org2d_b)       ! zm_conv_intr.F90:656-659
     rc = zm_conv_tend_hist_fields(heat_b, qtnd_b, eurt_b, dif_b, dnlf_b, dnif_b, tend_s_b, snwprd_b, snwevmlt_b, &
          ntprprd_b, ntsnprd_b, seten_b, pguall_b, pgdall_b, icwu_b, icwd_b)
-    rc = zm_conv_tend_batch(int(nchunks_b, c_int), ncol_b, t_b, q_b, u_b, v_b, pmid_b, pint_b, pdel_b, zm_b, zi_b, &
-         phis_b, pblh_b, tpert_b, landfrac_b, cld_b, real(ztodt, c_double), ptend_s_b, ptend_q_b, ptend_u_b, ptend_v_b, &
-         mcon_b, cme_b, pflx_b, zdu_b, rliq_b, rice_b, jctop_b, jcbot_b, prec_b, snow_b, ql_b, rprd_b, evapcdp_b, &
-         flxprec_b, flxsnow_b, dlf_b, mu_b, md_b, du_b, eu_b, ed_b, dp_b, dsubcld_b, jt_b, maxg_b, ideep_b, lengath_b, cape_b)
-    if (rc /= 0) call zm_batch_abort('zm_conv_tend_batch', rc)
-    rc = zm_conv_tend_diag_batch(int(nchunks_b, c_int), ncol_b, ps_b, pmid_b, mu_b, md_b, jt_b, maxg_b, ideep_b, &
-         lengath_b, freqzm_b, mu_out_b, md_out_b, pcont_b, pconb_b)
+    if (gathered_on) then
+       rc = zm_conv_tend_batch_gathered(int(nchunks_b, c_int), ncol_b, t_b, q_b, u_b, v_b, pmid_b, pint_b, pdel_b, &
+            zm_b, zi_b, phis_b, pblh_b, tpert_b, landfrac_b, cld_b, real(ztodt, c_double), rliq_b, rice_b, jctop_b, &
+            jcbot_b, prec_b, snow_b, cape_b, dsubcld_b, jt_b, maxg_b, ideep_b, lengath_b, 1_c_int, rec_b, &
+            size(rec_b, kind=c_long_long))
+       if (rc /= 0) call zm_batch_abort('zm_conv_tend_batch_gathered', rc)
+       rec_base_b(1) = 0
+       do c = 2, nchunks_b
+          rec_base_b(c) = rec_base_b(c-1) + lengath_b(c-1)
+       end do
+       ! mu, md, jt, maxg, ideep, lengath from the device mirror the step left
+       rc = zm_conv_tend_diag_batch(int(nchunks_b, c_int), ncol_b, ps_b, pmid_b, freqzm=freqzm_b, mu_out=mu_out_b, &
+            md_out=md_out_b, pcont=pcont_b, pconb=pconb_b)
+    else
+       rc = zm_conv_tend_batch(int(nchunks_b, c_int), ncol_b, t_b, q_b, u_b, v_b, pmid_b, pint_b, pdel_b, zm_b, zi_b, &
+            phis_b, pblh_b, tpert_b, landfrac_b, cld_b, real(ztodt, c_double), ptend_s_b, ptend_q_b, ptend_u_b, &
+            ptend_v_b, mcon_b, cme_b, pflx_b, zdu_b, rliq_b, rice_b, jctop_b, jcbot_b, prec_b, snow_b, ql_b, rprd_b, &
+            evapcdp_b, flxprec_b, flxsnow_b, dlf_b, mu_b, md_b, du_b, eu_b, ed_b, dp_b, dsubcld_b, jt_b, maxg_b, &
+            ideep_b, lengath_b, cape_b)
+       if (rc /= 0) call zm_batch_abort('zm_conv_tend_batch', rc)
+       rc = zm_conv_tend_diag_batch(int(nchunks_b, c_int), ncol_b, ps_b, pmid_b, mu_b, md_b, jt_b, maxg_b, ideep_b, &
+            lengath_b, freqzm_b, mu_out_b, md_out_b, pcont_b, pconb_b)
+    end if
     if (rc /= 0) call zm_batch_abort('zm_conv_tend_diag_batch', rc)
     call t_stopf('zm_conv_tend_batch')
   end subroutine zm_conv_tend_batched
@@ -264,7 +321,8 @@ contains
                                        dp_cldliq(pcols,pver), dp_cldice(pcols,pver), org2d(pcols,pver)
     logical  :: lq(pcnst)
     real(r8) :: ftem(pcols,pver)
-    integer  :: m, ncol, ixcldliq, ixcldice
+    integer  :: m, ncol, ixcldliq, ixcldice, i, j
+    integer(c_long_long) :: r
     ncol = ncol_b(ic)
     lq(:) = .false.; lq(1) = .true.
     do m = 2, pcnst
@@ -272,10 +330,47 @@ contains
     end do
     if (org_on) lq(ixorg) = .true.
     call physics_ptend_init(ptend_all, pcols, 'zm_conv_tend', ls=.true., lu=.true., lv=.true., lq=lq)
-    ptend_all%s(:ncol,:) = ptend_s_b(:ncol,:,ic)
-    ptend_all%u(:ncol,:) = ptend_u_b(:ncol,:,ic)
-    ptend_all%v(:ncol,:) = ptend_v_b(:ncol,:,ic)
-    ptend_all%q(:ncol,:,1) = ptend_q_b(:ncol,:,ic)
+    if (gathered_on) then
+       ! everything is zero outside the convective columns (rows above lengath for the pbuf fields): zero, then
+       ! scatter the chunk's records, column ideep(j) (row j for the pbuf fields) from record rec_base_b(ic)+j
+       mcon = 0._r8; cme = 0._r8; pflx = 0._r8; zdu = 0._r8; ql = 0._r8; rprd = 0._r8; evapcdp = 0._r8
+       flxprec = 0._r8; flxsnow = 0._r8; dlf = 0._r8
+       mu = 0._r8; md = 0._r8; du = 0._r8; eu = 0._r8; ed = 0._r8; dp = 0._r8
+       do j = 1, lengath_b(ic)
+          r = (rec_base_b(ic) + j - 1) * rec_len_b           ! doubles before the record
+          i = ideep_b(j,ic)
+          ptend_all%s(i,:)   = rec_b(r+1         : r+pver)
+          ptend_all%q(i,:,1) = rec_b(r+pver+1    : r+2*pver)
+          ptend_all%u(i,:)   = rec_b(r+2*pver+1  : r+3*pver)
+          ptend_all%v(i,:)   = rec_b(r+3*pver+1  : r+4*pver)
+          cme(i,:)     = rec_b(r+4*pver+1  : r+5*pver)
+          zdu(i,:)     = rec_b(r+5*pver+1  : r+6*pver)
+          ql(i,:)      = rec_b(r+6*pver+1  : r+7*pver)
+          rprd(i,:)    = rec_b(r+7*pver+1  : r+8*pver)
+          evapcdp(i,:) = rec_b(r+8*pver+1  : r+9*pver)
+          dlf(i,:)     = rec_b(r+9*pver+1  : r+10*pver)
+          mcon(i,:)    = rec_b(r+10*pver+1 : r+11*pver+1)
+          pflx(i,:)    = rec_b(r+11*pver+2 : r+12*pver+2)
+          flxprec(i,:) = rec_b(r+12*pver+3 : r+13*pver+3)
+          flxsnow(i,:) = rec_b(r+13*pver+4 : r+14*pver+4)
+          mu(j,:)      = rec_b(r+14*pver+5 : r+15*pver+4)
+          md(j,:)      = rec_b(r+15*pver+5 : r+16*pver+4)
+          du(j,:)      = rec_b(r+16*pver+5 : r+17*pver+4)
+          eu(j,:)      = rec_b(r+17*pver+5 : r+18*pver+4)
+          ed(j,:)      = rec_b(r+18*pver+5 : r+19*pver+4)
+          dp(j,:)      = rec_b(r+19*pver+5 : r+20*pver+4)
+       end do
+       mconzm = mcon
+    else
+       ptend_all%s(:ncol,:) = ptend_s_b(:ncol,:,ic)
+       ptend_all%u(:ncol,:) = ptend_u_b(:ncol,:,ic)
+       ptend_all%v(:ncol,:) = ptend_v_b(:ncol,:,ic)
+       ptend_all%q(:ncol,:,1) = ptend_q_b(:ncol,:,ic)
+       mcon = mcon_b(:,:,ic); cme = cme_b(:,:,ic); pflx = pflx_b(:,:,ic); zdu = zdu_b(:,:,ic)
+       ql = ql_b(:,:,ic); rprd = rprd_b(:,:,ic); evapcdp = evapcdp_b(:,:,ic)
+       flxprec = flxprec_b(:,:,ic); flxsnow = flxsnow_b(:,:,ic); dlf = dlf_b(:,:,ic); mconzm = mcon_b(:,:,ic)
+       mu = mu_b(:,:,ic); md = md_b(:,:,ic); du = du_b(:,:,ic); eu = eu_b(:,:,ic); ed = ed_b(:,:,ic); dp = dp_b(:,:,ic)
+    end if
     do m = 2, pcnst
        if (lq(m) .and. doconvtran1(m) /= 0) ptend_all%q(:ncol,:,m) = ptend_q3_b(:ncol,:,m,ic)
     end do
@@ -290,11 +385,8 @@ contains
     if (present(dnifzm))    dnifzm = dnif_b(:,:,ic)
     if (present(dp_cldliq)) dp_cldliq = 0._r8
     if (present(dp_cldice)) dp_cldice = 0._r8
-    mcon = mcon_b(:,:,ic); cme = cme_b(:,:,ic); pflx = pflx_b(:,:,ic); zdu = zdu_b(:,:,ic)
     rliq = rliq_b(:,ic); rice = rice_b(:,ic); jctop = jctop_b(:,ic); jcbot = jcbot_b(:,ic)
-    prec = prec_b(:,ic); snow = snow_b(:,ic); ql = ql_b(:,:,ic); rprd = rprd_b(:,:,ic); evapcdp = evapcdp_b(:,:,ic)
-    flxprec = flxprec_b(:,:,ic); flxsnow = flxsnow_b(:,:,ic); dlf = dlf_b(:,:,ic); mconzm = mcon_b(:,:,ic)
-    mu = mu_b(:,:,ic); md = md_b(:,:,ic); du = du_b(:,:,ic); eu = eu_b(:,:,ic); ed = ed_b(:,:,ic); dp = dp_b(:,:,ic)
+    prec = prec_b(:,ic); snow = snow_b(:,ic)
     dsubcld = dsubcld_b(:,ic); jt = jt_b(:,ic); maxg = maxg_b(:,ic); ideep = ideep_b(:,ic); lengath = lengath_b(ic)
     ! history (zm_conv_intr.F90:676-729, 796-801, 882-883)
     call outfld('CAPE',     cape_b(:,ic),   pcols, lchnk)
@@ -309,8 +401,13 @@ contains
     call outfld('EVAPQZM ', ftem,           pcols, lchnk)
     call outfld('PRECCDZM   ', prec,        pcols, lchnk)
     call outfld('PRECZ   ', prec,           pcols, lchnk)
-    call outfld('ZMMTU',    ptend_u_b(:,:,ic), pcols, lchnk)
-    call outfld('ZMMTV',    ptend_v_b(:,:,ic), pcols, lchnk)
+    if (gathered_on) then                         ! no rank-level ptend_u/v: the chunk's, 0 beyond ncol like the step's
+       call outfld('ZMMTU',    ptend_all%u,    pcols, lchnk)
+       call outfld('ZMMTV',    ptend_all%v,    pcols, lchnk)
+    else
+       call outfld('ZMMTU',    ptend_u_b(:,:,ic), pcols, lchnk)
+       call outfld('ZMMTV',    ptend_v_b(:,:,ic), pcols, lchnk)
+    end if
     call cnst_get_ind('CLDLIQ', ixcldliq)
     call cnst_get_ind('CLDICE', ixcldice)
     call outfld('ZMDICE ', ptend_q3_b(:,:,ixcldice,ic), pcols, lchnk)

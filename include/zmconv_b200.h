@@ -171,6 +171,41 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
                        double* eu, double* ed, double* dp, double* dsubcld, int* jt, int* maxg, int* ideep,
                        int* lengath, double* cape, void* stream);
 
+/* zm_conv_tend_batch with the (pcols,pver[p]) outputs returned as one record of doubles per convective column, for a
+ * caller that scatters them in its own chunk loop (the batched Fortran binding's zm_batch_scatter in gathered mode).
+ * Those outputs are zero outside the convective columns -- the reference computes on the gathered columns
+ * ideep(1:lengath), zm_conv.F90:926-940 -- so a caller that zeroes its chunk arrays (physics_ptend_init does) and
+ * scatters the records gets zm_conv_tend_batch's arrays exactly, from about a third of the device->host bytes.
+ *
+ * Per-column outputs travel whole as in zm_conv_tend_batch.  ideep and lengath are required (NULL: -9);
+ * dsubcld, jt, maxg may be NULL (they then stay in the device pbuf mirror only).
+ *
+ * Records: chunk after chunk, within a chunk in gathered order (slot j = 1..lengath(c) is column ideep(j) of chunk c);
+ * chunk c's first record has the index sum(lengath(1:c-1)).  With L = pver, a record holds, at these offsets in doubles:
+ *   column-indexed, the values of column ideep(j), levels 1..L (or 1..L+1):
+ *     ptend_s 0, ptend_q L, ptend_u 2L, ptend_v 3L, cme 4L, zdu 5L, ql 6L, rprd 7L, evapcdp 8L, dlf 9L,
+ *     mcon 10L (L+1), pflx 11L+1 (L+1), flxprec 12L+2 (L+1), flxsnow 13L+3 (L+1);
+ *   pbuf_in_records != 0 only, slot-indexed (gathered row j of the pbuf field, as zm_conv_tend_batch returns it):
+ *     mu 14L+4, md 15L+4, du 16L+4, eu 17L+4, ed 18L+4, dp 19L+4.
+ * rec_len = 20L+4 with the pbuf fields, 14L+4 without; with pbuf_in_records = 0 mu..dp stay in the device mirror
+ * only (zm_conv_tend_2_batch, zm_conv_tend_diag_batch read them there).  In Fortran one chunk's records are
+ * g(rec_len, lengath(c)) and one field of one column a contiguous slice g(off+1:off+nlev, j).
+ *
+ * rec_cap (doubles) must be >= nchunks*pcols*rec_len, checked before anything else (-9, nothing written); only
+ * sum(lengath)*rec_len doubles are written and moved; a sub-batch's records leave the device as soon as its kernels
+ * end, while later sub-batches compute.  The copies into rec are asynchronous when the caller has registered it once
+ * with cudaHostRegister.  Everything else -- sub-batch pipelining (ZM_TEND_SUBBATCHES,
+ * ZM_TEND_SCHEDULE), the one-shot attachments (their arrays travel whole), the device pbuf mirror (published on
+ * success only), zm_tend_trace, zm_tend_transfer_bytes, the Brent-failure return -- is that of zm_conv_tend_batch.
+ * ZM_TEND_RETURN does not apply. */
+int zm_conv_tend_batch_gathered(int nchunks, const int* ncol, const double* t, const double* q, const double* u,
+                                const double* v, const double* pmid, const double* pint, const double* pdel,
+                                const double* zm, const double* zi, const double* phis, const double* pblh,
+                                const double* tpert, const double* landfrac, const double* cld, double ztodt,
+                                double* rliq, double* rice, double* jctop, double* jcbot, double* prec, double* snow,
+                                double* cape, double* dsubcld, int* jt, int* maxg, int* ideep, int* lengath,
+                                int pbuf_in_records, double* rec, long long rec_cap);
+
 /* Per-rank terms of the global water/energy budget check (the quantities check_energy_chng compares
  * after ZM, physpkg.F90:2865-2867); all pointers are device pointers, out6 receives
  * [sum pdel/g*ptend_q, sum 1000*(prec+rliq), sum pdel/g*ptend_s,
@@ -290,11 +325,12 @@ int zm_conv_tend_diag_batch_dev(int nchunks, const int* ncol, const double* ps, 
                             double* freqzm, double* mu_out, double* md_out, double* pcont, double* pconb,
                             void* stream);
 
-/* Pipeline timeline of the calling thread's last zm_conv_tend_batch (diagnostics): per sub-batch six times in
- * ms (inputs on device, late inputs on device, zm_convr done, all kernels done, zm_convr outputs on host,
- * remaining outputs on host).  Returns the number of sub-batches; fills at most cap doubles. */
+/* Pipeline timeline of the calling thread's last zm_conv_tend_batch[_gathered] (diagnostics): per sub-batch six times
+ * in ms (inputs on device, late inputs on device, zm_convr done, all kernels done, zm_convr outputs on host,
+ * remaining outputs -- in the gathered call the records -- on host).  Returns the number of sub-batches; fills at most
+ * cap doubles. */
 int zm_tend_trace(double* ms, int cap);
-/* bytes the calling thread's last zm_conv_tend_batch moved over PCIe in each direction */
+/* bytes the calling thread's last zm_conv_tend_batch[_gathered] moved over PCIe in each direction */
 int zm_tend_transfer_bytes(long long* h2d, long long* d2h);
 
 /* Synchronises `stream` (NULL = the CUDA default stream) and returns the number of
