@@ -5,7 +5,8 @@
 //   momtran       zm_conv.F90:2315-2715   warp per gathered column, lane = level, the four wind recurrences in one
 //                                         instruction stream
 //   convtran      zm_conv.F90:1976-2311   block per chunk (k_convtran_c); thread per (gathered column, constituent)
-//                                         as the fallback (k_convtran_t)
+//                                         as the fallback (k_convtran_t); both also as <true> instantiations that
+//                                         read and write the convective columns' records (zm_conv_tend_2 gathered)
 // The chunk-wide loop bounds ktm/kbm (zm_conv.F90:2076-2081, 2449-2454) are reproduced exactly
 // by a tiny per-chunk reduction kernel so the level ranges match the reference bit for bit.
 #pragma once
@@ -417,6 +418,11 @@ struct TranArgs {
   const double *q, *fracis, *mu, *md, *du, *eu, *ed, *dp, *dpdry;
   double* dqdt;
 };
+// Gathered instantiations of k_convtran_t / k_convtran_c (zm_conv_tend_2_batch_gathered): q, fracis and dqdt are the
+// convective columns' records instead of (pcols,pver,ncnst) chunk arrays.  Chunk c's block starts at
+// nactive*pver*rbase[c] (rbase, an extra kernel argument: exclusive prefix of lengath, k_lengath_scan); inside it the
+// Fortran array g(lengath(c), pver, nactive), i.e. element (gathered slot gi, level k0, active constituent j) at
+// (j*pver + k0)*lengath(c) + gi.  The default instantiations ignore rbase.
 
 // dqdt(:,:,m) = 0 for every active constituent (zm_conv.F90:2298): one block per (chunk, active m) slice
 __global__ void __launch_bounds__(128)
@@ -455,8 +461,11 @@ __device__ __forceinline__ double convtran_chat(double cm, double ck) {
 // occupancy than it saved: 1.16 vs 0.98 ms).
 // constituents per block: 4 up to 64 levels, 2 above
 __host__ __device__ inline int convtran_cnst_per_block(int pver) { return pver <= 64 ? 4 : 2; }
+// GATH: q / fracis / dqdt are records (see TranArgs); level k of the pair is element rb + (k-1)*len, the
+// updraft value is parked in dqdt_rec the same way, and every record element is written (no k_convtran_zero)
+template <bool GATH = false>
 __global__ void __launch_bounds__(128)
-k_convtran_t(TranArgs a) {
+k_convtran_t(TranArgs a, const int* rbase) {
   zmm::hot_tables_load();                              // before any return (block-wide barrier inside)
   const int pcols = P.pcols, pver = P.pver;
   const int tid = blockIdx.y * blockDim.x + threadIdx.x;
@@ -465,14 +474,17 @@ k_convtran_t(TranArgs a) {
   const int slot = a.slots[tid];
   const int c = slot / pcols, gi = slot - c * pcols;
   const int m = a.active[j];
-  const int ii = a.ideep[slot] - 1;
+  const int ii = GATH ? 0 : a.ideep[slot] - 1;
   const int mx = a.mx[slot];
   const int ktm = a.ktm[c], kbm = a.kbm[c];
   const double mbsth = 1.e-15;
   const bool dry = a.is_dry[m] != 0;
   const size_t mb = ((size_t)c * a.ncnst + m) * pver;
+  size_t rb = 0;
+  int rlen = 0;
+  if (GATH) { rlen = a.lengath[c]; rb = ((size_t)rbase[c] * a.nactive + (size_t)j * rlen) * pver + gi; }
 #define GA(arr, k) a.arr[cidx(c, (k) - 1, gi, pver)]
-#define QI(k) ((mb + (k) - 1) * pcols + ii)
+#define QI(k) (GATH ? rb + (size_t)((k) - 1) * rlen : (mb + (k) - 1) * pcols + ii)
 #define QS(k) a.q[QI(k)]
 #define CU(k) a.dqdt[QI(k)]
   // per-level mass-flux terms with the dry/moist switch of zm_conv.F90:2087-2105
@@ -581,6 +593,7 @@ k_convtran_t(TranArgs a) {
 // Shared memory, one row per level: [const | chat | eu*fis*c*dp -> conu | ed*fis*c*dp -> cond | mupdudp -> dcondt]
 // x 32 lanes, then mu[pcols], md[pcols]; every access is lane pointer + level*row + compile-time offset.
 // Used when pcols is a power of two from 2 to 32, the rows fit and dqdt is 16-byte aligned; k_convtran_t otherwise.
+// The gathered instantiation (records in, records out) needs no alignment: it stores 8-byte elements.
 #define CTC_T 32
 #define CTC_NW 8
 #define CTC_BPC 3
@@ -605,8 +618,12 @@ __host__ inline int convtran_c_blocks_per_chunk(int nactive, int pcols) {
   return groups < CTC_BPC ? groups : CTC_BPC;
 }
 
+// GATH (zm_conv_tend_2_batch_gathered): q / fracis / dqdt are records (see TranArgs).  Phase A1 reads a pair's
+// levels len apart from its record plane (no column map), phase D stores each constituent's pver x len plane
+// contiguously, and a chunk without convective columns has nothing to write.
+template <bool GATH = false>
 __global__ void __launch_bounds__(32 * CTC_NW, 4)
-k_convtran_c(TranArgs a, int bpc) {
+k_convtran_c(TranArgs a, int bpc, const int* rbase) {
   extern __shared__ double sm_ctc[];
   __shared__ int s_inv[CTC_T];
   const int pcols = P.pcols, pver = P.pver;
@@ -617,6 +634,10 @@ k_convtran_c(TranArgs a, int bpc) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int slice = pver * pcols;
   const size_t cbase = (size_t)c * a.ncnst * slice;    // this chunk's q / fracis / dqdt slices
+  // gathered: this chunk's record block, a constituent's plane is pver*len doubles, a level len doubles
+  const size_t rblk = GATH ? (size_t)rbase[c] * a.nactive * pver : 0;
+  const int qs = GATH ? len : pcols;                   // stride between levels of q / fracis
+  if (GATH && len == 0) return;
   if (len == 0) {                                      // nothing convective in this chunk: dqdt(:,:,m) = 0
     for (int g = g0; g * G < a.nactive; g += bpc)
       for (int j = g * G; j < min(g * G + G, a.nactive); ++j) {
@@ -628,9 +649,11 @@ k_convtran_c(TranArgs a, int bpc) {
   const int row = convtran_c_row(pcols);
   const double mbsth = 1.e-15;
   // once per block: column -> gathered position, mu / md of the chunk's convective columns
-  if (threadIdx.x < pcols) s_inv[threadIdx.x] = -1;
-  __syncthreads();
-  if (threadIdx.x < len) s_inv[a.ideep[(size_t)c * pcols + threadIdx.x] - 1] = threadIdx.x;
+  if (!GATH) {
+    if (threadIdx.x < pcols) s_inv[threadIdx.x] = -1;
+    __syncthreads();
+    if (threadIdx.x < len) s_inv[a.ideep[(size_t)c * pcols + threadIdx.x] - 1] = threadIdx.x;
+  }
   if (lane < len) {
     const double* mup = a.mu + (size_t)c * slice + lane;
     const double* mdp = a.md + (size_t)c * slice + lane;
@@ -646,10 +669,10 @@ k_convtran_c(TranArgs a, int bpc) {
   // phase D: a warp stores one constituent's slice, a lane two neighbouring columns of a row (16 bytes)
   const int hp = pcols >> 1;
   const int di = (lane % hp) * 2, dk = lane / hp, dstep = 32 / hp;
-  const int ds0 = s_inv[di], ds1 = s_inv[di + 1];
+  const int ds0 = GATH ? 0 : s_inv[di], ds1 = GATH ? 0 : s_inv[di + 1];
   // this lane's (column, constituent) pair inside a group
   const int jl = lane / len, gi = lane - jl * len;
-  const int ii = a.ideep[(size_t)c * pcols + gi] - 1;
+  const int ii = GATH ? gi : a.ideep[(size_t)c * pcols + gi] - 1;         // gathered: slot of the record plane
   const int mx = a.mx[(size_t)c * pcols + gi];
   const size_t go = (size_t)c * slice + gi;                                // gathered arrays, + k0*pcols
   double* rl = sm_ctc + lane;                                              // + k0*row + CTC_*
@@ -660,15 +683,16 @@ k_convtran_c(TranArgs a, int bpc) {
     const bool on = jl < ng;
     const int m = a.active[j0 + (on ? jl : 0)];
     const bool dry = a.is_dry[m] != 0;
-    const double* qp = a.q + cbase + (size_t)m * slice + ii;               // + k0*pcols
-    const double* fp = a.fracis + cbase + (size_t)m * slice + ii;
+    const size_t qo = GATH ? rblk + (size_t)(j0 + (on ? jl : 0)) * pver * len + ii : cbase + (size_t)m * slice + ii;
+    const double* qp = a.q + qo;                                           // + k0*qs
+    const double* fp = a.fracis + qo;
 
     // ---- phase A1: gather const and fisg (every DRAM-latency load of the group is in flight here) ----
     if (on) {
 #pragma unroll 4
       for (int k0 = warp; k0 < pver; k0 += CTC_NW) {
-        rl[k0 * row + CTC_CONST] = qp[k0 * pcols];
-        rl[k0 * row + CTC_CONU] = fp[k0 * pcols];      // fisg, replaced by the updraft term in phase A2
+        rl[k0 * row + CTC_CONST] = qp[k0 * qs];
+        rl[k0 * row + CTC_CONU] = fp[k0 * qs];         // fisg, replaced by the updraft term in phase A2
       }
     }
     __syncthreads();
@@ -735,10 +759,10 @@ k_convtran_c(TranArgs a, int bpc) {
       // the other warps pull the next group's q / fracis rows into L2 meanwhile
       const int j0n = (g + bpc) * G;
       if (jl < min(G, a.nactive - j0n)) {
-        const size_t mo = cbase + (size_t)a.active[j0n + jl] * slice + ii;
+        const size_t mo = GATH ? rblk + (size_t)(j0n + jl) * pver * len + ii : cbase + (size_t)a.active[j0n + jl] * slice + ii;
         for (int k0 = warp - 2; k0 < pver; k0 += CTC_NW - 2) {
-          asm volatile("prefetch.global.L2 [%0];" ::"l"(a.q + mo + k0 * pcols));
-          asm volatile("prefetch.global.L2 [%0];" ::"l"(a.fracis + mo + k0 * pcols));
+          asm volatile("prefetch.global.L2 [%0];" ::"l"(a.q + mo + k0 * qs));
+          asm volatile("prefetch.global.L2 [%0];" ::"l"(a.fracis + mo + k0 * qs));
         }
       }
     }
@@ -784,6 +808,16 @@ k_convtran_c(TranArgs a, int bpc) {
     }
     __syncthreads();
     // ---- phase D: dqdt(:,:,m) = 0, dqdt(ideep(i),k,m) = dcondt(i,k) (2298-2304) as whole rows ----
+    if (GATH) {                  // the records: a warp stores one constituent's pver x len plane contiguously
+      for (int j = warp; j < ng; j += CTC_NW) {
+        double* d = a.dqdt + rblk + (size_t)(j0 + j) * pver * len;
+        const double* s = sm_ctc + CTC_DC + j * len;
+        for (int e = lane; e < pver * len; e += 32) {
+          const int k0 = e / len;
+          d[e] = s[k0 * row + (e - k0 * len)];
+        }
+      }
+    } else
     for (int j = warp; j < ng; j += CTC_NW) {
       double* d = a.dqdt + cbase + (size_t)a.active[j0 + j] * slice + (dk * pcols + di);
       const double* s = sm_ctc + CTC_DC + j * len + dk * row;

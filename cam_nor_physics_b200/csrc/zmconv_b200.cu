@@ -151,6 +151,8 @@ thread_local HistFields tls_hist;
 thread_local Workspace tls_work;     // kernel work arrays
 thread_local Workspace tls_stage;    // device staging of user arrays for the host-pointer API
 thread_local Workspace tls_stage2;   // staging for zm_conv_tend_2_batch
+// bytes the thread's last zm_conv_tend_2_batch[_gathered] moved over PCIe (zm_tend_2_transfer_bytes)
+thread_local long long tls_t2_h2d = 0, tls_t2_d2h = 0;
 thread_local Workspace tls_mirror_ws; // the device pbuf mirror (see PbufMirror)
 
 // Host worker threads of the sparse return path (zero-fill of the caller's dense output arrays while the GPU works,
@@ -737,11 +739,11 @@ int convtran_enqueue(cudaStream_t s, TranArgs a, const ChunkBounds& cb) {
     const size_t smem = convtran_c_smem_bytes(pver, pcols);
     static size_t smem_set = 0;
     if (smem > smem_set) {
-      CK(cudaFuncSetAttribute(k_convtran_c, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      CK(cudaFuncSetAttribute(k_convtran_c<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       smem_set = smem;
     }
     const int bpc = convtran_c_blocks_per_chunk(a.nactive, pcols);
-    k_convtran_c<<<(unsigned)((size_t)a.nchunks * bpc), 32 * CTC_NW, smem, s>>>(a, bpc); ++tls_launches;
+    k_convtran_c<false><<<(unsigned)((size_t)a.nchunks * bpc), 32 * CTC_NW, smem, s>>>(a, bpc, nullptr); ++tls_launches;
     CK(cudaGetLastError());
     return 0;
   }
@@ -749,7 +751,37 @@ int convtran_enqueue(cudaStream_t s, TranArgs a, const ChunkBounds& cb) {
   const int cpb = convtran_cnst_per_block(pver);
   dim3 blk(32, cpb);
   dim3 grd((a.nactive + cpb - 1) / cpb, (ncolpad + 31) / 32);       // x: constituent groups, y: column groups
-  k_convtran_t<<<grd, blk, 0, s>>>(a);
+  k_convtran_t<false><<<grd, blk, 0, s>>>(a, nullptr);
+  ++tls_launches;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+// The same transport on the convective columns' records (zm_conv_tend_2_batch_gathered): q / fracis / dqdt are record
+// buffers and rbase[c] is chunk c's first record column (k_lengath_scan).  Every record element is written, so there
+// is no zero-fill launch; the block kernel takes any dqdt alignment.  One launch.
+int convtran_enqueue_gathered(cudaStream_t s, TranArgs a, const int* rbase, const ChunkBounds& cb) {
+  const int pcols = g_params.pcols, pver = g_params.pver;
+  const int ncolpad = a.nchunks * pcols;
+  if (a.nactive == 0) return 0;
+  a.ktm = cb.ktm; a.kbm = cb.kbm; a.slots = cb.slots; a.count = cb.count;
+  static const bool force_t = [] { const char* e = getenv("ZM_CONVTRAN_KERNEL"); return e && e[0] == 't'; }();
+  if (!force_t && convtran_c_fits(pver, pcols)) {
+    const size_t smem = convtran_c_smem_bytes(pver, pcols);
+    static size_t smem_set = 0;
+    if (smem > smem_set) {
+      CK(cudaFuncSetAttribute(k_convtran_c<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      smem_set = smem;
+    }
+    const int bpc = convtran_c_blocks_per_chunk(a.nactive, pcols);
+    k_convtran_c<true><<<(unsigned)((size_t)a.nchunks * bpc), 32 * CTC_NW, smem, s>>>(a, bpc, rbase); ++tls_launches;
+    CK(cudaGetLastError());
+    return 0;
+  }
+  const int cpb = convtran_cnst_per_block(pver);
+  dim3 blk(32, cpb);
+  dim3 grd((a.nactive + cpb - 1) / cpb, (ncolpad + 31) / 32);
+  k_convtran_t<true><<<grd, blk, 0, s>>>(a, rbase);
   ++tls_launches;
   CK(cudaGetLastError());
   return 0;
@@ -931,6 +963,22 @@ __global__ void k_dpdry_gather(int nchunks, const int* ideep, const int* lengath
       const int k = r / pcols, i = r - k * pcols;
       double v = 0.0;
       if (i < len) v = pdeldry[cidx(c, k, ideep[(size_t)c * pcols + i] - 1, pver)] / 100.0;
+      dpdry[(size_t)c * nper + r] = v;
+    }
+  }
+}
+// the same from the records of zm_conv_tend_2_batch_gathered: chunk c's pdeldry(ideep(1:n),:) is the Fortran array
+// (n, pver) at pver*base(c)
+__global__ void k_dpdry_gather_rec(int nchunks, const int* lengath, const int* base, const double* pdeldry_rec,
+                                   double* dpdry) {
+  const int pcols = P.pcols, pver = P.pver, nper = pcols * pver;
+  for (int c = blockIdx.x; c < nchunks; c += gridDim.x) {
+    const int len = lengath[c];
+    const double* src = pdeldry_rec + (size_t)base[c] * pver;
+    for (int r = threadIdx.x; r < nper; r += blockDim.x) {
+      const int k = r / pcols, i = r - k * pcols;
+      double v = 0.0;
+      if (i < len) v = src[k * len + i] / 100.0;
       dpdry[(size_t)c * nper + r] = v;
     }
   }
@@ -2324,6 +2372,7 @@ int zm_conv_tend_2_batch_dev(int nchunks, const int* doconvtran, const double* q
 int zm_conv_tend_2_batch(int nchunks, const int* doconvtran, const double* q, int pcnst, const double* pdeldry,
                          const double* fracis, double* ptend_q, double ztodt, const int* cnst_is_dry) {
   NEED_INIT();
+  tls_t2_h2d = tls_t2_d2h = 0;
   if (nchunks <= 0) return 0;
   const PbufMirror M = tls_mirror;
   if (M.nchunks != nchunks || !M.mu) {
@@ -2337,6 +2386,7 @@ int zm_conv_tend_2_batch(int nchunks, const int* doconvtran, const double* q, in
   const double *d_q = S.in(q, n3), *d_fr = S.in(fracis, n3), *d_pdd = S.in(pdeldry, n2);
   double* d_dpdry = st.take<double>(n2);
   double* d_dqdt = S.inout(ptend_q, n3);
+  tls_t2_h2d = (long long)(3 * n3 + n2) * (long long)sizeof(double);     // q, fracis, pdeldry, ptend_q (inout)
   // dpdry(i,:) = pdeldry(ideep(i),:)/100 for i <= lengath, else 0 (zm_conv_intr.F90:1014-1017)
   k_dpdry_gather<<<1184, 256, 0, st.stream>>>(nchunks, M.ideep, M.lengath, d_pdd, d_dpdry); ++tls_launches;
   for (auto e : st.tev) cudaEventDestroy(e);
@@ -2347,7 +2397,106 @@ int zm_conv_tend_2_batch(int nchunks, const int* doconvtran, const double* q, in
                                  (void*)st.stream);
   if (rc) return rc;
   tick(st, st.stream, "convtran2");
-  return S.flush();
+  rc = S.flush();
+  if (rc == 0) tls_t2_d2h = (long long)n3 * (long long)sizeof(double);
+  return rc;
+}
+
+// zm_conv_tend_2 on the convective columns' records (include/zmconv_b200.h): the caller packs q, fracis (and pdeldry
+// when a flagged constituent is dry) of the columns ideep(1:lengath) of the flagged constituents and scatters the
+// returned tendencies itself; the mass-flux fields come from the device mirror as in zm_conv_tend_2_batch.
+int zm_conv_tend_2_batch_gathered(int nchunks, const int* lengath, const int* doconvtran, int pcnst,
+                                  const int* cnst_is_dry, const double* q_rec, const double* fracis_rec,
+                                  const double* pdeldry_rec, double* dqdt_rec, long long rec_cap, double ztodt) {
+  NEED_INIT();
+  (void)ztodt;
+  tls_t2_h2d = tls_t2_d2h = 0;
+  if (nchunks <= 0) return 0;
+  const PbufMirror M = tls_mirror;
+  if (M.nchunks != nchunks || !M.mu) {
+    tls_err = "zm_conv_tend_2_batch_gathered: no device mirror from a zm_conv_tend_batch call with the same nchunks on "
+              "this thread";
+    return -7;
+  }
+  if (!doconvtran || pcnst < 1) {
+    tls_err = "zm_conv_tend_2_batch_gathered: doconvtran is required and pcnst must be >= 1";
+    return -9;
+  }
+  // the active list of the layout: m = 2..pcnst (1-based) with doconvtran(m), ascending
+  int nact = 0;
+  bool any_dry = false;
+  for (int m = 1; m < pcnst; ++m)
+    if (doconvtran[m]) { ++nact; any_dry = any_dry || (cnst_is_dry && cnst_is_dry[m]); }
+  if (nact == 0) return 0;
+  if (!lengath || !q_rec || !fracis_rec || !dqdt_rec || (any_dry && !pdeldry_rec)) {
+    tls_err = "zm_conv_tend_2_batch_gathered: lengath, q_rec, fracis_rec, dqdt_rec are required, and pdeldry_rec when a "
+              "flagged constituent is dry";
+    return -9;
+  }
+  const size_t pc = g_params.pcols, L = g_params.pver, nc = (size_t)nchunks * pc, n2 = nc * L;
+  Workspace& st = tls_stage2;
+  if (!st.stream && st.ensure(0)) return -100;
+  // the caller's lengath must be the mirror's: the records were packed with it and the kernels address them with it
+  std::vector<int> mlen(nchunks);
+  CK(cudaMemcpyAsync(mlen.data(), M.lengath, nchunks * sizeof(int), cudaMemcpyDeviceToHost, st.stream));
+  CK(cudaStreamSynchronize(st.stream));
+  tls_t2_d2h = (long long)nchunks * (long long)sizeof(int);
+  long long ncols = 0;
+  for (int c = 0; c < nchunks; ++c) {
+    if (lengath[c] != mlen[c]) {
+      tls_err = "zm_conv_tend_2_batch_gathered: lengath(" + std::to_string(c + 1) + ") = " + std::to_string(lengath[c]) +
+                " differs from the device mirror's " + std::to_string(mlen[c]);
+      return -9;
+    }
+    ncols += mlen[c];
+  }
+  const long long nrec = ncols * (long long)L * nact;
+  if (rec_cap < nrec) {
+    tls_err = "zm_conv_tend_2_batch_gathered: rec_cap = " + std::to_string(rec_cap) + " doubles, need sum(lengath)*pver*nact = " +
+              std::to_string(nrec);
+    return -9;
+  }
+  if (nrec == 0) return 0;                   // no convective column anywhere: nothing to transport or write
+  const size_t npd = any_dry ? (size_t)ncols * L : 0;
+  if (st.ensure(al(nchunks + 1, 4) + 3 * al(nrec, 8) + al(npd, 8) + (any_dry ? al(n2, 8) : 0) +
+                chunk_bounds_bytes(nchunks, (int)nc) + 4096)) return -100;
+  if (tls_tmeta.set(doconvtran, cnst_is_dry, pcnst)) return -100;
+  Stager S(st);
+  const double *d_q = S.in(q_rec, nrec), *d_fr = S.in(fracis_rec, nrec);
+  const double* d_pdd = any_dry ? S.in(pdeldry_rec, npd) : nullptr;
+  double* d_dqdt = S.out(dqdt_rec, nrec);
+  tls_t2_h2d = (long long)(2 * nrec + npd) * (long long)sizeof(double);
+  int* d_base = st.take<int>(nchunks + 1);
+  k_lengath_scan<<<1, 256, 0, st.stream>>>(nchunks, M.lengath, d_base); ++tls_launches;
+  double* d_dpdry = nullptr;
+  if (any_dry) {
+    // dpdry(i,:) = pdeldry(ideep(i),:)/100 for i <= lengath, else 0 (zm_conv_intr.F90:1014-1017), slot layout
+    d_dpdry = st.take<double>(n2);
+    k_dpdry_gather_rec<<<1184, 256, 0, st.stream>>>(nchunks, M.lengath, d_base, d_pdd, d_dpdry); ++tls_launches;
+  }
+  for (auto e : st.tev) cudaEventDestroy(e);
+  st.tev.clear(); st.tnames.clear();
+  tick(st, st.stream, "start");
+  TranArgs a;
+  a.nchunks = nchunks; a.ncnst = pcnst; a.nactive = tls_tmeta.nactive; a.jt = M.jt; a.mx = M.maxg; a.ideep = M.ideep;
+  a.lengath = M.lengath; a.active = tls_tmeta.active(); a.is_dry = tls_tmeta.dry();
+  a.q = d_q; a.fracis = d_fr; a.mu = M.mu; a.md = M.md; a.du = M.du; a.eu = M.eu; a.ed = M.ed; a.dp = M.dp;
+  a.dpdry = d_dpdry; a.dqdt = d_dqdt;
+  ChunkBounds cb;
+  if (chunk_bounds_enqueue(st, st.stream, nchunks, M.jt, M.maxg, M.lengath, cb)) return -100;
+  int rc = convtran_enqueue_gathered(st.stream, a, d_base, cb);
+  if (rc) return rc;
+  tick(st, st.stream, "convtran2");
+  rc = S.flush();
+  if (rc == 0) tls_t2_d2h += nrec * (long long)sizeof(double);
+  return rc;
+}
+
+// bytes the calling thread's last zm_conv_tend_2_batch[_gathered] moved over PCIe (host->device, device->host)
+int zm_tend_2_transfer_bytes(long long* h2d, long long* d2h) {
+  if (h2d) *h2d = tls_t2_h2d;
+  if (d2h) *d2h = tls_t2_d2h;
+  return 0;
 }
 
 // ---- N4 neighbours: geopotential_t, convect_diagnostics_calc ----------------------------------------

@@ -79,7 +79,7 @@ EXPORTS = [
     "zm_set_profiling", "zm_get_kernel_times", "zm_launch_count",
     "zm_convtran1_fields", "zm_conv_tend_diag_batch", "zm_conv_tend_diag_batch_dev", "zm_get_timers",
     "zm_conv_tend_2_batch_dev", "zm_tend_transfer_bytes", "zm_build_info", "zm_conv_tend_hist_fields",
-    "zm_conv_tend_batch_gathered",
+    "zm_conv_tend_batch_gathered", "zm_conv_tend_2_batch_gathered", "zm_tend_2_transfer_bytes",
 ]
 
 
@@ -293,6 +293,103 @@ def zm_conv_tend_2(doconvtran, q, pdeldry, fracis, ztodt, cnst_is_dry, ptend_q=N
                                     _dp(_f(fracis)), _dp(dq), C.c_double(ztodt), _ip(_i(cnst_is_dry)))
     _check(rc, "zm_conv_tend_2")
     return dq
+
+
+# ---- zm_conv_tend_2 on the convective columns' records (zm_conv_tend_2_batch_gathered) ----------------------------
+def convtran2_active(doconvtran, pcnst: int) -> np.ndarray:
+    """0-based indices m >= 1 with doconvtran[m] (the reference's m = 2..pcnst loop), ascending: the constituent axis
+    of the records."""
+    do = np.asarray(doconvtran)
+    return np.array([m for m in range(1, pcnst) if do[m]], dtype=np.int64)
+
+
+def convtran2_offsets(lengath, pver: int, nact: int) -> np.ndarray:
+    """[nchunks + 1] offsets (doubles) of the chunks' blocks in q_rec / fracis_rec / dqdt_rec: nact*pver*base(c) with
+    base(c) = sum(lengath(1:c-1)); the last entry is the records' total size.  pdeldry_rec's are these / nact."""
+    lg = np.asarray(lengath, dtype=np.int64)
+    return nact * pver * np.concatenate([[0], np.cumsum(lg)])
+
+
+def convtran2_records(q, fracis, pdeldry, ideep, lengath, doconvtran, cnst_is_dry=None):
+    """The caller's pack (loop 1 of the batched Fortran binding in gathered mode): q, fracis `[nchunks, pcnst, pver,
+    pcols]` and pdeldry `[nchunks, pver, pcols]` of each chunk's convective columns ideep(1:lengath) and flagged
+    constituents.  Returns (q_rec, fracis_rec, pdeldry_rec) as 1-D float64 arrays; pdeldry_rec is None when no flagged
+    constituent is dry.  Chunk c's block is g(n, pver, nact) in Fortran order (include/zmconv_b200.h)."""
+    q, fracis = np.asarray(q), np.asarray(fracis)
+    nch, pcnst, L, _ = q.shape
+    lengath = np.asarray(lengath)
+    act = convtran2_active(doconvtran, pcnst)
+    off = convtran2_offsets(lengath, L, len(act))
+    any_dry = cnst_is_dry is not None and len(act) > 0 and bool(np.asarray(cnst_is_dry)[act].any())
+    q_rec, f_rec = np.empty(off[-1]), np.empty(off[-1])
+    p_rec = np.empty(off[-1] // max(len(act), 1)) if any_dry else None
+    for c in range(nch):
+        n = int(lengath[c])
+        if n == 0 or len(act) == 0:
+            continue
+        cols = np.asarray(ideep[c][:n]) - 1
+        q_rec[off[c]:off[c + 1]] = q[c][act][:, :, cols].ravel()
+        f_rec[off[c]:off[c + 1]] = fracis[c][act][:, :, cols].ravel()
+        if any_dry:
+            o = off[c] // len(act)
+            p_rec[o:o + L * n] = np.asarray(pdeldry[c])[:, cols].ravel()
+    return q_rec, f_rec, p_rec
+
+
+def scatter_convtran2(dqdt_rec, ideep, lengath, doconvtran, pcnst: int, pver: int | None = None):
+    """The caller's scatter (loop 2): the dense `[nchunks, pcnst, pver, pcols]` tendency zm_conv_tend_2 returns, rebuilt
+    from dqdt_rec -- zero everywhere except the flagged constituents' convective columns.  pver defaults to the records'
+    size over sum(lengath)*nact (or zm_init's pver when there are no records)."""
+    ideep, lengath = np.asarray(ideep), np.asarray(lengath)
+    nch, pc = ideep.shape
+    act = convtran2_active(doconvtran, pcnst)
+    nact = len(act)
+    tot = int(lengath.astype(np.int64).sum())
+    L = pver if pver is not None else (np.asarray(dqdt_rec).size // (tot * nact) if tot and nact else _grid()[1])
+    off = convtran2_offsets(lengath, L, nact)
+    out = np.zeros((nch, pcnst, L, pc))
+    for c in range(nch):
+        n = int(lengath[c])
+        if n == 0 or nact == 0:
+            continue
+        cols = ideep[c][:n] - 1
+        out[c][act[:, None, None], np.arange(L)[None, :, None], cols[None, None, :]] = \
+            dqdt_rec[off[c]:off[c + 1]].reshape(nact, L, n)
+    return out
+
+
+def zm_conv_tend_2_gathered(lengath, doconvtran, pcnst, cnst_is_dry, q_rec, fracis_rec, pdeldry_rec, ztodt,
+                            out=None):
+    """zm_conv_tend_2 on the records of convtran2_records (zm_conv_tend_2_batch_gathered), the mass-flux fields taken
+    from the device mirror of this thread's last zm_conv_tend call.  Returns dqdt_rec (sum(lengath)*pver*nact doubles,
+    scatter_convtran2 gives the dense tendency).  `out` may be a preallocated 1-D float64 buffer (e.g. page-locked) of
+    at least that size; the result is then a view of it."""
+    _, L = _grid()
+    lengath = _i(lengath)
+    nch = lengath.shape[0]
+    do = _i(doconvtran)
+    nact = len(convtran2_active(do, pcnst))
+    need = int(lengath.astype(np.int64).sum()) * L * nact
+    if out is None:
+        out = np.empty(need)
+    if out.dtype != np.float64 or out.ndim != 1 or not out.flags.c_contiguous:
+        raise ZmError("out must be a 1-D C-contiguous float64 array")
+    # converted copies are bound to names: the library reads them through raw pointers while the call runs
+    dry = _i(cnst_is_dry) if cnst_is_dry is not None else None
+    qr, fr = _f(q_rec), _f(fracis_rec)
+    pr = _f(pdeldry_rec) if pdeldry_rec is not None else None
+    rc = lib().zm_conv_tend_2_batch_gathered(
+        C.c_int(nch), _ip(lengath), _ip(do), C.c_int(pcnst), _ip(dry) if dry is not None else None, _dp(qr), _dp(fr),
+        _dp(pr) if pr is not None else None, _dp(out), C.c_longlong(out.size), C.c_double(ztodt))
+    _check(rc, "zm_conv_tend_2_gathered")
+    return out[:need]
+
+
+def last_tend_2_transfer_bytes():
+    """(host->device, device->host) bytes the last zm_conv_tend_2[_gathered] call of this thread moved over PCIe."""
+    a, b = C.c_longlong(0), C.c_longlong(0)
+    lib().zm_tend_2_transfer_bytes(C.byref(a), C.byref(b))
+    return {"h2d": int(a.value), "d2h": int(b.value)}
 
 
 def zm_conv_tend(ncol, state: dict, ztodt: float, out: dict | None = None, keep_pbuf_on_device: bool = False,

@@ -16,7 +16,10 @@ module zm_conv_intr_batched
 ! record per convective column (zm_conv_tend_batch_gathered) instead of twenty dense rank-level arrays, and
 ! zm_batch_scatter writes each chunk's records into ptend_all (zeroed by physics_ptend_init) and into the dummy
 ! outputs and pbuf fields, which it zeroes first.  The outputs are the same; about a third of the bytes cross PCIe
-! and host memory (INTEGRATION.md section 2).
+! and host memory (INTEGRATION.md section 2).  zm_conv_tend_2 follows suit: zm_batch_gather_2 packs the convective
+! columns of the constituents flagged convtran2 (and their pdeldry when one of them is dry), zm_conv_tend_2_batched
+! transports those records (zm_conv_tend_2_batch_gathered) and zm_batch_scatter_2 scatters them into the ptend that
+! physics_ptend_init has just zeroed.  The columns are ideep_b / lengath_b of this time step's zm_conv_tend_batched.
 !
 ! The five GPTL timers of the reference (t_startf/t_stopf 'zm_convr', 'zm_conv_evap', 'momtran', 'convtran1',
 ! zm_conv_intr.F90:654-880, and 'convtran2', :1019-1025) cannot bracket host code any more -- the phases run
@@ -78,6 +81,12 @@ module zm_conv_intr_batched
   integer :: rec_len_b = 0
   real(c_double), allocatable :: rec_b(:)
   integer(c_long_long), allocatable :: rec_base_b(:)
+  ! gathered mode, zm_conv_tend_2: the records of the nact2 constituents iact2 flagged convtran2; chunk c's block is
+  ! g(lengath_b(c), pver, nact2) at nact2*pver*rec_base_b(c), its pdeldry(ideep(1:n),:) at pver*rec_base_b(c)
+  integer :: nact2 = 0
+  integer, allocatable :: iact2(:)
+  logical :: dry2_any = .false.
+  real(c_double), allocatable :: q2rec_b(:), fracis2rec_b(:), pdeldry2rec_b(:), dq2rec_b(:)
 
   interface
      integer(c_int) function zm_conv_tend_batch(nchunks, ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, &
@@ -126,6 +135,19 @@ module zm_conv_intr_batched
        real(c_double), value :: ztodt
        integer(c_int), intent(in) :: cnst_is_dry(*)
      end function zm_conv_tend_2_batch
+
+     integer(c_int) function zm_conv_tend_2_batch_gathered(nchunks, lengath, doconvtran, pcnst, cnst_is_dry, q_rec, &
+          fracis_rec, pdeldry_rec, dqdt_rec, rec_cap, ztodt) bind(C, name='zm_conv_tend_2_batch_gathered')
+       import :: c_int, c_double, c_long_long
+       integer(c_int), value :: nchunks
+       integer(c_int), intent(in) :: lengath(*), doconvtran(*)
+       integer(c_int), value :: pcnst
+       integer(c_int), intent(in) :: cnst_is_dry(*)
+       real(c_double), intent(in) :: q_rec(*), fracis_rec(*), pdeldry_rec(*)
+       real(c_double), intent(out) :: dqdt_rec(*)
+       integer(c_long_long), value :: rec_cap
+       real(c_double), value :: ztodt
+     end function zm_conv_tend_2_batch_gathered
 
      integer(c_int) function zm_convtran1_fields(pcnst, doconvtran, cnst_is_dry, q, fracis, ptend_q) &
           bind(C, name='zm_convtran1_fields')
@@ -239,6 +261,22 @@ contains
        if (cnst_is_convtran2(m)) doconvtran2(m) = 1
        if (cnst_get_type_byind(m) == 'dry') cnst_is_dry(m) = 1
     end do
+    if (gathered_on) then
+       ! convtran2's records: the flagged constituents m = 2..pcnst in ascending order (the library's active list;
+       ! doconvtran2(1) is 0)
+       nact2 = count(doconvtran2 /= 0)
+       allocate(iact2(nact2))
+       iact2 = pack([(m, m = 1, pcnst)], doconvtran2 /= 0)
+       dry2_any = any(cnst_is_dry(iact2) /= 0)
+       allocate(q2rec_b(int(pcols, c_long_long)*nchunks*pver*max(nact2, 1)), &
+                fracis2rec_b(int(pcols, c_long_long)*nchunks*pver*max(nact2, 1)), &
+                dq2rec_b(int(pcols, c_long_long)*nchunks*pver*max(nact2, 1)))
+       if (dry2_any) then
+          allocate(pdeldry2rec_b(int(pcols, c_long_long)*nchunks*pver))
+       else
+          allocate(pdeldry2rec_b(1))
+       end if
+    end if
   end subroutine zm_batch_init
 
   !-------------------------------------------------------------------------------
@@ -455,6 +493,22 @@ contains
     integer, intent(in) :: ic
     type(physics_state), intent(in) :: state
     real(r8), intent(in) :: fracis(pcols,pver,pcnst)
+    integer :: n
+    integer(c_long_long) :: o, sz
+    if (gathered_on) then
+       ! the chunk's convective columns ideep(1:n) of the flagged constituents (and their pdeldry), each one section
+       n = lengath_b(ic)
+       if (n == 0 .or. nact2 == 0) return
+       o = int(nact2, c_long_long)*pver*rec_base_b(ic)
+       sz = int(n, c_long_long)*pver*nact2
+       q2rec_b(o+1:o+sz) = reshape(state%q(ideep_b(1:n,ic),:,iact2), [sz])
+       fracis2rec_b(o+1:o+sz) = reshape(fracis(ideep_b(1:n,ic),:,iact2), [sz])
+       if (dry2_any) then
+          o = int(pver, c_long_long)*rec_base_b(ic)
+          pdeldry2rec_b(o+1:o+int(n, c_long_long)*pver) = reshape(state%pdeldry(ideep_b(1:n,ic),:), [n*pver])
+       end if
+       return
+    end if
     q3_b(:,:,:,ic) = state%q
     pdeldry_b(:,:,ic) = state%pdeldry
     fracis_b(:,:,:,ic) = fracis
@@ -464,6 +518,14 @@ contains
     real(r8), intent(in) :: ztodt
     integer(c_int) :: rc
     call t_startf('zm_conv_tend_2_batch')
+    if (gathered_on) then
+       ! mass fluxes, ideep and lengath from the device mirror; lengath_b is checked against it
+       rc = zm_conv_tend_2_batch_gathered(int(nchunks_b, c_int), lengath_b, doconvtran2, int(pcnst, c_int), cnst_is_dry, &
+            q2rec_b, fracis2rec_b, pdeldry2rec_b, dq2rec_b, size(dq2rec_b, kind=c_long_long), real(ztodt, c_double))
+       if (rc /= 0) call zm_batch_abort('zm_conv_tend_2_batch_gathered', rc)
+       call t_stopf('zm_conv_tend_2_batch')
+       return
+    end if
     ptend_q3_b = 0._r8
     rc = zm_conv_tend_2_batch(int(nchunks_b, c_int), doconvtran2, q3_b, int(pcnst, c_int), pdeldry_b, fracis_b, &
                               ptend_q3_b, real(ztodt, c_double), cnst_is_dry)
@@ -476,12 +538,22 @@ contains
     integer, intent(in) :: ic
     type(physics_ptend), intent(out) :: ptend
     logical :: lq(pcnst)
-    integer :: m, ncol
+    integer :: m, ncol, n
+    integer(c_long_long) :: o, sz
     ncol = ncol_b(ic)
     do m = 1, pcnst
        lq(m) = doconvtran2(m) /= 0
     end do
     call physics_ptend_init(ptend, pcols, 'convtran2', lq=lq)
+    if (gathered_on) then
+       ! ptend%q is zero: only the chunk's records go to their columns ideep(1:n) of the flagged constituents
+       n = lengath_b(ic)
+       if (n == 0 .or. nact2 == 0) return
+       o = int(nact2, c_long_long)*pver*rec_base_b(ic)
+       sz = int(n, c_long_long)*pver*nact2
+       ptend%q(ideep_b(1:n,ic),:,iact2) = reshape(dq2rec_b(o+1:o+sz), [n, pver, nact2])
+       return
+    end if
     do m = 2, pcnst
        if (lq(m)) ptend%q(:ncol,:,m) = ptend_q3_b(:ncol,:,m,ic)
     end do

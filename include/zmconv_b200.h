@@ -273,6 +273,32 @@ int zm_conv_tend_2_batch_dev(int nchunks, const int* doconvtran, const double* q
                          const double* ed, const double* dp, const double* dsubcld, const int* jt,
                          const int* maxg, const int* ideep, const int* lengath, void* stream);
 
+/* zm_conv_tend_2_batch on the convective columns' records, for a caller that packs and scatters them in its own chunk
+ * loops (the batched Fortran binding's gathered mode).  convtran reads and writes only the gathered columns
+ * ideep(1:lengath) (zm_conv.F90:2109-2114, 2298-2304; dpdry zm_conv_intr.F90:1014-1017) and the model copies the
+ * result into a ptend that physics_ptend_init has just zeroed, so only those columns of the flagged constituents
+ * need to cross PCIe and host memory.
+ *
+ * Active list: m = 2..pcnst (1-based) with doconvtran(m) != 0, ascending, nact of them; entry 1 is ignored as in
+ * zm_conv_tend_2_batch.  cnst_is_dry[pcnst] may be NULL (all moist).
+ * Layout, with base(c) = sum(lengath(1:c-1)) and n = lengath(c): chunk c's block of q_rec, fracis_rec and dqdt_rec
+ * starts at nact*pver*base(c) and is the Fortran array g(n, pver, nact) = q(ideep(1:n), :, iact(1:nact)) of the chunk
+ * (C order [a][k][slot]); pdeldry_rec holds pdeldry(ideep(1:n), :) at pver*base(c).  The pack and the scatter of a
+ * chunk are each one array section.
+ * mu..dp, jt, maxg, ideep, lengath come from the calling thread's device pbuf mirror as in zm_conv_tend_2_batch
+ * (none, or another nchunks: -7).  Refused with -9 before anything is written: lengath differing from the mirror's
+ * (read back from the device: 4*nchunks bytes), rec_cap (doubles; the size of each of q_rec, fracis_rec, dqdt_rec)
+ * below sum(lengath)*pver*nact, pdeldry_rec NULL while a flagged constituent is dry.  nact = 0: returns 0, writes
+ * nothing.  Exactly sum(lengath)*pver*nact doubles of dqdt_rec are written; the records are the only data that cross
+ * PCIe besides that lengath check.  Device times go to the GPTL name convtran2 (zm_get_timers). */
+int zm_conv_tend_2_batch_gathered(int nchunks, const int* lengath, const int* doconvtran, int pcnst,
+                                  const int* cnst_is_dry, const double* q_rec, const double* fracis_rec,
+                                  const double* pdeldry_rec, double* dqdt_rec, long long rec_cap, double ztodt);
+/* bytes the calling thread's last zm_conv_tend_2_batch[_gathered] moved over PCIe in each direction (its data arrays
+ * and, in the gathered call, the lengath check; the constituent flag table, uploaded only when the flags change, is
+ * not counted) */
+int zm_tend_2_transfer_bytes(long long* h2d, long long* d2h);
+
 /* zm_org = 1 (zmconv_org, SURVEY N3): attach the pointer dummies org / orgt / org2d of zm_convr
  * (zm_conv.F90:242, 421-423; zm_conv_intr.F90:656-659) for the NEXT zm_convr_batch / zm_conv_tend_batch [_dev] call
  * of the calling thread: host pointers for the host-pointer entry points, device pointers for *_dev.  All three are
