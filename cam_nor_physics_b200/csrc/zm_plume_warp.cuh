@@ -53,6 +53,63 @@ struct PlumeShT {
 #define PAR(k, lo, hi) _Pragma("unroll 1") for (int k = (lo) + lane; k <= (hi); k += 32)
 #define WSYNC() __syncwarp()
 
+// Phase timers (built only with -DZM_PLUME_PHASE_CLOCKS, scripts/plume_phase_cycles.py): lane 0 of every warp adds the
+// clock64() cycles since the previous mark to its kernel's row (0 = k_cldprp_pass1_w, 1 = k_plume_w); the last slot
+// counts the columns.  cldprp_warp keeps a clock of its own (PH_BEGIN), the kernels restart theirs when it returns.
+// Without the macro the marks expand to nothing and the kernels compile as without them.
+enum PlumePhase {
+  PH_GATHER, PH_INIT, PH_J0, PH_K1_PREP, PH_K1, PH_EXPDIF, PH_F, PH_FMAX, PH_MU, PH_HU, PH_JT, PH_CLDTOP,
+  PH_EU_SCAN, PH_SUQU_PREP, PH_SUQU, PH_SAT_CU, PH_QL_PREP, PH_QL, PH_HD_PREP, PH_HD, PH_SD_PREP, PH_SD, PH_PFLX,
+  PH_CLOSURE, PH_Q1Q2, PH_SCATTER,
+  PH_COUNT
+};
+#ifdef ZM_PLUME_PHASE_CLOCKS
+__device__ unsigned long long g_plume_phase[2][PH_COUNT + 1];
+#define PH_BEGIN(kern)                                                                       \
+  const int ph_kern_ = (kern);                                                               \
+  long long ph_t_ = clock64()
+#define PH_COLUMN() (lane == 0 ? (void)atomicAdd(&g_plume_phase[ph_kern_][PH_COUNT], 1ull) : (void)0)
+#define PH_RESTART() (ph_t_ = clock64())
+#define PH_MARK(ph)                                                                          \
+  do {                                                                                       \
+    const long long ph_now_ = clock64();                                                     \
+    if (lane == 0) atomicAdd(&g_plume_phase[ph_kern_][ph], (unsigned long long)(ph_now_ - ph_t_)); \
+    ph_t_ = ph_now_;                                                                         \
+  } while (0)
+#else
+#define PH_BEGIN(kern) ((void)0)
+#define PH_COLUMN() ((void)0)
+#define PH_RESTART() ((void)0)
+#define PH_MARK(ph) ((void)0)
+#endif
+
+// Warp collectives over lane == level values.  For the searches below they reproduce the serial scans exactly: each
+// predicate or value is evaluated per level as the scan would, and only the position of a hit is reduced.
+__device__ __forceinline__ double warp_min(double v) {
+  for (int off = 16; off; off >>= 1) v = fmin2(v, __shfl_xor_sync(0xffffffffu, v, off));
+  return v;
+}
+__device__ __forceinline__ int warp_max(int v) { return __reduce_max_sync(0xffffffffu, v); }
+
+// Level where `for (k...) if (valid(k) && v(k) <= vmin) { vmin = v(k); kbest = k; }` (vmin starting at 1.E6) ends up:
+// the highest valid level whose value equals the minimum over the valid levels with v <= 1.E6 (a value the running
+// minimum accepts; NaN never is).  -0 == +0, so the level does not depend on which zero the reduction returns.
+// Returns 0 when no level is accepted.  The caller reads the value back at that level, so it keeps its sign.
+template <class PlumeSh>
+__device__ __forceinline__ int warp_last_argmin(const PlumeSh& S, int arr, int lo, int hi, int lane) {
+  double m = 1.E6;
+  bool any = false;
+  PAR(k, lo, hi) {
+    const double v = S(arr, k);
+    if (v <= 1.E6) { m = fmin2(m, v); any = true; }
+  }
+  m = warp_min(m);
+  if (!__any_sync(0xffffffffu, any)) return 0;
+  int kbest = 0;
+  PAR(k, lo, hi) if (S(arr, k) == m) kbest = k;        // == never holds for a NaN or for a value above 1.E6 (m <= 1.E6)
+  return warp_max(kbest);
+}
+
 // gather one column into shared arrays (zm_conv.F90:926-940, 980-1027 / 1114-1195); returns dsubcld
 template <class PlumeSh>
 __device__ __forceinline__ double gather_column_w(const PlumeSh& S, const ConvrIn& in, int c, int i, int maxg,
@@ -105,6 +162,7 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
   const int mx = jb;
   const double c0mask = P.c0_ocn * (1.0 - landfrac) + P.c0_lnd * landfrac;
   const double tiedke_msk = P.tiedke_add * (1.0 - landfrac) + P.tiedke_lnd * landfrac;
+  PH_BEGIN(FULL ? 1 : 0);
 
   // ---- level-parallel initialisation (zm_conv.F90:3256-3314) ----
   PAR(k, 1, pver + 1) {
@@ -151,16 +209,15 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
     }
   }
   WSYNC();
+  PH_MARK(PH_INIT);
 
   // ---- scalars (redundant on every lane) ----
   int jt = max(lel, limcnv + 1);
   jt = min(jt, pver);
-  int jd = pver, jlcl = lel, j0 = 0;
-  double hmin = 1.E6;
-  for (int k = msg + 1; k <= pver; ++k) {
-    const double hs = S(A_HSAT, k);
-    if (hs <= hmin && k >= jt && k <= jb) { hmin = hs; j0 = k; }
-  }
+  int jd = pver, jlcl = lel;
+  // zm_conv.F90:3422-3428: last level of least hsat in [jt, jb]
+  int j0 = warp_last_argmin(S, A_HSAT, max(msg + 1, jt), min(pver, jb), lane);
+  PH_MARK(PH_J0);
   j0 = min(j0, jb - 2);
   j0 = max(j0, jt + 2);
   j0 = min(j0, pver);
@@ -175,32 +232,35 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
   // k1, i2, i3, i4 recurrences (zm_conv.F90:3430-3442) -- serial, redundant on every lane
   PAR(k, msg + 1, pver) S(A_W1, k) = (hmn_mx - S(A_HMN, k)) * S(A_DZ, k);
   WSYNC();
+  PH_MARK(PH_K1_PREP);
   {
-    double k1p = 0.0, i2p = 0.0, i3p = 0.0, i4p = 0.0;        // values at k+1 (zero at k = jb and below)
-    for (int k = pver - 1; k >= msg + 1; --k) {
-      if (k < jb && k >= jt) {
-        const double dz = S(A_DZ, k);
-        const double k1 = k1p + S(A_W1, k);
-        const double ihat = 0.5 * (k1p + k1);
-        const double i2 = i2p + ihat * dz;
-        const double idag = 0.5 * (i2p + i2);
-        const double i3 = i3p + idag * dz;
-        const double iprm = 0.5 * (i3p + i3);
-        const double i4 = i4p + iprm * dz;
-        S(A_K1, k) = k1; S(A_I2, k) = i2; S(A_I3, k) = i3; S(A_I4, k) = i4;
-        k1p = k1; i2p = i2; i3p = i3; i4p = i4;
-      } else {
-        k1p = S(A_K1, k); i2p = S(A_I2, k); i3p = S(A_I3, k); i4p = S(A_I4, k);
-      }
+    // The reference walks k = pver-1 .. msg+1 and, outside [jt, jb), only carries k1..i4 of level k (the zeros of the
+    // initialisation: nothing else has written these arrays yet) to the next level; below jb that leaves zeros, above
+    // jt nothing reads them.  So the walk starts at jb-1 from zeros and stops at jt.  The next level's operands are
+    // loaded before this level's stores (nvcc does not move a shared load above a shared store).
+    double k1p = 0.0, i2p = 0.0, i3p = 0.0, i4p = 0.0;        // values at k+1
+    const int klo = max(jt, msg + 1);
+    double dz = S(A_DZ, jb - 1), w1 = S(A_W1, jb - 1);
+    for (int k = jb - 1; k >= klo; --k) {
+      const double dzn = S(A_DZ, k - 1), w1n = S(A_W1, k - 1);
+      const double k1 = k1p + w1;
+      const double ihat = 0.5 * (k1p + k1);
+      const double i2 = i2p + ihat * dz;
+      const double idag = 0.5 * (i2p + i2);
+      const double i3 = i3p + idag * dz;
+      const double iprm = 0.5 * (i3p + i3);
+      const double i4 = i4p + iprm * dz;
+      S(A_K1, k) = k1; S(A_I2, k) = i2; S(A_I3, k) = i3; S(A_I4, k) = i4;
+      k1p = k1; i2p = i2; i3p = i3; i4p = i4;
+      dz = dzn; w1 = w1n;
     }
   }
-  hmin = 1.E6;
-  double expdif = 0.0;
-  for (int k = msg + 1; k <= pver; ++k) {
-    const double h = S(A_HMN, k);
-    if (k >= j0 && k <= jb && h <= hmin) { hmin = h; expdif = hmn_mx - hmin; }
-  }
+  PH_MARK(PH_K1);
+  // zm_conv.F90:3444-3450: expdif from the last level of least hmn in [j0, jb]
+  const int khmin = warp_last_argmin(S, A_HMN, max(msg + 1, j0), min(pver, jb), lane);
+  const double expdif = khmin > 0 ? hmn_mx - S(A_HMN, khmin) : 0.0;
   WSYNC();
+  PH_MARK(PH_EXPDIF);
   PAR(k, msg + 2, pver) {
     double expnum = 0.0;
     double k1 = S(A_K1, k);
@@ -221,10 +281,21 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
     }
   }
   WSYNC();
+  PH_MARK(PH_F);
   if (j0 < jb)
     if (S(A_F, j0) < 1.E-6 && S(A_F, j0 + 1) > S(A_F, j0)) j0 = j0 + 1;
-  for (int k = msg + 2; k <= pver; ++k)
-    if (k >= jt && k <= j0) S(A_F, k) = fmax2(S(A_F, k), S(A_F, k - 1));
+  {
+    // running max of f over [max(jt, msg+2), j0], seeded with f one level above; the carried value is the one the
+    // previous level stored, so fmax2 sees the same operands in the same order
+    const int klo = max(jt, msg + 2);
+    double fp = S(A_F, klo - 1), f = S(A_F, klo);
+    for (int k = klo; k <= j0; ++k) {
+      const double fn = S(A_F, k + 1);
+      fp = fmax2(f, fp);
+      S(A_F, k) = fp;
+      f = fn;
+    }
+  }
   const double eps0 = S(A_F, j0);
   WSYNC();
   PAR(k, msg + 1, pver) {           // zm_conv.F90:3500-3518, same assignment order
@@ -235,6 +306,7 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
     S(A_EPS, k) = v;
   }
   WSYNC();
+  PH_MARK(PH_FMAX);
   // updraft mass flux (zm_conv.F90:3550-3571): level parallel (mu(k) does not depend on mu(k+1))
   const double zf_jb = S(A_ZF, jb);
   if (eps0 > 0.0) {
@@ -280,33 +352,43 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
     PAR(k, msg + 1, pver) {
       if (k >= lel && k <= jb - 1 && S(A_W3, k) != 0.0) { S(A_MU, k) = 0.0; S(A_EU, k) = 0.0; S(A_DU, k) = S(A_W4, k); }
     }
+    PH_MARK(PH_MU);
     {
+      // the next level's coefficients are loaded before this level's store
       double hup = S(A_HU, jb);
+      double w3 = S(A_W3, jb - 1), hmn = S(A_HMN, jb - 1), a = S(A_W1, jb - 1), b = S(A_W2, jb - 1);
       for (int k = jb - 1; k >= lel; --k) {
-        hup = (S(A_W3, k) != 0.0) ? S(A_HMN, k) : S(A_W1, k) * hup + S(A_W2, k);
+        const double w3n = S(A_W3, k - 1), hmnn = S(A_HMN, k - 1), an = S(A_W1, k - 1), bn = S(A_W2, k - 1);
+        hup = (w3 != 0.0) ? hmn : a * hup + b;
         S(A_HU, k) = hup;
+        w3 = w3n; hmn = hmnn; a = an; b = bn;
       }
     }
     WSYNC();
+    PH_MARK(PH_HU);
   }
   {
-    bool doit = true;
-    const double totfrz = 0.0;
+    // zm_conv.F90:3600-3618: the first level going up from jb-2 (down to lel-1) where the updraft stops; each level's
+    // test reads only hu, hsthat and mu, so it is evaluated lane == level and the hit nearest jb is kept
     const double hu_jb = S(A_HU, jb);
-    for (int k = jb - 2; k >= lel - 1; --k)
-      if (doit) {
-        const double hu = S(A_HU, k), hst = S(A_HSTHAT, k), muk = S(A_MU, k);
-        if (hu <= hst && S(A_HU, k + 1) > S(A_HSTHAT, k + 1) && muk >= 0.02) {
-          if (hu - hst < -2000.0) { jt = k + 1; doit = false; }
-          else                    { jt = k;     doit = false; }
-        } else if ((hu > hu_jb && totfrz <= 0.0) || muk < 0.02) {
-          jt = k + 1;
-          doit = false;
-        }
-      }
+    int khit = -1;
+    PAR(k, lel - 1, jb - 2) {
+      const double hu = S(A_HU, k), hst = S(A_HSTHAT, k), muk = S(A_MU, k);
+      const bool stop = (hu <= hst && S(A_HU, k + 1) > S(A_HSTHAT, k + 1) && muk >= 0.02) || hu > hu_jb || muk < 0.02;
+      if (stop) khit = k;
+    }
+    khit = warp_max(khit);
+    if (khit >= 0) {
+      const int k = khit;
+      const double hu = S(A_HU, k), hst = S(A_HSTHAT, k), muk = S(A_MU, k);
+      if (hu <= hst && S(A_HU, k + 1) > S(A_HSTHAT, k + 1) && muk >= 0.02) jt = (hu - hst < -2000.0) ? k + 1 : k;
+      else jt = k + 1;
+    }
   }
+  PH_MARK(PH_JT);
   if (eps0 > 0.0) {
-    for (int k = pver; k >= msg + 1; --k) {
+    // cloud-top reset (zm_conv.F90:3620-3634), level parallel: level jt reads mu(jt+1), which no level changes
+    PAR(k, msg + 1, pver) {
       if (k >= lel && k <= jt) {
         S(A_MU, k) = 0.0; S(A_EU, k) = 0.0; S(A_DU, k) = 0.0; S(A_HU, k) = S(A_HMN, k);
       }
@@ -318,6 +400,7 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
     }
   }
   WSYNC();
+  PH_MARK(PH_CLDTOP);
   PlumeIdx R{jt, jlcl, j0, jd};
   if (!FULL) return R;
 
@@ -350,16 +433,22 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
       }
     }
     WSYNC();
+    PH_MARK(PH_SUQU_PREP);
     {
+      // the next level's coefficients are loaded before this level's stores
       double sup = S(A_SU, jb), qup = S(A_QU, jb);
-      for (int k = jb - 1; k > jt && k >= msg + 2; --k) {
-        const double a = S(A_W3, k);
-        sup = a * sup + S(A_W4, k);
-        qup = a * qup + S(A_W5, k);
+      const int klo = max(jt + 1, msg + 2);
+      double a = S(A_W3, jb - 1), bs = S(A_W4, jb - 1), bq = S(A_W5, jb - 1);
+      for (int k = jb - 1; k >= klo; --k) {
+        const double an = S(A_W3, k - 1), bsn = S(A_W4, k - 1), bqn = S(A_W5, k - 1);
+        sup = a * sup + bs;
+        qup = a * qup + bq;
         S(A_W1, k) = sup; S(A_W2, k) = qup;
+        a = an; bs = bsn; bq = bqn;
       }
     }
     WSYNC();
+    PH_MARK(PH_SUQU);
     int kfirst = 0;      // highest k (first met going up from jb-1) with qu >= qstu
     PAR(k, msg + 2, pver) {
       bool sat = false;
@@ -402,6 +491,7 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
     }
     WSYNC();
   }
+  PH_MARK(PH_SAT_CU);
   // rain production (zm_conv.F90:3846-3870), serial
   double totpcp = 0.0, totevp = 0.0;
   PAR(k, msg + 2, pver) {
@@ -418,24 +508,39 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
     }
   }
   WSYNC();
-  {
-    double qlp = S(A_QL, pver + 1);
-    for (int k = pver; k >= msg + 2; --k) {
-      if (k >= jt && k < jb && eps0 > 0.0 && S(A_MU, k) >= 0.0) {
+  PH_MARK(PH_QL_PREP);
+  if (eps0 > 0.0) {
+    // The reference walks k = pver .. msg+2; a level outside [jt, jb) or with mu < 0 only carries ql(k), a zero of the
+    // initialisation (this loop is the only writer of ql), to the next level.  So the walk starts at jb-1 from zero,
+    // stops at jt and carries zero past a level with mu < 0.  mu and the coefficients of the next level are loaded
+    // before this level's store.
+    double qlp = 0.0;
+    const int khi = min(pver, jb - 1), klo = max(jt, msg + 2);
+    double mup = S(A_MU, khi + 1), mu = S(A_MU, khi);
+    double w1 = S(A_W1, khi), w2 = S(A_W2, khi), w3 = S(A_W3, khi), w4 = S(A_W4, khi), w5 = S(A_W5, khi);
+    for (int k = khi; k >= klo; --k) {
+      const double mun = S(A_MU, k - 1);
+      const double w1n = S(A_W1, k - 1), w2n = S(A_W2, k - 1), w3n = S(A_W3, k - 1), w4n = S(A_W4, k - 1),
+                   w5n = S(A_W5, k - 1);
+      const double dz = S(A_DZ, k), cu = S(A_CU, k), du = S(A_DU, k);
+      if (mu >= 0.0) {
         double ql = 0.0;
-        if (S(A_MU, k) > 0.0) {
-          const double ql1 = S(A_W1, k) * (S(A_MU, k + 1) * qlp - S(A_W2, k) * qlp + S(A_W3, k));
-          ql = zmm::div_rcp(ql1, S(A_W4, k), S(A_W5, k));    // == ql1 / (1 + dz*c0mask)
+        if (mu > 0.0) {
+          const double ql1 = w1 * (mup * qlp - w2 * qlp + w3);
+          ql = zmm::div_rcp(ql1, w4, w5);    // == ql1 / (1 + dz*c0mask)
         }
         S(A_QL, k) = ql;
-        totpcp = totpcp + S(A_DZ, k) * (S(A_CU, k) - S(A_DU, k) * qlp);
+        totpcp = totpcp + dz * (cu - du * qlp);
         qlp = ql;
       } else {
-        qlp = S(A_QL, k);
+        qlp = 0.0;
       }
+      mup = mu; mu = mun;
+      w1 = w1n; w2 = w2n; w3 = w3n; w4 = w4n; w5 = w5n;
     }
   }
   WSYNC();
+  PH_MARK(PH_QL);
   PAR(k, msg + 2, pver) {
     if (k >= jt && k < jb && eps0 > 0.0 && S(A_MU, k) >= 0.0) {
       const double ql = S(A_QL, k);
@@ -498,15 +603,23 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
       }
     }
     WSYNC();
+    PH_MARK(PH_HD_PREP);
     {
-      const int k0 = max(jt, msg + 1);
+      // The reference runs hd down to pver, but below jb nothing reads it (qds, td and sd use hd of [jd, jb] only, and
+      // hd's storage is not read again after the downdraft), so the walk stops at jb.  The next level's operands are
+      // loaded before this level's store.
+      const int k0 = max(jt, msg + 1), khi = min(jb, pver);
       double hdp = S(A_HD, k0 - 1);
-      for (int k = k0; k <= pver; ++k) {
-        hdp = zmm::div_rcp(S(A_MD, k - 1) * hdp - S(A_W1, k), S(A_W2, k), S(A_W3, k));
+      double md = S(A_MD, k0 - 1), w1 = S(A_W1, k0), w2 = S(A_W2, k0), w3 = S(A_W3, k0);
+      for (int k = k0; k <= khi; ++k) {
+        const double mdn = S(A_MD, k), w1n = S(A_W1, k + 1), w2n = S(A_W2, k + 1), w3n = S(A_W3, k + 1);
+        hdp = zmm::div_rcp(md * hdp - w1, w2, w3);
         S(A_HD, k) = hdp;
+        md = mdn; w1 = w1n; w2 = w2n; w3 = w3n;
       }
     }
     WSYNC();
+    PH_MARK(PH_HD);
     if (jd < jb) {
       PAR(k, msg + 2, pver) {
         if (k >= jd && k <= jb) {
@@ -549,12 +662,19 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
       }
     }
     WSYNC();
+    PH_MARK(PH_SD_PREP);
+    // the next level's operands are loaded before this level's store
     double sdp = S(A_SD, k0);
+    double w1 = S(A_W1, k0), md = S(A_MD, k0), w2 = S(A_W2, k0), w4 = S(A_W4, k0);
     for (int k = k0; k < jb; ++k) {
-      sdp = zmm::div_rcp(S(A_W1, k) + S(A_MD, k) * sdp, S(A_W2, k), S(A_W4, k));
+      const double w1n = S(A_W1, k + 1), mdn = S(A_MD, k + 1), w2n = S(A_W2, k + 1), w4n = S(A_W4, k + 1);
+      const double w3 = S(A_W3, k);
+      sdp = zmm::div_rcp(w1 + md * sdp, w2, w4);
       S(A_SD, k + 1) = sdp;
-      totevp = totevp - S(A_W3, k);
+      totevp = totevp - w3;
+      w1 = w1n; md = mdn; w2 = w2n; w4 = w4n;
     }
+    PH_MARK(PH_SD);
   }
   totevp = totevp + S(A_MD, jd) * S(A_QD, jd) - S(A_MD, jb) * S(A_QD, jb);
   totpcp = fmax2(totpcp, 0.0);
@@ -581,10 +701,17 @@ __device__ __forceinline__ PlumeIdx cldprp_warp(const PlumeSh& S, int jb, int le
     WSYNC();
     double pf = 0.0;
     S(A_PFLX, 1) = 0.0;
-    for (int k = 2; k <= pverp; ++k) { pf = pf + S(A_W1, k - 1); S(A_PFLX, k) = pf; }
+    double w = S(A_W1, 1);
+    for (int k = 2; k <= pverp; ++k) {
+      const double wn = S(A_W1, k);           // loaded before this level's store
+      pf = pf + w;
+      S(A_PFLX, k) = pf;
+      w = wn;
+    }
   }
   PAR(k, msg + 1, pver) S(A_MC, k) = S(A_MU, k) + S(A_MD, k);
   WSYNC();
+  PH_MARK(PH_PFLX);
   R.jt = jt; R.j0 = j0; R.jlcl = jlcl; R.jd = jd;
   return R;
 }
@@ -621,8 +748,12 @@ k_cldprp_pass1_w(ConvrIn in, ConvrWork w) {
   const int c = col / pcols, i = col - c * pcols;
   const PlumeShT<LD> S{sm_pl + (size_t)wib * A_FRONT_COUNT * LD};     // the front arrays only
   const int maxg = w.mx[col];
+  PH_BEGIN(0);
+  PH_COLUMN();
   gather_column_w(S, in, c, i, maxg, lane);
+  PH_MARK(PH_GATHER);
   cldprp_warp<false>(S, maxg, w.lel[col], in.landfrac[(size_t)c * pcols + i], lane);
+  PH_RESTART();
   double hk = 0.0, dmmx = 0.0, dmsm = 0.0;
   const double orgc = 1.0;
   double dm = -1.0;
@@ -639,6 +770,7 @@ k_cldprp_pass1_w(ConvrIn in, ConvrWork w) {
     dm = dmsm * orgc + dmmx * (1.0 - orgc);
   }
   if (lane == 0) w.dmpdz[col] = dm;
+  PH_MARK(PH_EU_SCAN);
 }
 
 // ---- final plume: cldprp #2 + closure + limiter + q1q2 + scatter + prec -----------------------
@@ -660,8 +792,12 @@ k_plume_w(ConvrIn in, ConvrOut o, ConvrWork w) {
   const int maxg = w.mx[col], lel = w.lel[col], lcl = w.lcl[col];
   const double capeg = w.cape[col], tlg = w.tl[col];
   const double landfrac = in.landfrac[(size_t)c * pcols + i];
+  PH_BEGIN(1);
+  PH_COLUMN();
   const double dsubcld = gather_column_w(S, in, c, i, maxg, lane);
+  PH_MARK(PH_GATHER);
   const PlumeIdx R = cldprp_warp<true>(S, maxg, lel, landfrac, lane);
+  PH_RESTART();
   const int jt = R.jt, mx = maxg;
   const double dmpdz = w.dmpdz[col];
 
@@ -760,6 +896,7 @@ k_plume_w(ConvrIn in, ConvrOut o, ConvrWork w) {
     S(A_PFLX, k + 1) = div_z(S(A_PFLX, k + 1) * mb * 100.0, grav);
   }
   WSYNC();
+  PH_MARK(PH_CLOSURE);
 
   // ---- q1q2_pjr (zm_conv.F90:4262-4421): dsdt -> W1, dqdt -> W2, dl -> W3 ----
   PAR(k, msg + 1, pver) {
@@ -784,6 +921,7 @@ k_plume_w(ConvrIn in, ConvrOut o, ConvrWork w) {
     }
   }
   WSYNC();
+  PH_MARK(PH_Q1Q2);
   // scatter to the ungathered column i of chunk c (zm_conv.F90:1495-1511, 1616-1620)
   PAR(k, msg + 1, pver) {
     const size_t e = cidx(c, k - 1, i, pver);
@@ -831,6 +969,7 @@ k_plume_w(ConvrIn in, ConvrOut o, ConvrWork w) {
     o.jt[(size_t)c * pcols + gi] = jt;
     o.maxg[(size_t)c * pcols + gi] = maxg;
   }
+  PH_MARK(PH_SCATTER);
 }
 #undef PAR
 #undef WSYNC

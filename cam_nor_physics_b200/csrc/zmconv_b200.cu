@@ -1171,6 +1171,20 @@ const char* zm_build_info(void) { return "ZMSRCHASH:" ZM_SOURCE_HASH " sm_100a";
 int zm_set_profiling(int on) { g_profile = on != 0; return 0; }
 long long zm_launch_count(int reset) { long long v = tls_launches; if (reset) tls_launches = 0; return v; }
 
+#ifdef ZM_PLUME_PHASE_CLOCKS
+// Phase cycles of the cloud-model kernels (zm_plume_warp.cuh): out[2][PH_COUNT + 1], summed over the warps since the
+// last reset, the last entry of each row the column count.  Returns PH_COUNT, or -1 when a copy fails.
+int zm_plume_phase_cycles(unsigned long long* out, int reset) {
+  if (cudaDeviceSynchronize() != cudaSuccess) return -1;
+  if (out && cudaMemcpyFromSymbol(out, g_plume_phase, sizeof(g_plume_phase)) != cudaSuccess) return -1;
+  if (reset) {
+    static const unsigned long long zero[2][PH_COUNT + 1] = {};
+    if (cudaMemcpyToSymbol(g_plume_phase, zero, sizeof(zero)) != cudaSuccess) return -1;
+  }
+  return PH_COUNT;
+}
+#endif
+
 int zm_get_kernel_times(int* n, const char** names, float* ms) {
   Workspace& ws = tls_work;
   int cnt = 0;
