@@ -15,11 +15,6 @@
 #include <string>
 #include <mutex>
 #include <chrono>
-#include <thread>
-#include <condition_variable>
-#include <functional>
-#include <atomic>
-#include <deque>
 
 namespace {
 
@@ -155,62 +150,10 @@ thread_local Workspace tls_stage2;   // staging for zm_conv_tend_2_batch
 thread_local long long tls_t2_h2d = 0, tls_t2_d2h = 0;
 thread_local Workspace tls_mirror_ws; // the device pbuf mirror (see PbufMirror)
 
-// Host worker threads of the sparse return path (zero-fill of the caller's dense output arrays while the GPU works,
-// then the scatter of the convective columns' records): ZM_HOST_THREADS, default min(8, hardware threads).
-class HostPool {
- public:
-  explicit HostPool(int n) {
-    for (int i = 0; i < n; ++i) th_.emplace_back([this] { run(); });
-  }
-  ~HostPool() {
-    { std::lock_guard<std::mutex> lk(mu_); stop_ = true; }
-    cv_.notify_all();
-    for (auto& t : th_) t.join();
-  }
-  int size() const { return (int)th_.size(); }
-  void submit(std::function<void()> f) {
-    { std::lock_guard<std::mutex> lk(mu_); q_.push_back(std::move(f)); ++pending_; }
-    cv_.notify_one();
-  }
-  void wait_all() {
-    std::unique_lock<std::mutex> lk(mu_);
-    done_.wait(lk, [this] { return pending_ == 0; });
-  }
- private:
-  void run() {
-    for (;;) {
-      std::function<void()> f;
-      {
-        std::unique_lock<std::mutex> lk(mu_);
-        cv_.wait(lk, [this] { return stop_ || !q_.empty(); });
-        if (stop_ && q_.empty()) return;
-        f = std::move(q_.front()); q_.pop_front();
-      }
-      f();
-      { std::lock_guard<std::mutex> lk(mu_); if (--pending_ == 0) done_.notify_all(); }
-    }
-  }
-  std::vector<std::thread> th_;
-  std::deque<std::function<void()>> q_;
-  std::mutex mu_;
-  std::condition_variable cv_, done_;
-  int pending_ = 0;
-  bool stop_ = false;
-};
-HostPool& host_pool() {
-  static HostPool* pool = [] {
-    int n = 0;
-    if (const char* e = getenv("ZM_HOST_THREADS")) n = atoi(e);
-    if (n <= 0) { n = (int)std::thread::hardware_concurrency(); n = n > 8 ? 8 : (n < 1 ? 1 : n); }
-    return new HostPool(n > 64 ? 64 : n);
-  }();
-  return *pool;
-}
-
-// Sparse return of zm_conv_tend_batch: the 2-D outputs are zero outside the convective columns (zm_conv.F90:559-563,
+// Records of zm_conv_tend_batch_gathered: the 2-D outputs are zero outside the convective columns (zm_conv.F90:559-563,
 // 625-650; zm_conv_evap and momtran add nothing where zm_convr produced no rain and no mass flux), so only the
-// convective columns' levels travel device -> host, as one record per column, and worker threads scatter them into
-// the caller's arrays, which they zero-filled while the GPU was busy.  Field order of a record:
+// convective columns' levels travel device -> host, as one record per column, and the caller scatters them into its
+// arrays in its own chunk loop.  Field order of a record:
 enum { SF_PS, SF_PQ, SF_PU, SF_PV, SF_CME, SF_ZDU, SF_QL, SF_RPRD, SF_EVAP, SF_DLF,     // (pcols,pver), by column
        SF_MCON, SF_PFLX, SF_FP, SF_FS,                                                   // (pcols,pverp), by column
        SF_MU, SF_MD, SF_DU, SF_EU, SF_ED, SF_DP,                                         // (pcols,pver), by gathered slot
@@ -220,7 +163,6 @@ struct SparseFields {
   int off[SF_N];             // offset of the field inside a record (doubles), -1 = absent
   int rec_len;               // doubles per record
 };
-// zm_conv_tend_batch_gathered: the same records go straight to the caller, who scatters them in its own chunk loop
 struct GatheredOut {
   double* rec;               // caller's record buffer (capacity checked by the entry point)
   bool pbuf;                 // the slot-indexed pbuf fields mu..dp are part of the records
@@ -267,25 +209,9 @@ struct TendPipe {
   cudaStream_t h2d = nullptr, d2h_early = nullptr, d2h_final = nullptr;
   cudaEvent_t in_ready[MAXB] = {}, late_ready[MAXB] = {}, convr_done[MAXB] = {}, done[MAXB] = {};
   cudaEvent_t early_back[MAXB] = {}, final_back[MAXB] = {}, t0 = nullptr;   // timeline of the last call (zm_tend_trace)
-  int ninit = 0, last_nb = 0, dev_nb = 0;
-  // sparse return: pinned host staging of the records and of the per-sub-batch (lengath, ideep, count) triple
-  cudaEvent_t small_back[MAXB] = {}, rec_back[MAXB] = {};
-  double* h_rec = nullptr; size_t h_rec_cap = 0;       // doubles
-  int* h_small = nullptr; size_t h_small_cap = 0;      // ints
+  int ninit = 0, last_nb = 0;
+  cudaEvent_t small_back[MAXB] = {};                   // gathered return: a sub-batch's lengath is on the host
   long long last_h2d = 0, last_d2h = 0;                // bytes moved by the last call (zm_tend_transfer_bytes)
-  int ensure_pinned(size_t rec_doubles, size_t small_ints) {
-    if (rec_doubles > h_rec_cap) {
-      if (h_rec) { CK(cudaDeviceSynchronize()); CK(cudaFreeHost(h_rec)); h_rec = nullptr; }
-      h_rec_cap = rec_doubles + (rec_doubles >> 2) + 1024;
-      CK(cudaHostAlloc((void**)&h_rec, h_rec_cap * sizeof(double), cudaHostAllocDefault));
-    }
-    if (small_ints > h_small_cap) {
-      if (h_small) { CK(cudaDeviceSynchronize()); CK(cudaFreeHost(h_small)); h_small = nullptr; }
-      h_small_cap = small_ints + 1024;
-      CK(cudaHostAlloc((void**)&h_small, h_small_cap * sizeof(int), cudaHostAllocDefault));
-    }
-    return 0;
-  }
   // ZM_TEND_SUBBATCHES (1..8, default 8); a sub-batch is never smaller than 128 chunks
   int subbatches(int nchunks) const {
     int nb = 8;
@@ -338,11 +264,9 @@ struct TendPipe {
     for (int b = 0; b < ninit; ++b) {
       cudaEventDestroy(in_ready[b]); cudaEventDestroy(late_ready[b]); cudaEventDestroy(convr_done[b]);
       cudaEventDestroy(done[b]); cudaEventDestroy(early_back[b]); cudaEventDestroy(final_back[b]);
-      cudaEventDestroy(small_back[b]); cudaEventDestroy(rec_back[b]);
+      cudaEventDestroy(small_back[b]);
     }
-    if (h_rec) { cudaFreeHost(h_rec); h_rec = nullptr; h_rec_cap = 0; }
-    if (h_small) { cudaFreeHost(h_small); h_small = nullptr; h_small_cap = 0; }
-    ninit = 0; last_nb = 0; dev_nb = 0;
+    ninit = 0; last_nb = 0;
     if (t0) { cudaEventDestroy(t0); t0 = nullptr; }
     if (h2d) { cudaStreamDestroy(h2d); cudaStreamDestroy(d2h_early); cudaStreamDestroy(d2h_final); h2d = d2h_early = d2h_final = nullptr; }
   }
@@ -361,7 +285,6 @@ struct TendPipe {
       CK(cudaEventCreate(&early_back[ninit]));
       CK(cudaEventCreate(&final_back[ninit]));
       CK(cudaEventCreateWithFlags(&small_back[ninit], cudaEventDisableTiming));
-      CK(cudaEventCreateWithFlags(&rec_back[ninit], cudaEventDisableTiming));
       // earlier sub-batches get higher stream priority: the first results reach the return stream sooner
       int lo = 0, hi = 0;
       CK(cudaDeviceGetStreamPriorityRange(&lo, &hi));       // hi = greatest priority (numerically lowest)
@@ -822,35 +745,28 @@ __global__ void k_state_update(int n2, int nper, const double* t, const double* 
     }
   }
 }
-// ptend_all = sum of the three ptend_loc (physics_ptend_sum, physics_types.F90:698-844) and, unless the plume kernel
-// has done it (MCON = false), the mcon unit conversion mb/s -> kg/m2/s (zm_conv_intr.F90:693).
-// MODE 0: cam3, no momentum transport (zm_conv_intr.F90:808); 1: wind tendencies unpacked from wind_tends(pcols,pver,2);
-// 2: momtran has written ptend_u / ptend_v itself (split wind arrays).  evapcdp == ev_q when zm_conv_evap wrote its
-// tend_q straight into the caller's evapcdp.
-template <int MODE, bool MCON>
-__global__ void k_tend_finalize(int n2, int n2p, int nper, const double* heat, const double* qtnd,
+// ptend_all = sum of the three ptend_loc (physics_ptend_sum, physics_types.F90:698-844) in the packed glue form (mcon
+// has left the plume kernel in kg/m2/s already).  MODE 0: cam3, no momentum transport (zm_conv_intr.F90:808);
+// 1: wind tendencies unpacked from wind_tends(pcols,pver,2).  evapcdp == ev_q when zm_conv_evap wrote its tend_q
+// straight into the caller's evapcdp.
+template <int MODE>
+__global__ void k_tend_finalize(int n2, int nper, const double* heat, const double* qtnd,
                                 const double* ev_s, const double* ev_q, const double* seten,
                                 const double* wtend, double* ps, double* pq, double* pu, double* pv,
-                                double* evapcdp, double* mcon) {
-  const int n = MCON ? n2p : n2;
-  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) {
-    if (MCON) mcon[e] = div_z(mcon[e] * 100.0, P.gravit);
-    if (e < n2) {
-      const double evq = ev_q[e];
-      pq[e] = qtnd[e] + evq;
-      if (MODE) {
-        ps[e] = (heat[e] + ev_s[e]) + seten[e];
-        if (MODE == 1) {
-          int c = e / nper, r = e - c * nper;
-          pu[e] = wtend[(size_t)c * 2 * nper + r];
-          pv[e] = wtend[(size_t)c * 2 * nper + nper + r];
-        }
-      } else {
-        ps[e] = heat[e] + ev_s[e];
-        pu[e] = 0.0; pv[e] = 0.0;
-      }
-      if (evapcdp != ev_q) evapcdp[e] = evq;
+                                double* evapcdp) {
+  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n2; e += gridDim.x * blockDim.x) {
+    const double evq = ev_q[e];
+    pq[e] = qtnd[e] + evq;
+    if (MODE) {
+      ps[e] = (heat[e] + ev_s[e]) + seten[e];
+      int c = e / nper, r = e - c * nper;
+      pu[e] = wtend[(size_t)c * 2 * nper + r];
+      pv[e] = wtend[(size_t)c * 2 * nper + nper + r];
+    } else {
+      ps[e] = heat[e] + ev_s[e];
+      pu[e] = 0.0; pv[e] = 0.0;
     }
+    if (evapcdp != ev_q) evapcdp[e] = evq;
   }
 }
 
@@ -1229,19 +1145,7 @@ int zm_get_timers(int* n, const char** names, float* ms) {
 
 // sync the thread's stream and return the Brent failure count of the last zm_convr_batch_dev
 int zm_sync_check(void* stream) {
-  cudaStream_t s = (cudaStream_t)stream;      // NULL = the CUDA default stream
-  TendPipe& tp = tls_pipe;
-  if (tp.dev_nb > 1) {                        // last device call ran as sub-batches on the library's own streams
-    CK(cudaStreamSynchronize(s));
-    int fails = 0;
-    for (int b = tp.dev_nb - 1; b >= 0; --b) {
-      const int f = read_failures(tp.work[b], tp.work[b].stream);
-      if (f < 0) return f;
-      fails += f;
-    }
-    return fails;
-  }
-  return read_failures(tls_work, s);
+  return read_failures(tls_work, (cudaStream_t)stream);      // NULL = the CUDA default stream
 }
 
 int zm_convr_batch_dev(int nchunks, const int* ncol, const double* t, const double* qh, double* prec,
@@ -1258,7 +1162,6 @@ int zm_convr_batch_dev(int nchunks, const int* ncol, const double* t, const doub
   if (nchunks <= 0) return 0;
   Workspace& ws = tls_work;
   if (ws.ensure(0)) return -100;
-  tls_pipe.dev_nb = 0;
   cudaStream_t s = (cudaStream_t)stream;      // NULL = the CUDA default stream
   ConvrIn in{nchunks, ncol, t, qh, pap, paph, dpp, zm, zi, geos, pblh, tpert, landfrac, delt};
   ConvrOut o{prec, jctop, jcbot, qtnd, heat, mcon, cme, cape, eurt, dlf, pflx, zdu, rprd,
@@ -1476,7 +1379,7 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
   NEED_INIT();
   if (nchunks <= 0) return 0;
   const size_t pc = g_params.pcols, L = g_params.pver, nc = (size_t)nchunks * pc;
-  const size_t n2 = nc * L, n2p = nc * (L + 1);
+  const size_t n2 = nc * L;
   const HistFields H = hist ? *hist : HistFields{};
   if (ws.ensure(convr_work_bytes(nc, (int)L) + 19 * al(n2, 8) + 6 * al(2 * n2, 8) + chunk_bounds_bytes(nchunks, (int)nc) + 8192 +
                 (H.any() ? 4 * al(n2, 8) + 4 * al(2 * n2, 8) : 0)))
@@ -1504,14 +1407,17 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
   // zm_conv_evap's tend_q IS evapcdp (zm_conv_intr.F90:764-769 passes ptend_loc%q(:,:,1), :796 outputs it): written in place
   double* ev_q = evapcdp ? evapcdp : ev_q_scratch;
   const bool do_mom = !g_params.cam3;          // zm_conv_intr.F90:808: momentum transport is non-cam3 physics
-  // momtran reads state%u / state%v and writes ptend_u / ptend_v directly when they can take 16-byte stores
-  const bool split_env = !(getenv("ZM_TEND_SPLIT_WINDS") && atoi(getenv("ZM_TEND_SPLIT_WINDS")) == 0);   // 0: round-2a glue
-  const bool split = split_env && do_mom && !(n2 & 1) &&
-                     (((uintptr_t)ptend_u | (uintptr_t)ptend_v | (uintptr_t)seten) & 15) == 0;
+  // Glue form, chosen from what the call shows.  Split (fast): momtran reads state%u / state%v and writes ptend_u /
+  // ptend_v itself, zm_conv_evap stores the summed tendencies, k_add_seten adds seten.  Its zero-fills and k_add_seten
+  // make 16-byte stores, so it needs momtran (not cam3), an even pcols*pver and 16-byte aligned ptend_u, ptend_v, seten
+  // and ptend_s.  Packed otherwise: state update, momtran on winds(pcols,pver,2) and k_tend_finalize
+  // (zm_conv_intr.F90:814-833).
+  const bool split = do_mom && !(n2 & 1) &&
+                     (((uintptr_t)ptend_u | (uintptr_t)ptend_v | (uintptr_t)seten | (uintptr_t)ptend_s) & 15) == 0;
   ConvrIn in{nchunks, ncol, t, q, pmid, pint, pdel, zm, zi, phis, pblh, tpert, landfrac, 0.5 * ztodt};
   ConvrOut o{prec, jctop, jcbot, qtnd, heat, mcon, cme, cape, eurt, dlf, pflx, zdu, rprd,
              mu, md, du, eu, ed, dp, dsubcld, jt, maxg, ideep, lengath, ql, rliq, dif, dnlf, dnif, rice};
-  o.mcon_kgm2s = split_env ? 1 : 0;            // unit conversion of zm_conv_intr.F90:693 inside the plume kernel
+  o.mcon_kgm2s = 1;                            // unit conversion of zm_conv_intr.F90:693 inside the plume kernel
   in.org = g_params.zm_org ? org : nullptr;
   // split winds: ptend_u / ptend_v / seten are zero outside the convective columns momtran writes -- filled with
   // zm_convr's own outputs at the start of the step
@@ -1540,10 +1446,8 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
   const bool fork = !g_profile;
   // With the split winds nothing but zm_conv_evap needs the updated state: the kernel applies physics_update to its
   // own operands and stores heat + tend_s / qtnd + tend_q straight into ptend_s / ptend_q (k_conv_evap<true>); what is
-  // left for the end of the step is ptend_s += seten.  ZM_TEND_FUSE_EVAP=0: separate state update and final sum.
-  const bool fuse_evap = split && o.mcon_kgm2s && (((uintptr_t)ptend_s) & 15) == 0 &&
-                         !(getenv("ZM_TEND_FUSE_EVAP") && atoi(getenv("ZM_TEND_FUSE_EVAP")) == 0);
-  if (fuse_evap) {     // tend_s stays: k_conv_evap<true, true> also stores it and the four snow diagnostics
+  // left for the end of the step is ptend_s += seten.
+  if (split) {         // tend_s stays: k_conv_evap<true, true> also stores it and the four snow diagnostics
     ea.t = t; ea.q = q; ea.heat = heat; ea.qtnd = qtnd; ea.ps = ptend_s; ea.pq = ptend_q;
     if (!hist_evap) ea.tend_s = nullptr;
   }
@@ -1551,15 +1455,15 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
     if (ws.ensure_side()) return -100;
     CK(cudaEventRecord(ws.ev_fork, s));
     CK(cudaStreamWaitEvent(ws.side, ws.ev_fork, 0));
-    if (!fuse_evap) {
+    if (!split) {
       k_state_update<1><<<1184, 256, 0, ws.side>>>((int)n2, nper, t, q, heat, qtnd, u, v, ztodt, t1, q1, winds);
       ++tls_launches;
+      if (do_mom) {             // packed winds feed momtran only
+        k_state_update<2><<<1184, 256, 0, s>>>((int)n2, nper, t, q, heat, qtnd, u, v, ztodt, t1, q1, winds);
+        ++tls_launches;
+      }
     }
-    if (do_mom && !split) {     // packed winds feed momtran only
-      k_state_update<2><<<1184, 256, 0, s>>>((int)n2, nper, t, q, heat, qtnd, u, v, ztodt, t1, q1, winds);
-      ++tls_launches;
-    }
-  } else if (!fuse_evap) {
+  } else if (!split) {
     k_state_update<0><<<1184, 256, 0, s>>>((int)n2, nper, t, q, heat, qtnd, u, v, ztodt, t1, q1, winds);
     ++tls_launches;
   }
@@ -1616,14 +1520,12 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
   }
   if (tran_stream != s) CK(cudaStreamWaitEvent(s, ws.ev_join2, 0));
   if (fork) CK(cudaStreamWaitEvent(s, ws.ev_join, 0));
-  if (fuse_evap) {
+  if (split) {
     k_add_seten<<<1184, 256, 0, s>>>(n2 / 2, (double2*)ptend_s, (const double2*)seten);
   } else {
-    auto fin = !do_mom ? (o.mcon_kgm2s ? k_tend_finalize<0, false> : k_tend_finalize<0, true>)
-               : split ? (o.mcon_kgm2s ? k_tend_finalize<2, false> : k_tend_finalize<2, true>)
-                       : (o.mcon_kgm2s ? k_tend_finalize<1, false> : k_tend_finalize<1, true>);
-    fin<<<1184, 256, 0, s>>>((int)n2, (int)n2p, nper, heat, qtnd, ev_s, ev_q, seten, wtend, ptend_s, ptend_q, ptend_u,
-                             ptend_v, evapcdp ? evapcdp : ev_q, mcon);
+    auto fin = do_mom ? k_tend_finalize<1> : k_tend_finalize<0>;
+    fin<<<1184, 256, 0, s>>>((int)n2, nper, heat, qtnd, ev_s, ev_q, seten, wtend, ptend_s, ptend_q, ptend_u, ptend_v,
+                             evapcdp ? evapcdp : ev_q);
   }
   ++tls_launches;
   tick(ws, s, "tend_finalize");
@@ -1645,15 +1547,6 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
                            int* jt, int* maxg, int* ideep, int* lengath, double* cape, void* stream) {
   NEED_INIT();
   if (nchunks <= 0) return 0;
-  // Optionally cut the batch into sub-batches of whole chunks that run on their own (prioritised) streams:
-  // every kernel of the path is latency-bound at low occupancy, so the passes of different sub-batches
-  // fill each other's idle issue slots.  ZM_DEV_SUBBATCHES = 1 keeps everything on `stream`.
-  TendPipe& tp = tls_pipe;
-  int NB = 1;
-  if (const char* e = getenv("ZM_DEV_SUBBATCHES")) NB = atoi(e);
-  NB = NB < 1 ? 1 : (NB > TendPipe::MAXB ? TendPipe::MAXB : NB);
-  while (NB > 1 && nchunks / NB < 128) --NB;
-  tp.dev_nb = 0;
   const OrgFields of = tls_org; tls_org = OrgFields{};       // one-shot
   const Tran1Fields tf = tls_tran1; tls_tran1 = Tran1Fields{};   // one-shot
   const HistFields hf = tls_hist; tls_hist = HistFields{};       // one-shot
@@ -1666,91 +1559,54 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
     td = Tran1Dev{n, tls_tmeta1.nactive, tls_tmeta1.active(), tls_tmeta1.dry(), tls_tmeta1.any_dry, tf.q, tf.fracis, tf.ptend_q};
     tdp = &td;
   }
-  if (NB == 1 || g_profile) {
-    auto direct = [&](Workspace& ws, void* on) {
-      return conv_tend_impl(ws, nchunks, ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, tpert, landfrac,
-                            cld, ztodt, ptend_s, ptend_q, ptend_u, ptend_v, mcon, cme, pflx, zdu, rliq, rice, jctop,
-                            jcbot, prec, snow, ql, rprd, evapcdp, flxprec, flxsnow, dlf, mu, md, du, eu, ed, dp,
-                            dsubcld, jt, maxg, ideep, lengath, cape, on, nullptr, of.org, of.orgt, of.org2d, tdp, hfp);
-    };
-    static const bool use_graph = !(getenv("ZM_DEV_GRAPH") && atoi(getenv("ZM_DEV_GRAPH")) == 0);
-    if (g_profile || !use_graph) { tls_graph.clear(); return direct(tls_work, stream); }
-    Workspace& ws = tls_work;
-    TendGraph& G = tls_graph;
-    double zt = ztodt; const void* ztbits; std::memcpy(&ztbits, &zt, sizeof ztbits);
-    std::vector<const void*> key = {ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, tpert, landfrac, cld,
-        ptend_s, ptend_q, ptend_u, ptend_v, mcon, cme, pflx, zdu, rliq, rice, jctop, jcbot, prec, snow, ql, rprd,
-        evapcdp, flxprec, flxsnow, dlf, mu, md, du, eu, ed, dp, dsubcld, jt, maxg, ideep, lengath, cape,
-        of.org, of.orgt, of.org2d, ztbits, (const void*)(size_t)nchunks, (const void*)(size_t)g_epoch,
-        tf.q, tf.fracis, tf.ptend_q, (const void*)(size_t)tf.pcnst, (const void*)tls_tmeta1.d,
-        (const void*)(size_t)(tdp ? tls_tmeta1.version : 0)};
-    // attached history fields: a replay must write where this call asked, and attaching or detaching recaptures
-    key.insert(key.end(), hf.p, hf.p + H_N);
-    key.push_back((const void*)ws.dbuf); key.push_back((const void*)ws.dcap);
-    cudaStream_t s = (cudaStream_t)stream;
-    if (key == G.key) {
-      if (!G.exec) {                                   // second identical call: capture on the library's own stream
-        cudaGraph_t graph = nullptr;
-        const long long l0 = tls_launches;
-        bool ok = ws.stream && cudaStreamBeginCapture(ws.stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
-        if (ok) {
-          const int rc = direct(ws, (void*)ws.stream);
-          const cudaError_t ee = cudaStreamEndCapture(ws.stream, &graph);
-          ok = rc == 0 && ee == cudaSuccess && graph && cudaGraphInstantiate(&G.exec, graph, 0) == cudaSuccess;
-          if (graph) cudaGraphDestroy(graph);
-        }
-        G.launches = tls_launches - l0;
-        tls_launches = l0;                             // captured launches did not run
-        if (!ok) { cudaGetLastError(); G.clear(); return direct(ws, stream); }
-      }
-      CK(cudaGraphLaunch(G.exec, s));
-      tls_launches += G.launches;
-      return 0;
-    }
-    G.clear();
-    const int rc = direct(ws, stream);                 // first call with these arguments: run, remember
-    if (rc == 0) {
-      G.key = key;
-      G.key[G.key.size() - 2] = (const void*)ws.dbuf;  // the arena may have been (re)allocated by this call
-      G.key[G.key.size() - 1] = (const void*)ws.dcap;
-    }
-    return rc;
-  }
-  if (tp.init(NB)) return -100;
+  auto direct = [&](Workspace& ws, void* on) {
+    return conv_tend_impl(ws, nchunks, ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, tpert, landfrac,
+                          cld, ztodt, ptend_s, ptend_q, ptend_u, ptend_v, mcon, cme, pflx, zdu, rliq, rice, jctop,
+                          jcbot, prec, snow, ql, rprd, evapcdp, flxprec, flxsnow, dlf, mu, md, du, eu, ed, dp,
+                          dsubcld, jt, maxg, ideep, lengath, cape, on, nullptr, of.org, of.orgt, of.org2d, tdp, hfp);
+  };
+  static const bool use_graph = !(getenv("ZM_DEV_GRAPH") && atoi(getenv("ZM_DEV_GRAPH")) == 0);
+  if (g_profile || !use_graph) { tls_graph.clear(); return direct(tls_work, stream); }
+  Workspace& ws = tls_work;
+  TendGraph& G = tls_graph;
+  double zt = ztodt; const void* ztbits; std::memcpy(&ztbits, &zt, sizeof ztbits);
+  std::vector<const void*> key = {ncol, t, q, u, v, pmid, pint, pdel, zm, zi, phis, pblh, tpert, landfrac, cld,
+      ptend_s, ptend_q, ptend_u, ptend_v, mcon, cme, pflx, zdu, rliq, rice, jctop, jcbot, prec, snow, ql, rprd,
+      evapcdp, flxprec, flxsnow, dlf, mu, md, du, eu, ed, dp, dsubcld, jt, maxg, ideep, lengath, cape,
+      of.org, of.orgt, of.org2d, ztbits, (const void*)(size_t)nchunks, (const void*)(size_t)g_epoch,
+      tf.q, tf.fracis, tf.ptend_q, (const void*)(size_t)tf.pcnst, (const void*)tls_tmeta1.d,
+      (const void*)(size_t)(tdp ? tls_tmeta1.version : 0)};
+  // attached history fields: a replay must write where this call asked, and attaching or detaching recaptures
+  key.insert(key.end(), hf.p, hf.p + H_N);
+  key.push_back((const void*)ws.dbuf); key.push_back((const void*)ws.dcap);
   cudaStream_t s = (cudaStream_t)stream;
-  const size_t pc = g_params.pcols, L = g_params.pver, s2 = pc * L, s2p = pc * (L + 1), s1 = pc;
-  CK(cudaEventRecord(tp.in_ready[0], s));
-  for (int b = 0; b < NB; ++b) {
-    const int c0 = tp.first(b, nchunks, NB), nb = tp.first(b + 1, nchunks, NB) - c0;
-    Workspace& ws = tp.work[b];
-    ws.chunk0 = c0;
-    CK(cudaStreamWaitEvent(ws.stream, tp.in_ready[0], 0));
-    Tran1Dev tb = td;            // this sub-batch's slice of the constituent arrays
-    if (tdp) {
-      const size_t o3 = (size_t)c0 * s2 * td.ncnst;
-      tb.q = td.q + o3; tb.fracis = td.fracis + o3; tb.dqdt = td.dqdt + o3;
+  if (key == G.key) {
+    if (!G.exec) {                                   // second identical call: capture on the library's own stream
+      cudaGraph_t graph = nullptr;
+      const long long l0 = tls_launches;
+      bool ok = ws.stream && cudaStreamBeginCapture(ws.stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
+      if (ok) {
+        const int rc = direct(ws, (void*)ws.stream);
+        const cudaError_t ee = cudaStreamEndCapture(ws.stream, &graph);
+        ok = rc == 0 && ee == cudaSuccess && graph && cudaGraphInstantiate(&G.exec, graph, 0) == cudaSuccess;
+        if (graph) cudaGraphDestroy(graph);
+      }
+      G.launches = tls_launches - l0;
+      tls_launches = l0;                             // captured launches did not run
+      if (!ok) { cudaGetLastError(); G.clear(); return direct(ws, stream); }
     }
-    const HistFields hb = hf.slice(c0, s2);
-#define O2(x)  ((x) + (size_t)c0 * s2)
-#define O2P(x) ((x) + (size_t)c0 * s2p)
-#define O1(x)  ((x) + (size_t)c0 * s1)
-    int rc = conv_tend_impl(ws, nb, ncol + c0, O2(t), O2(q), O2(u), O2(v), O2(pmid), O2P(pint), O2(pdel), O2(zm),
-                            O2P(zi), O1(phis), O1(pblh), O1(tpert), O1(landfrac), O2(cld), ztodt, O2(ptend_s),
-                            O2(ptend_q), O2(ptend_u), O2(ptend_v), O2P(mcon), O2(cme), O2P(pflx), O2(zdu), O1(rliq),
-                            O1(rice), O1(jctop), O1(jcbot), O1(prec), O1(snow), O2(ql), O2(rprd), O2(evapcdp),
-                            O2P(flxprec), O2P(flxsnow), O2(dlf), O2(mu), O2(md), O2(du), O2(eu), O2(ed), O2(dp),
-                            O1(dsubcld), O1(jt), O1(maxg), O1(ideep), lengath + c0, O1(cape), (void*)ws.stream, nullptr,
-                            of.org ? O2(of.org) : nullptr, of.orgt ? O2(of.orgt) : nullptr,
-                            of.org2d ? O2(of.org2d) : nullptr, tdp ? &tb : nullptr, hfp ? &hb : nullptr);
-#undef O2
-#undef O2P
-#undef O1
-    if (rc) return rc;
-    CK(cudaEventRecord(tp.done[b], ws.stream));
-    CK(cudaStreamWaitEvent(s, tp.done[b], 0));
+    CK(cudaGraphLaunch(G.exec, s));
+    tls_launches += G.launches;
+    return 0;
   }
-  tp.dev_nb = NB;
-  return 0;
+  G.clear();
+  const int rc = direct(ws, stream);                 // first call with these arguments: run, remember
+  if (rc == 0) {
+    G.key = key;
+    G.key[G.key.size() - 2] = (const void*)ws.dbuf;  // the arena may have been (re)allocated by this call
+    G.key[G.key.size() - 1] = (const void*)ws.dcap;
+  }
+  return rc;
 }
 
 // The host-pointer step behind zm_conv_tend_batch (g == NULL) and zm_conv_tend_batch_gathered (g != NULL: the
@@ -1795,29 +1651,13 @@ static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const 
   // whole batch (4: in, before the first sub-batch; 5: out, after the last) instead of once per sub-batch
   struct Arr { const void* h; void* d; size_t stride, esz; int kind; };
   std::vector<Arr> arrs; arrs.reserve(64);
-  // Return path of the 2-D outputs: dense (default) copies the arrays whole; ZM_TEND_RETURN=sparse moves only the
-  // convective columns' records and scatters them on the host into the arrays worker threads zero-filled meanwhile.
-  // The sparse path moves a third of the bytes over PCIe but writes the caller's arrays with CPU stores, and on a
-  // host whose memory bandwidth is of the order of the PCIe rate (the B200 boxes of this project: 70-78 GB/s for a
-  // parallel memset against 56 GB/s D2H) that costs more than it saves -- measured 11.7 against 8.2 ms per f09 step
-  // (DESIGN.md section 5) -- so it is opt-in, for hosts with memory bandwidth to spare.
-  // ZM_TEND_OUTPUTS_PREZEROED=1: the caller's arrays are all-zero on entry (as after physics_ptend_init), the
-  // zero-fill is skipped.  The gathered entry point ignores ZM_TEND_RETURN: its records are its return path.
-  const char* ret_env = getenv("ZM_TEND_RETURN");
-  const bool sparse = !g && ret_env && !strcmp(ret_env, "sparse");
-  const bool prezeroed = getenv("ZM_TEND_OUTPUTS_PREZEROED") && atoi(getenv("ZM_TEND_OUTPUTS_PREZEROED")) != 0;
-  double* sf_host[SF_N] = {};               // caller's arrays of the sparse fields (NULL: not wanted)
-  double* sf_dev[SF_N] = {};
-  int sf_next = -1;                          // id of the sparse field the next dev() call stages
+  double* sf_dev[SF_N] = {};                 // device arrays of the record fields, packed by the gathered return
+  int sf_next = -1;                          // id of the record field the next dev() call stages
   bool to_mirror = false;                    // the pbuf fields go to the mirror arena
   auto dev = [&](const void* h, size_t stride, size_t esz, int kind, bool always = true) -> void* {
     void* d = (void*)(to_mirror ? mw : st).take<char>((size_t)nchunks * stride * esz);
     if (stride <= pc) kind = (kind <= 1) ? 4 : 5;
-    if (sf_next >= 0) {
-      sf_host[sf_next] = (double*)h; sf_dev[sf_next] = (double*)d;
-      if (sparse && h) kind = 6;             // no dense copy: travels in the records
-      sf_next = -1;
-    }
+    if (sf_next >= 0) { sf_dev[sf_next] = (double*)d; sf_next = -1; }
     if (h || always) arrs.push_back({h, d, stride, esz, h ? kind : -1});
     return d;
   };
@@ -1856,7 +1696,7 @@ static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const 
     }
     d_org = DIN(of.org, s2); d_org2d = DOUTE(of.org2d, s2); d_orgt = DOUTF(of.orgt, s2);
   }
-  // history fields travel whole, also under ZM_TEND_RETURN=sparse: zm_convr's as soon as the plume kernel is done,
+  // history fields travel whole, also with the gathered return: zm_convr's as soon as the plume kernel is done,
   // zm_conv_evap's and momtran's at the end of the sub-batch
   HistFields dh;
   for (int j = 0; j < H_N; ++j)
@@ -1868,20 +1708,18 @@ static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const 
 #undef DOUTF
 #undef SPE
 #undef SPF
-  // sparse return: record layout (fields the caller asked for), device record buffer sized for the worst case so
-  // that a sub-batch's region does not depend on the counts of the others.  gathered: the 14 column-indexed fields,
-  // then the pbuf fields if asked for.
+  // gathered: record layout (the 14 column-indexed fields, then the pbuf fields if asked for), device record buffer
+  // sized for the worst case so that a sub-batch's region does not depend on the counts of the others
   int sf_off[SF_N], rec_len = 0;
   for (int qf = 0; qf < SF_N; ++qf) {
     const int nlev = (qf >= SF_MCON && qf <= SF_FS) ? (int)L + 1 : (int)L;
-    const bool packed = sparse ? sf_host[qf] != nullptr : (g && (qf < SF_MU || g->pbuf));
+    const bool packed = g && (qf < SF_MU || g->pbuf);
     if (packed) { sf_off[qf] = rec_len; rec_len += nlev; } else sf_off[qf] = -1;
   }
   double* d_rec = nullptr; int* d_base = nullptr;
   if (rec_len > 0) {
     d_rec = st.take<double>(nc * rec_len);
     d_base = st.take<int>((size_t)nchunks + TendPipe::MAXB + 1);
-    if (sparse && tp.ensure_pinned(0, 2 * (nc + nchunks + 2 * TendPipe::MAXB))) return -100;
   }
   // convtran1 (zm_conv_intr.F90:865-880): only the slices of the transported constituents travel; on the device
   // they are stored compactly, (pcols,pver,nactive) per chunk
@@ -1929,12 +1767,6 @@ static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const 
     }                                                                                               \
   } while (0)
   long long moved_h2d = 0, moved_d2h = 0;
-  // zero-fill of the caller's arrays of the sparse fields by the worker threads, one counter per sub-batch
-  HostPool* pool = (sparse && rec_len > 0) ? &host_pool() : nullptr;
-  std::atomic<int> zero_left[TendPipe::MAXB];
-  for (auto& z : zero_left) z.store(0);
-  // anything that returns early must not leave worker tasks (which write the caller's arrays) behind
-  struct PoolGuard { HostPool* p; ~PoolGuard() { if (p) p->wait_all(); } } pool_guard{pool};
   auto copy_kind = [&](int kind, int c0, int nb, cudaStream_t on) {
     for (auto& a : arrs) {
       if (a.kind != kind) continue;
@@ -1963,23 +1795,6 @@ static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const 
     CKP(cudaEventRecord(tp.late_ready[b], tp.h2d));
     return 0;
   };
-  if (pool && !prezeroed) {
-    for (int b = 0; b < NB; ++b) {
-      const int c0 = tp.sched_first[b], nb = tp.sched_first[b + 1] - c0;
-      for (int qf = 0; qf < SF_N; ++qf) {
-        if (sf_off[qf] < 0) continue;
-        const size_t str = ((qf >= SF_MCON && qf <= SF_FS) ? s2p : s2);
-        char* base = (char*)(sf_host[qf] + (size_t)c0 * str);
-        const size_t bytes = (size_t)nb * str * 8, piece = 2u << 20;
-        for (size_t o = 0; o < bytes; o += piece) {
-          zero_left[b].fetch_add(1);
-          const size_t n = bytes - o < piece ? bytes - o : piece;
-          std::atomic<int>* cnt = &zero_left[b];
-          pool->submit([base, o, n, cnt] { std::memset(base + o, 0, n); cnt->fetch_sub(1); });
-        }
-      }
-    }
-  }
   CKP(cudaEventRecord(tp.t0, tp.h2d));
   const double w_t0 = wall_ms();
   copy_kind(4, 0, nchunks, tp.h2d);
@@ -2028,15 +1843,6 @@ static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const 
       tls_launches += 2;
     }
     CKP(cudaEventRecord(tp.done[b], ws.stream));
-    if (pool) {         // (count, lengath, ideep) of the sub-batch: what the host needs to size and scatter the records
-      int* hs = tp.h_small + 2 * ((size_t)c0 * pc + c0 + 2 * b);
-      CKP(cudaStreamWaitEvent(tp.d2h_final, tp.done[b], 0));
-      CKP(cudaMemcpyAsync(hs, d_base + c0 + b + nb, sizeof(int), cudaMemcpyDeviceToHost, tp.d2h_final));
-      CKP(cudaMemcpyAsync(hs + 2, d_len + c0, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, tp.d2h_final));
-      CKP(cudaMemcpyAsync(hs + 2 + nb, d_ideep + (size_t)c0 * s1, (size_t)nb * pc * sizeof(int), cudaMemcpyDeviceToHost, tp.d2h_final));
-      CKP(cudaEventRecord(tp.small_back[b], tp.d2h_final));
-      moved_d2h += (long long)(1 + nb + nb * pc) * 4;
-    }
     if (b + 1 < NB && send_inputs(b + 1)) { drain(); return -100; }
     const double w_in = wall_ms();
     // device->host: zm_convr's outputs as soon as they are final, the rest when the sub-batch ends
@@ -2050,70 +1856,6 @@ static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const 
     CKP(cudaEventRecord(tp.final_back[b], tp.d2h_early));
     if (dbg) fprintf(stderr, "  sub-batch %d: kernels enqueued %.3f, next inputs enqueued %.3f, returns enqueued %.3f ms\n",
                      b, w_k, w_in, wall_ms());
-  }
-  if (rc == 0 && pool) {
-    // records: as soon as a sub-batch's count is known its records are fetched (exact size) while the worker threads
-    // scatter the previous sub-batch's
-    size_t hoff = 0;                       // doubles into the pinned record staging
-    size_t rec_off[TendPipe::MAXB]; int rec_cnt[TendPipe::MAXB];
-    auto scatter = [&](int b) {
-      const int c0 = tp.sched_first[b], nb = tp.sched_first[b + 1] - c0;
-      const int* hs = tp.h_small + 2 * ((size_t)c0 * pc + c0 + 2 * b);
-      const int* len = hs + 2; const int* idp = hs + 2 + nb;
-      while (zero_left[b].load() > 0) std::this_thread::yield();
-      const int ntask = pool->size() * 2, total = rec_cnt[b];
-      const double* recs = tp.h_rec + rec_off[b];
-      int ca = 0, j0 = 0;
-      for (int tsk = 0; tsk < ntask && ca < nb; ++tsk) {
-        const int want = (int)(((long long)total * (tsk + 1)) / ntask);
-        int cb = ca, j1 = j0;
-        while (cb < nb && (j1 < want || tsk == ntask - 1)) j1 += len[cb++];
-        if (cb == ca) continue;
-        double* const* hostp = sf_host; const int* offp = sf_off;
-        const int pcl = (int)pc, Ll = (int)L, rl = rec_len;
-        pool->submit([=] {
-          int j = j0;
-          for (int c = ca; c < cb; ++c)
-            for (int slot = 0; slot < len[c]; ++slot, ++j) {
-              const int i = idp[(size_t)c * pcl + slot] - 1;
-              const double* r = recs + (size_t)j * rl;
-              for (int qf = 0; qf < SF_N; ++qf) {
-                if (offp[qf] < 0) continue;
-                const int nlev = (qf >= SF_MCON && qf <= SF_FS) ? Ll + 1 : Ll;
-                double* dst = hostp[qf] + ((size_t)(c0 + c) * nlev) * pcl + (qf >= SF_MU ? slot : i);
-                const double* src = r + offp[qf];
-                for (int k = 0; k < nlev; ++k) dst[(size_t)k * pcl] = src[k];
-              }
-            }
-        });
-        ca = cb; j0 = j1;
-      }
-    };
-    for (int b = 0; b < NB && rc == 0; ++b) {
-      const int c0 = tp.sched_first[b];
-      if (cudaEventSynchronize(tp.small_back[b]) != cudaSuccess) { rc = -100; break; }
-      rec_cnt[b] = tp.h_small[2 * ((size_t)c0 * pc + c0 + 2 * b)];
-      rec_off[b] = hoff;
-      const size_t n = (size_t)rec_cnt[b] * rec_len;
-      if (hoff + n > tp.h_rec_cap) {       // grow the pinned staging: earlier records must be scattered first
-        for (int p2 = 0; p2 < b; ++p2) cudaEventSynchronize(tp.rec_back[p2]);
-        pool->wait_all();
-        if (tp.ensure_pinned(nc * rec_len, 0)) { rc = -100; break; }
-      }
-      if (n && cudaMemcpyAsync(tp.h_rec + hoff, d_rec + (size_t)c0 * pc * rec_len, n * sizeof(double),
-                               cudaMemcpyDeviceToHost, tp.d2h_early) != cudaSuccess) rc = -100;
-      if (cudaEventRecord(tp.rec_back[b], tp.d2h_early) != cudaSuccess) rc = -100;
-      moved_d2h += (long long)n * 8;
-      hoff += n;
-      if (b > 0) {
-        if (cudaEventSynchronize(tp.rec_back[b - 1]) != cudaSuccess) { rc = -100; break; }
-        scatter(b - 1);
-      }
-    }
-    if (rc == 0) {
-      if (cudaEventSynchronize(tp.rec_back[NB - 1]) != cudaSuccess) rc = -100;
-      else scatter(NB - 1);
-    }
   }
   if (rc == 0 && g) {
     // gathered: a sub-batch's lengath comes back as soon as its kernels are done, into the caller's array; its sum is
@@ -2172,7 +1914,6 @@ static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const 
     fails += f;
   }
   if (fails == 0) tls_mirror = new_mirror;   // a failed step (the reference stops in endrun) leaves no mirror
-  if (pool) pool->wait_all();
   tp.last_h2d = moved_h2d; tp.last_d2h = moved_d2h;
   return fails;
 #undef CKP

@@ -139,17 +139,10 @@ int zm_convtran_batch_dev(int nchunks, const int* doconvtran, const double* q, i
  *     equal sub-batches; ZM_TEND_SUBBATCHES=n
  *     (1..8) or ZM_TEND_SCHEDULE=uniform selects equal parts (default 8, never below 128 chunks each);
  *     ZM_TEND_SCHEDULE="1,2,3,4,6" gives explicit sizes in sixteenths; ZM_TEND_DEBUG prints the host-side timing.
- *     Return path of the (pcols,pver[p]) outputs: whole arrays by default.  They are zero outside the convective
- *     columns, so ZM_TEND_RETURN=sparse sends only the convective columns' levels device->host, one record per column,
- *     and ZM_HOST_THREADS worker threads (default min(8, hardware threads)) scatter them into the caller's arrays,
- *     which they zero-filled while the GPU worked; every element of every output is defined on return exactly as in
- *     the dense mode.  A third of the PCIe bytes, three times the host-memory traffic: it pays only on hosts whose
- *     memory bandwidth is well above the PCIe rate (not the case on this project's B200 boxes, where it is slower).
- *     ZM_TEND_OUTPUTS_PREZEROED=1 tells the library the arrays are all-zero on entry (as after physics_ptend_init)
- *     and skips the zero-fill.  Per-column outputs always travel whole.
+ *     Every output array travels whole; zm_conv_tend_batch_gathered returns the (pcols,pver[p]) outputs as the
+ *     convective columns' records instead.
  *   _dev variant: from the third call with an identical argument list on, the step is replayed as a CUDA graph on
- *     `stream` (ZM_DEV_GRAPH=0 disables); ZM_DEV_SUBBATCHES (default 1) optionally splits the step over the
- *     library's own prioritised streams, joined back into `stream`. */
+ *     `stream` (ZM_DEV_GRAPH=0 disables). */
 int zm_conv_tend_batch(int nchunks, const int* ncol, const double* t, const double* q, const double* u,
                        const double* v, const double* pmid, const double* pint, const double* pdel,
                        const double* zm, const double* zi, const double* phis, const double* pblh,
@@ -196,8 +189,7 @@ int zm_conv_tend_batch_dev(int nchunks, const int* ncol, const double* t, const 
  * end, while later sub-batches compute.  The copies into rec are asynchronous when the caller has registered it once
  * with cudaHostRegister.  Everything else -- sub-batch pipelining (ZM_TEND_SUBBATCHES,
  * ZM_TEND_SCHEDULE), the one-shot attachments (their arrays travel whole), the device pbuf mirror (published on
- * success only), zm_tend_trace, zm_tend_transfer_bytes, the Brent-failure return -- is that of zm_conv_tend_batch.
- * ZM_TEND_RETURN does not apply. */
+ * success only), zm_tend_trace, zm_tend_transfer_bytes, the Brent-failure return -- is that of zm_conv_tend_batch. */
 int zm_conv_tend_batch_gathered(int nchunks, const int* ncol, const double* t, const double* q, const double* u,
                                 const double* v, const double* pmid, const double* pint, const double* pdel,
                                 const double* zm, const double* zi, const double* phis, const double* pblh,
@@ -331,8 +323,8 @@ int zm_convtran1_fields(int pcnst, const int* doconvtran, const int* cnst_is_dry
  * as momtran returns them; all others (pcols,pver) per chunk.  Any pointer may be NULL: that field is neither
  * materialised nor copied.  Every element of an attached field is defined on return; padding columns (i > ncol) are 0,
  * and with cam3 = 1 (no momtran, zm_conv_intr.F90:808) the five momtran fields are 0.  The regular outputs do not
- * depend on what is attached.  The host-pointer variant copies the attached fields whole, also under
- * ZM_TEND_RETURN=sparse, and zm_tend_transfer_bytes counts them. */
+ * depend on what is attached.  The host-pointer variants copy the attached fields whole, also with the gathered
+ * return, and zm_tend_transfer_bytes counts them. */
 int zm_conv_tend_hist_fields(double* heat, double* qtnd, double* eurt, double* dif, double* dnlf, double* dnif,
                              double* tend_s, double* tend_s_snwprd, double* tend_s_snwevmlt,
                              double* ntprprd, double* ntsnprd,

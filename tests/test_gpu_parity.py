@@ -547,73 +547,68 @@ def test_conv_tend_with_convtran1_and_cam3(built, ncols, cam3):
 
 @pytest.mark.parametrize("pcols,pver", [(16, 32), (13, 29), (24, 26)])
 def test_conv_tend_glue_variants(built, monkeypatch, pcols, pver):
-    """The fused step's glue has two forms: momtran reading state%u / state%v and writing ptend_u / ptend_v itself, mcon
-    converted to kg/m2/s in the plume kernel, zm_conv_evap's tend_q written straight into evapcdp (default, needs
-    an even pcols*pver for its 16-byte zero-fills) -- and the packed winds(pcols,pver,2) / wind_tends form of
-    zm_conv_intr.F90:814-826 with the conversion in the final kernel (ZM_TEND_SPLIT_WINDS=0, and the automatic fallback
-    for odd pcols*pver); with the split form zm_conv_evap's kernel also applies physics_update itself and stores the
-    summed tendencies (ZM_TEND_FUSE_EVAP=0: separate kernels).  All bit for bit against the oracle, host-pointer and
-    device-resident calls."""
+    """The fused step's glue has two forms, chosen from what the call shows.  Split: momtran reads state%u / state%v
+    and writes ptend_u / ptend_v itself, zm_conv_evap applies physics_update and stores the summed tendencies; it needs
+    momtran, an even nchunks*pcols*pver and 16-byte aligned ptend_u, ptend_v, seten and ptend_s.  Packed: the
+    winds(pcols,pver,2) / wind_tends form of zm_conv_intr.F90:814-826 with separate state update and final sum.
+    (16,32) and (24,26) take the split form, (13,29) and a device-resident ptend_s one element off 16-byte alignment
+    the packed one.  All bit for bit against the oracle, host-pointer and device-resident calls."""
+    import torch
     Z = init_cuda(pcols, pver)
     o, _, _ = get_oracle("pm", pcols, pver)
     from cam_nor_physics_b200.device import DeviceTend
     ch = S.make_chunks(pcols * 91 - 3, pver, pcols, p_conv=0.6)      # 91 chunks: 13 x 29 x 91 elements are odd
     ref = o.conv_tend_batch(ch)
     assert int(ref["lengath"].sum()) > 100
-    for split, fuse in (("1", "1"), ("1", "0"), ("0", "1")):
-        monkeypatch.setenv("ZM_TEND_SPLIT_WINDS", split)
-        monkeypatch.setenv("ZM_TEND_FUSE_EVAP", fuse)     # physics_update + the ptend sums inside zm_conv_evap's kernel
-        monkeypatch.setenv("ZM_DEV_GRAPH", "0")
-        out = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt)
-        assert_same(out, ref, TEND_KEYS, pcols, exact=True, what=f"host-pointer step, split={split} fuse={fuse}")
-        dev = DeviceTend(ch)
-        dev.step()
-        assert dev.check() == 0
-        dout = {k: v.cpu().numpy() for k, v in dev.out.items()}
-        assert_same(dout, ref, TEND_KEYS, pcols, exact=True, what=f"device-resident step, split={split} fuse={fuse}")
+    monkeypatch.setenv("ZM_DEV_GRAPH", "0")
+    out = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt)
+    assert_same(out, ref, TEND_KEYS, pcols, exact=True, what="host-pointer step")
+    L = Z.lib()
+    dev = DeviceTend(ch)
+    L.zm_launch_count(1)
+    dev.step()
+    assert dev.check() == 0
+    n_step = L.zm_launch_count(1)
+    dout = {k: v.cpu().numpy() for k, v in dev.out.items()}
+    assert_same(dout, ref, TEND_KEYS, pcols, exact=True, what="device-resident step")
+    # ptend_s 8 bytes past a 16-byte boundary, pre-filled with garbage
+    ps = dev.out["ptend_s"]
+    buf = torch.full((ps.numel() + 1,), 1.25, dtype=ps.dtype, device=ps.device)
+    dev.out["ptend_s"] = buf[1:].view(ps.shape)
+    assert dev.out["ptend_s"].data_ptr() % 16 == 8
+    dev.step()
+    assert dev.check() == 0
+    # the packed form's two state-update halves, momtran's own initialisation and the final sum, against the split
+    # form's ptend_s += seten
+    assert L.zm_launch_count(1) == n_step + (3 if (pcols * pver) % 2 == 0 else 0)
+    dout = {k: v.cpu().numpy() for k, v in dev.out.items()}
+    assert_same(dout, ref, TEND_KEYS, pcols, exact=True, what="device-resident step, misaligned ptend_s")
     assert np.count_nonzero(ref["ptend_u"]) > 0 and np.count_nonzero(ref["mcon"]) > 0
 
 
 @pytest.mark.parametrize("ncols", [16 * 70, 16 * 1100 + 5])
-def test_sparse_return_equals_dense_return(built, ncols, monkeypatch):
-    """zm_conv_tend_batch moves only the convective columns' records device->host and scatters them into arrays its
-    worker threads zero-fill (default); ZM_TEND_RETURN=dense copies the arrays whole.  Both must define every element
-    identically, whatever the arrays held before, with and without the pbuf fields kept on the device."""
+def test_dense_return_defines_every_element(built, ncols):
+    """zm_conv_tend_batch copies the outputs device->host whole: every element is defined, whatever the arrays held
+    before, with and without the pbuf fields kept on the device, and equals the oracle bit for bit."""
     Z = init_cuda(16, 32)
     ch = S.make_chunks(ncols, 32, 16, p_conv=0.45)
-    res = {}
-    for mode in ("dense", "sparse", "sparse-prezeroed"):
-        monkeypatch.setenv("ZM_TEND_RETURN", mode.split("-")[0])
-        monkeypatch.setenv("ZM_TEND_OUTPUTS_PREZEROED", "1" if mode.endswith("prezeroed") else "0")
-        out = None
-        for rep in range(2):                   # the second call finds the first call's values (or garbage) in the arrays
-            if out is not None and not mode.endswith("prezeroed"):
-                for k, a in out.items():
-                    a[...] = 7 if a.dtype.kind == "i" else 1.25
-            elif out is not None:
-                for a in out.values():
-                    a[...] = 0
-            out = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt, out)
-        res[mode] = {k: v.copy() for k, v in out.items()}
-        moved = Z.last_transfer_bytes()
-        dense_bytes = sum(v.nbytes for v in out.values())
-        if mode == "dense":
-            assert moved["d2h"] >= dense_bytes
-        else:
-            assert moved["d2h"] < 0.75 * dense_bytes
-    for mode in ("sparse", "sparse-prezeroed"):
-        for k in res["dense"]:
-            assert np.array_equal(res[mode][k], res["dense"][k]), (mode, k)
-    monkeypatch.setenv("ZM_TEND_RETURN", "sparse")
-    monkeypatch.setenv("ZM_TEND_OUTPUTS_PREZEROED", "0")
+    out = None
+    for rep in range(2):                   # the second call finds garbage in the arrays
+        if out is not None:
+            for k, a in out.items():
+                a[...] = 7 if a.dtype.kind == "i" else 1.25
+        out = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt, out)
+    dense = {k: v.copy() for k, v in out.items()}
+    moved = Z.last_transfer_bytes()
+    assert moved["d2h"] >= sum(v.nbytes for v in out.values())
     out = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt, keep_pbuf_on_device=True)
-    for k in res["dense"]:
+    for k in dense:
         if k in ("mu", "md", "du", "eu", "ed", "dp", "dsubcld", "jt", "maxg"):
             assert not out[k].any()
         else:
-            assert np.array_equal(out[k], res["dense"][k]), k
+            assert np.array_equal(out[k], dense[k]), k
     o, _, _ = get_oracle("pm", 16, 32)
-    assert_same(res["sparse"], o.conv_tend_batch(ch), TEND_KEYS, 16, exact=True, what="sparse return vs oracle")
+    assert_same(dense, o.conv_tend_batch(ch), TEND_KEYS, 16, exact=True, what="dense return vs oracle")
 
 
 def test_finalize_releases_and_reinit_reproduces(built):

@@ -263,11 +263,6 @@ def test_gathered_step(built, monkeypatch, name):
             assert same_bits(r2["rec"], res["rec"]), (name, pbuf, var, val)
             for k in Z_.GATHERED_COL_OUT + ["jt", "maxg", "ideep", "lengath"]:
                 assert same_bits(r2[k], res[k]), (name, pbuf, var, val, k)
-        # ZM_TEND_RETURN does not apply to this entry point
-        monkeypatch.setenv("ZM_TEND_RETURN", "sparse")
-        r3 = Z_.zm_conv_tend_gathered(ch.ncol, st, ch.ztodt, keep_pbuf_on_device=keep)
-        monkeypatch.delenv("ZM_TEND_RETURN")
-        assert same_bits(r3["rec"], res["rec"]) and Z_.last_transfer_bytes() == bg
         # (e) the device mirror the gathered step leaves
         Z_.zm_conv_tend_gathered(ch.ncol, st, ch.ztodt, keep_pbuf_on_device=keep)
         dq = Z_.zm_conv_tend_2(do, q3, pdeldry, fracis, ch.ztodt, dry)

@@ -126,41 +126,39 @@ def test_host_step_history_fields(built, name):
 
 
 @pytest.mark.gpu
-def test_pipelined_history_fields_and_transfer_bytes(built, monkeypatch):
+def test_pipelined_history_fields_and_transfer_bytes(built):
     """1,100 chunks: the default schedule of four sub-batches slices the history arrays like every other output;
-    they travel whole (also under ZM_TEND_RETURN=sparse) and are exactly the extra device->host bytes."""
+    they travel whole and are exactly the extra device->host bytes."""
     Z = init_cuda(16, 32)
     o, p, _ = get_oracle("pm", 16, 32)
     ch = S.make_chunks(16 * 1100, 32, 16, p_conv=0.5)
     ref = o.conv_tend_batch(ch)
     href, _, _, _ = chain_reference(o, p, ch)
-    for ret in ("dense", "sparse"):
-        monkeypatch.setenv("ZM_TEND_RETURN", ret)
-        plain = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt)
-        b0 = Z.last_transfer_bytes()
-        out = {k: np.full_like(v, 7 if v.dtype.kind == "i" else SENTINEL) for k, v in plain.items()}
-        out.update(sentinel_out(ch.nchunks, 32, 16, HIST))
-        out = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt, out=out, hist=True)
-        b1 = Z.last_transfer_bytes()
-        assert Z.tend_trace().shape[0] == 4
-        for k in plain:
-            assert np.array_equal(out[k], plain[k]), (ret, k)
-        assert_same(out, ref, TEND_KEYS, 16, exact=True, what=f"pipelined ({ret}) regular outputs")
-        assert_hist(out, href, HIST, ch, f"pipelined ({ret})")
-        assert b1["h2d"] == b0["h2d"]
-        assert b1["d2h"] - b0["d2h"] == sum(out[k].nbytes for k in HIST), ret
+    plain = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt)
+    b0 = Z.last_transfer_bytes()
+    out = {k: np.full_like(v, 7 if v.dtype.kind == "i" else SENTINEL) for k, v in plain.items()}
+    out.update(sentinel_out(ch.nchunks, 32, 16, HIST))
+    out = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt, out=out, hist=True)
+    b1 = Z.last_transfer_bytes()
+    assert Z.tend_trace().shape[0] == 4
+    for k in plain:
+        assert np.array_equal(out[k], plain[k]), k
+    assert_same(out, ref, TEND_KEYS, 16, exact=True, what="pipelined regular outputs")
+    assert_hist(out, href, HIST, ch, "pipelined")
+    assert b1["h2d"] == b0["h2d"]
+    assert b1["d2h"] - b0["d2h"] == sum(out[k].nbytes for k in HIST)
 
 
 # ---- GPU: isolation -------------------------------------------------------------------------------------------------
 @pytest.mark.gpu
-@pytest.mark.parametrize("split", ["1", "0"])
-def test_subset_attach_and_one_shot(built, monkeypatch, split):
+@pytest.mark.parametrize("pc,nlev", [(16, 32), (13, 29)])
+def test_subset_attach_and_one_shot(built, pc, nlev):
     """A subset attaches only itself (the other arrays keep their contents); the attachment is one-shot and leaves
-    the next step exactly a never-attached step, launch count included.  With every field attached the zero-fill list
-    of the split-wind step is at its limit (an overflow would fail the call)."""
-    monkeypatch.setenv("ZM_TEND_SPLIT_WINDS", split)
-    Z = init_cuda(16, 32)
-    ch = S.make_chunks(16 * 150 - 7, 32, 16, p_conv=0.6)
+    the next step exactly a never-attached step, launch count included.  (16, 32) takes the split-wind glue, whose
+    zero-fill list is at its limit with every field attached (an overflow would fail the call); (13, 29), with an odd
+    pcols*pver, the packed one."""
+    Z = init_cuda(pc, nlev)
+    ch = S.make_chunks(pc * 150 - 7, nlev, pc, p_conv=0.6)
     st = state_of(ch)
     L = Z.lib()
     L.zm_launch_count(1)
@@ -171,7 +169,7 @@ def test_subset_attach_and_one_shot(built, monkeypatch, split):
     assert n_full == n_plain + 1                           # the in-cloud wind initialisation
     sub = ["tend_s", "icwd"]
     out = {k: v.copy() for k, v in plain.items()}
-    out.update(sentinel_out(ch.nchunks, 32, 16, HIST))
+    out.update(sentinel_out(ch.nchunks, nlev, pc, HIST))
     out = Z.zm_conv_tend(ch.ncol, st, ch.ztodt, out=out, hist=sub)
     for k in HIST:
         if k in sub:
@@ -188,16 +186,16 @@ def test_subset_attach_and_one_shot(built, monkeypatch, split):
 
 # ---- GPU: device-resident step ----------------------------------------------------------------------------------
 @pytest.mark.gpu
-@pytest.mark.parametrize("subbatches", ["1", "2"])
-def test_device_step_history_graph_replay(built, monkeypatch, subbatches):
+@pytest.mark.parametrize("pc,nlev", [(16, 32), (13, 29)])
+def test_device_step_history_graph_replay(built, pc, nlev):
     """DeviceTend(hist=True): direct, captured and replayed steps all write every history field (sentinel-filled
     before each step) with the host-pointer step's values; other pointers attached force a new capture, and the
-    graph never writes to the pointers of an earlier attachment."""
+    graph never writes to the pointers of an earlier attachment.  (16, 32) takes the split-wind glue, (13, 29) the
+    packed one."""
     import torch
     from cam_nor_physics_b200.device import DeviceTend
-    monkeypatch.setenv("ZM_DEV_SUBBATCHES", subbatches)
-    Z = init_cuda(16, 32)
-    ch = S.make_chunks(16 * 300 - 5, 32, 16, p_conv=0.5)
+    Z = init_cuda(pc, nlev)
+    ch = S.make_chunks(pc * 300 - 5, nlev, pc, p_conv=0.5)
     ref = Z.zm_conv_tend(ch.ncol, state_of(ch), ch.ztodt, hist=True)
     dev = DeviceTend(ch, hist=True)
     plain = DeviceTend(ch)
