@@ -95,12 +95,15 @@ __global__ void k_convr_init_cols(ConvrIn in, ConvrOut o, ConvrWork w) {
 }
 // The per-level outputs (zero outside the convective columns; nothing reads them before the plume kernel writes the
 // convective columns) and whatever else the caller wants zeroed with them (the fused step: ptend_u, ptend_v and the KE
-// heating, which momtran writes for convective columns only): 16-byte stores over a list of arrays.
+// heating, which momtran writes for convective columns only): 16-byte stores over a list of arrays, scalar ones for
+// an array that is not 16-byte aligned or has an odd length.
 // Measured and dropped: the same fill on a side stream, either as ONE WARP PER SM with 32 registers -- resident beside
 // the single wave of the first CAPE pass, which leaves 1,024 of an SM's 65,536 registers free -- or as an ordinary grid
 // beside cldprp / the second CAPE pass, joined before the plume kernel: 2.107 / 2.109 ms against 2.108 ms with the
 // fill on the launching stream ahead of everything.
-#define ZM_FILL_MAX 24
+// Capacity: the fused step under cam3 with every history field attached lists 26 arrays -- zm_convr's 13 + 4 per-level
+// outputs, mcon and pflx, ptend_u and ptend_v, then pguall, pgdall, seten, icwu and icwd.
+#define ZM_FILL_MAX 26
 struct FillList {
   double* p[ZM_FILL_MAX];
   unsigned long long n[ZM_FILL_MAX];     // doubles

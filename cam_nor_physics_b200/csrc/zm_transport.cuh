@@ -21,8 +21,8 @@ struct EvapArgs {
       *flxprec, *flxsnow;
   double deltat;
   // Fused zm_conv_tend step (k_conv_evap<true>): t, q above are the state BEFORE zm_convr's tendencies and the kernel
-  // applies physics_update itself (t + heat*dt/cpair, q + qtnd*dt clipped at 1e-12: physics_types.F90:322-329, 427,
-  // the statements of k_state_update), then stores the sums of the two ptend_loc instead of its own tend_s:
+  // applies physics_update itself (t + heat*dt/cpair, q + qtnd*dt clipped at 1e-12: physics_types.F90:322-329, 427),
+  // then stores the sums of the two ptend_loc instead of its own tend_s:
   // ps = heat + tend_s, pq = qtnd + tend_q (zm_conv_intr.F90:736, 803); tend_q still goes to a.tend_q (= evapcdp).
   const double *heat = nullptr, *qtnd = nullptr;
   double *ps = nullptr, *pq = nullptr;
@@ -189,7 +189,8 @@ struct MomArgs {
   double *dq_u = nullptr, *dq_v = nullptr;   // (zero-filled, like seten, by the caller: momtran writes convective columns only)
 };
 
-// initialisation of the outgoing fields (zm_conv.F90:2429-2443, 2630)
+// initialisation of the outgoing fields (zm_conv.F90:2429-2443, 2630) for the packed arrays of zm_momtran_batch[_dev];
+// the fused step zero-fills its split arrays with zm_convr's outputs instead
 __global__ void k_momtran_init(MomArgs a) {
   const int pcols = P.pcols, pver = P.pver;
   const size_t n2 = (size_t)a.nchunks * pcols * pver;
@@ -198,8 +199,7 @@ __global__ void k_momtran_init(MomArgs a) {
     // e -> (c, m, k, i)
     size_t i = e % pcols, r = e / pcols;
     size_t m = (r / pver) % a.ncnst, c = r / ((size_t)pver * a.ncnst);
-    // pguall / pgdall / icwu / icwd are history diagnostics (ZMUPGU ... ZMICVD, zm_conv_intr.F90:846-857): all four
-    // NULL inside the fused zm_conv_tend step, which does not return them
+    // pguall / pgdall / icwu / icwd are history diagnostics (ZMUPGU ... ZMICVD, zm_conv_intr.F90:846-857)
     if (a.pguall) {
       a.pguall[e] = 0.0; a.pgdall[e] = 0.0;
       if ((int)i < a.ncol[c]) { a.icwu[e] = a.q[e]; a.icwd[e] = a.q[e]; }

@@ -591,8 +591,8 @@ int momtran_launch(Workspace& ws, cudaStream_t s, MomArgs a, bool own_arena = tr
     cb = &own;
   }
   a.ktm = cb->ktm; a.kbm = cb->kbm; a.slots = cb->slots; a.count = cb->count;
-  // fused step with split wind arrays: dq_u, dq_v and seten were zero-filled with zm_convr's outputs at the start of
-  // the step (k_zero_fill); the packed form initialises its outgoing fields here
+  // the fused step (split wind arrays) zero-filled dq_u, dq_v and seten with zm_convr's outputs at its start
+  // (k_zero_fill); the standalone packed form initialises its outgoing fields here
   if (!a.q_u) { k_momtran_init<<<592, 256, 0, s>>>(a); ++tls_launches; }
   const size_t smem_mom = momtran_smem_bytes(pver);
   if (smem_mom > 48 * 1024)
@@ -724,60 +724,22 @@ int convtran_launch(Workspace& ws, cudaStream_t s, TranArgs a, const int* doconv
 }
 
 // ---- zm_conv_tend glue (zm_conv_intr.F90:662-836) ------------------------------------------------
-// state1 after physics_update(ptend_loc of zm_convr): physics_types.F90:322-329 (q + qneg3 clip at
-// qmin(1)=1e-12) and :427 (t += s*dt/cpair); winds(:,:,1:2) = state1%u,v (zm_conv_intr.F90:815-816)
-// PART 0: both; 1: t1, q1 only (what zm_conv_evap needs); 2: winds only (what momtran needs) -- the two halves run on
-// the two branches of the evap / momtran fork
-template <int PART>
-__global__ void k_state_update(int n2, int nper, const double* t, const double* q, const double* heat,
-                               const double* qtnd, const double* u, const double* v, double ztodt,
-                               double* t1, double* q1, double* winds) {
-  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n2; e += gridDim.x * blockDim.x) {
-    if (PART != 2) {
-      t1[e] = t[e] + div_z(heat[e] * ztodt, P.cpair);
-      double qn = q[e] + qtnd[e] * ztodt;
-      q1[e] = (qn < 1.e-12) ? 1.e-12 : qn;
-    }
-    if (PART != 1) {
-      int c = e / nper, r = e - c * nper;            // nper = pcols*pver
-      winds[(size_t)c * 2 * nper + r] = u[e];
-      winds[(size_t)c * 2 * nper + nper + r] = v[e];
-    }
-  }
-}
-// ptend_all = sum of the three ptend_loc (physics_ptend_sum, physics_types.F90:698-844) in the packed glue form (mcon
-// has left the plume kernel in kg/m2/s already).  MODE 0: cam3, no momentum transport (zm_conv_intr.F90:808);
-// 1: wind tendencies unpacked from wind_tends(pcols,pver,2).  evapcdp == ev_q when zm_conv_evap wrote its tend_q
-// straight into the caller's evapcdp.
-template <int MODE>
-__global__ void k_tend_finalize(int n2, int nper, const double* heat, const double* qtnd,
-                                const double* ev_s, const double* ev_q, const double* seten,
-                                const double* wtend, double* ps, double* pq, double* pu, double* pv,
-                                double* evapcdp) {
-  for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n2; e += gridDim.x * blockDim.x) {
-    const double evq = ev_q[e];
-    pq[e] = qtnd[e] + evq;
-    if (MODE) {
-      ps[e] = (heat[e] + ev_s[e]) + seten[e];
-      int c = e / nper, r = e - c * nper;
-      pu[e] = wtend[(size_t)c * 2 * nper + r];
-      pv[e] = wtend[(size_t)c * 2 * nper + nper + r];
-    } else {
-      ps[e] = heat[e] + ev_s[e];
-      pu[e] = 0.0; pv[e] = 0.0;
-    }
-    if (evapcdp != ev_q) evapcdp[e] = evq;
-  }
-}
-
 // the last term of ptend_s when zm_conv_evap has stored heat + tend_s itself: ptend_s = (heat + tend_s) + seten
-// (zm_conv_intr.F90:833), every element like the reference (seten is +0 outside the columns momtran wrote)
-__global__ void k_add_seten(size_t nhalf, double2* ps, const double2* seten) {
-  for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < nhalf; e += (size_t)gridDim.x * blockDim.x) {
-    double2 a = ps[e];
-    const double2 b = seten[e];
-    a.x = a.x + b.x; a.y = a.y + b.y;
-    ps[e] = a;
+// (zm_conv_intr.F90:833), every element like the reference (seten is +0 outside the columns momtran wrote).
+// 16-byte loads and stores when both arrays are 16-byte aligned and n is even, scalar ones otherwise.
+__global__ void k_add_seten(size_t n, double* ps, const double* seten) {
+  const size_t tid = (size_t)blockIdx.x * blockDim.x + threadIdx.x, nth = (size_t)gridDim.x * blockDim.x;
+  if (((((uintptr_t)ps) | ((uintptr_t)seten)) & 15) == 0 && !(n & 1)) {
+    double2* p2 = reinterpret_cast<double2*>(ps);
+    const double2* s2 = reinterpret_cast<const double2*>(seten);
+    for (size_t e = tid; e < (n >> 1); e += nth) {
+      double2 a = p2[e];
+      const double2 b = s2[e];
+      a.x = a.x + b.x; a.y = a.y + b.y;
+      p2[e] = a;
+    }
+  } else {
+    for (size_t e = tid; e < n; e += nth) ps[e] = ps[e] + seten[e];
   }
 }
 
@@ -1126,7 +1088,7 @@ int zm_get_timers(int* n, const char** names, float* ms) {
     if (!strcmp(k, "momtran")) return 2;
     if (!strcmp(k, "convtran1")) return 3;
     if (!strcmp(k, "convtran2")) return 4;
-    if (!strcmp(k, "state_update") || !strcmp(k, "tend_finalize")) return 5;
+    if (!strcmp(k, "tend_finalize")) return 5;
     return 0;                                        // every kernel of zm_convr
   };
   for (Workspace* ws : {&tls_work, &tls_stage2}) {
@@ -1381,24 +1343,23 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
   const size_t pc = g_params.pcols, L = g_params.pver, nc = (size_t)nchunks * pc;
   const size_t n2 = nc * L;
   const HistFields H = hist ? *hist : HistFields{};
-  if (ws.ensure(convr_work_bytes(nc, (int)L) + 19 * al(n2, 8) + 6 * al(2 * n2, 8) + chunk_bounds_bytes(nchunks, (int)nc) + 8192 +
-                (H.any() ? 4 * al(n2, 8) + 4 * al(2 * n2, 8) : 0)))
+  if (ws.ensure(convr_work_bytes(nc, (int)L) + 16 * al(n2, 8) + 4 * al(2 * n2, 8) + chunk_bounds_bytes(nchunks, (int)nc) + 8192 +
+                (H.any() ? 5 * al(n2, 8) + 4 * al(2 * n2, 8) : 0)))
     return -100;
   cudaStream_t s = (cudaStream_t)stream;      // NULL = the CUDA default stream
-  // History fields (zm_conv_tend_hist_fields): an attached field is written where it is computed; heat, qtnd, tend_s
-  // and seten are needed anyway and live in scratch otherwise.  eurt, dif, dnlf, dnif of zm_convr, zm_conv_evap's four
-  // diagnostics and momtran's pguall / pgdall / icwu / icwd are not materialised unless attached; the kernels store
-  // the last two groups as a whole, so an attached group gets scratch for its unattached members.
+  // History fields (zm_conv_tend_hist_fields): an attached field is written where it is computed; heat, qtnd and
+  // seten are needed anyway and live in scratch otherwise.  eurt, dif, dnlf, dnif of zm_convr, zm_conv_evap's tend_s
+  // and four diagnostics and momtran's pguall / pgdall / icwu / icwd are not materialised unless attached; the kernels
+  // store the last two groups as a whole, so an attached group gets scratch for its unattached members.
   auto own = [&](int j, size_t n) { return H.p[j] ? H.p[j] : ws.take<double>(n); };
   const bool hist_evap = H.p[H_TEND_S] || H.p[H_SNWPRD] || H.p[H_SNWEVMLT] || H.p[H_NTPRPRD] || H.p[H_NTSNPRD];
   const bool hist_mom = H.p[H_PGUALL] || H.p[H_PGDALL] || H.p[H_ICWU] || H.p[H_ICWD];
   double *heat = own(H_HEAT, n2), *qtnd = own(H_QTND, n2), *eurt = H.p[H_EURT], *dif = H.p[H_DIF],
-         *dnlf = H.p[H_DNLF], *dnif = H.p[H_DNIF], *t1 = ws.take<double>(n2), *q1 = ws.take<double>(n2),
-         *ev_s = own(H_TEND_S, n2), *ev_q_scratch = ws.take<double>(n2), *snwprd = nullptr, *snwevmlt = nullptr,
-         *ntprprd = nullptr, *ntsnprd = nullptr, *seten = own(H_SETEN, n2);
-  double *winds = ws.take<double>(2 * n2), *wtend = ws.take<double>(2 * n2), *pgu = nullptr, *pgd = nullptr,
-         *icwu = nullptr, *icwd = nullptr;
+         *dnlf = H.p[H_DNLF], *dnif = H.p[H_DNIF], *ev_s = nullptr, *ev_q_scratch = ws.take<double>(n2),
+         *snwprd = nullptr, *snwevmlt = nullptr, *ntprprd = nullptr, *ntsnprd = nullptr, *seten = own(H_SETEN, n2);
+  double *pgu = nullptr, *pgd = nullptr, *icwu = nullptr, *icwd = nullptr;
   if (hist_evap) {
+    ev_s = own(H_TEND_S, n2);
     snwprd = own(H_SNWPRD, n2); snwevmlt = own(H_SNWEVMLT, n2); ntprprd = own(H_NTPRPRD, n2); ntsnprd = own(H_NTSNPRD, n2);
   }
   if (hist_mom) {
@@ -1407,67 +1368,45 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
   // zm_conv_evap's tend_q IS evapcdp (zm_conv_intr.F90:764-769 passes ptend_loc%q(:,:,1), :796 outputs it): written in place
   double* ev_q = evapcdp ? evapcdp : ev_q_scratch;
   const bool do_mom = !g_params.cam3;          // zm_conv_intr.F90:808: momentum transport is non-cam3 physics
-  // Glue form, chosen from what the call shows.  Split (fast): momtran reads state%u / state%v and writes ptend_u /
-  // ptend_v itself, zm_conv_evap stores the summed tendencies, k_add_seten adds seten.  Its zero-fills and k_add_seten
-  // make 16-byte stores, so it needs momtran (not cam3), an even pcols*pver and 16-byte aligned ptend_u, ptend_v, seten
-  // and ptend_s.  Packed otherwise: state update, momtran on winds(pcols,pver,2) and k_tend_finalize
-  // (zm_conv_intr.F90:814-833).
-  const bool split = do_mom && !(n2 & 1) &&
-                     (((uintptr_t)ptend_u | (uintptr_t)ptend_v | (uintptr_t)seten | (uintptr_t)ptend_s) & 15) == 0;
+  // The glue (zm_conv_intr.F90:814-833) works on the caller's separate wind arrays: momtran reads state%u / state%v
+  // and writes ptend_u / ptend_v itself, zm_conv_evap stores the summed tendencies, k_add_seten adds seten.  Its
+  // kernels take any pcols*pver and arrays of any 8-byte alignment.
   ConvrIn in{nchunks, ncol, t, q, pmid, pint, pdel, zm, zi, phis, pblh, tpert, landfrac, 0.5 * ztodt};
   ConvrOut o{prec, jctop, jcbot, qtnd, heat, mcon, cme, cape, eurt, dlf, pflx, zdu, rprd,
              mu, md, du, eu, ed, dp, dsubcld, jt, maxg, ideep, lengath, ql, rliq, dif, dnlf, dnif, rice};
   o.mcon_kgm2s = 1;                            // unit conversion of zm_conv_intr.F90:693 inside the plume kernel
   in.org = g_params.zm_org ? org : nullptr;
-  // split winds: ptend_u / ptend_v / seten are zero outside the convective columns momtran writes -- filled with
-  // zm_convr's own outputs at the start of the step
+  // ptend_u / ptend_v / seten are zero outside the convective columns momtran writes, and everywhere with cam3 (no
+  // momtran, zm_conv_intr.F90:808; seten is then filled only when attached) -- filled with zm_convr's own outputs at
+  // the start of the step.  momtran's diagnostics: pguall / pgdall are zero outside the convective columns; with cam3
+  // all five momtran fields return 0.
   FillList xf{};
   auto xadd = [&](double* p, size_t n) { xf.p[xf.cnt] = p; xf.n[xf.cnt] = n; ++xf.cnt; };
-  if (split) { xadd(ptend_u, n2); xadd(ptend_v, n2); xadd(seten, n2); }
-  // momtran's diagnostics: pguall / pgdall are zero outside the convective columns; with cam3 (no momtran,
-  // zm_conv_intr.F90:808) all five momtran fields return 0
+  xadd(ptend_u, n2); xadd(ptend_v, n2);
+  if (do_mom || H.p[H_SETEN]) xadd(seten, n2);
   if (hist_mom) { xadd(pgu, 2 * n2); xadd(pgd, 2 * n2); }
-  if (!do_mom) {
-    if (H.p[H_SETEN]) xadd(seten, n2);
-    if (hist_mom) { xadd(icwu, 2 * n2); xadd(icwd, 2 * n2); }
-  }
-  int rc = convr_launch(ws, s, in, o, false, orgt, org2d, xf.cnt ? &xf : nullptr);
+  if (!do_mom && hist_mom) { xadd(icwu, 2 * n2); xadd(icwd, 2 * n2); }
+  int rc = convr_launch(ws, s, in, o, false, orgt, org2d, &xf);
   if (rc) return rc;
   if (hooks) {
     CK(cudaEventRecord(hooks->convr_done, s));            // zm_convr outputs are final from here on
     CK(cudaStreamWaitEvent(s, hooks->late_inputs, 0));    // u, v, cld have arrived
   }
-  const int nper = (int)(pc * L);
-  EvapArgs ea{nchunks, ncol, t1, pmid, pdel, q1, landfrac, rprd, cld, ev_s, snwprd, snwevmlt, ev_q,
+  // Nothing but zm_conv_evap needs the updated state: the kernel applies physics_update to its own operands and
+  // stores heat + tend_s / qtnd + tend_q straight into ptend_s / ptend_q (k_conv_evap<true>); what is left for the end
+  // of the step is ptend_s += seten.  tend_s and the four snow diagnostics are stored only when history asks for them
+  // (k_conv_evap<true, true>).
+  EvapArgs ea{nchunks, ncol, t, pmid, pdel, q, landfrac, rprd, cld, ev_s, snwprd, snwevmlt, ev_q,
               prec, snow, ntprprd, ntsnprd, flxprec, flxsnow, ztodt};
-  // zm_conv_evap and momtran both depend only on zm_convr's outputs (zm_conv_intr.F90:764, 822): evap
-  // (with the t, q half of the state update) goes to a side stream and overlaps momtran (which only waits for
-  // the wind half); kept serial while per-kernel profiling is on
+  ea.heat = heat; ea.qtnd = qtnd; ea.ps = ptend_s; ea.pq = ptend_q;
+  // zm_conv_evap and momtran both depend only on zm_convr's outputs (zm_conv_intr.F90:764, 822): evap goes to a side
+  // stream and overlaps momtran; kept serial while per-kernel profiling is on
   const bool fork = !g_profile;
-  // With the split winds nothing but zm_conv_evap needs the updated state: the kernel applies physics_update to its
-  // own operands and stores heat + tend_s / qtnd + tend_q straight into ptend_s / ptend_q (k_conv_evap<true>); what is
-  // left for the end of the step is ptend_s += seten.
-  if (split) {         // tend_s stays: k_conv_evap<true, true> also stores it and the four snow diagnostics
-    ea.t = t; ea.q = q; ea.heat = heat; ea.qtnd = qtnd; ea.ps = ptend_s; ea.pq = ptend_q;
-    if (!hist_evap) ea.tend_s = nullptr;
-  }
   if (fork) {
     if (ws.ensure_side()) return -100;
     CK(cudaEventRecord(ws.ev_fork, s));
     CK(cudaStreamWaitEvent(ws.side, ws.ev_fork, 0));
-    if (!split) {
-      k_state_update<1><<<1184, 256, 0, ws.side>>>((int)n2, nper, t, q, heat, qtnd, u, v, ztodt, t1, q1, winds);
-      ++tls_launches;
-      if (do_mom) {             // packed winds feed momtran only
-        k_state_update<2><<<1184, 256, 0, s>>>((int)n2, nper, t, q, heat, qtnd, u, v, ztodt, t1, q1, winds);
-        ++tls_launches;
-      }
-    }
-  } else if (!split) {
-    k_state_update<0><<<1184, 256, 0, s>>>((int)n2, nper, t, q, heat, qtnd, u, v, ztodt, t1, q1, winds);
-    ++tls_launches;
   }
-  tick(ws, s, "state_update");
   rc = evap_launch(fork ? ws.side : s, ea);
   if (rc) return rc;
   if (g_params.zm_org) {     // zm_conv_intr.F90:773-777 (needs evapcdp = ev_q)
@@ -1494,10 +1433,10 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
     MomArgs ma;
     ma.nchunks = nchunks; ma.ncnst = 2; ma.ncol = ncol; ma.jt = jt; ma.mx = maxg; ma.ideep = ideep;
     ma.lengath = lengath; ma.ktm = nullptr; ma.kbm = nullptr; ma.domom[0] = 1; ma.domom[1] = 1;
-    ma.q = winds; ma.mu = mu; ma.md = md; ma.du = du; ma.eu = eu; ma.ed = ed; ma.dp = dp;
-    ma.dqdt = wtend; ma.pguall = pgu; ma.pgdall = pgd; ma.icwu = icwu; ma.icwd = icwd; ma.seten = seten;
+    ma.q = nullptr; ma.mu = mu; ma.md = md; ma.du = du; ma.eu = eu; ma.ed = ed; ma.dp = dp;
+    ma.dqdt = nullptr; ma.pguall = pgu; ma.pgdall = pgd; ma.icwu = icwu; ma.icwd = icwd; ma.seten = seten;
     ma.dt = ztodt;
-    if (split) { ma.q_u = u; ma.q_v = v; ma.dq_u = ptend_u; ma.dq_v = ptend_v; }
+    ma.q_u = u; ma.q_v = v; ma.dq_u = ptend_u; ma.dq_v = ptend_v;
     if (hist_mom) { k_icw_init<<<1184, 256, 0, s>>>(nchunks, ncol, u, v, icwu, icwd); ++tls_launches; }
     rc = momtran_launch(ws, s, ma, false, &cb);
     if (rc) return rc;
@@ -1520,14 +1459,8 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
   }
   if (tran_stream != s) CK(cudaStreamWaitEvent(s, ws.ev_join2, 0));
   if (fork) CK(cudaStreamWaitEvent(s, ws.ev_join, 0));
-  if (split) {
-    k_add_seten<<<1184, 256, 0, s>>>(n2 / 2, (double2*)ptend_s, (const double2*)seten);
-  } else {
-    auto fin = do_mom ? k_tend_finalize<1> : k_tend_finalize<0>;
-    fin<<<1184, 256, 0, s>>>((int)n2, nper, heat, qtnd, ev_s, ev_q, seten, wtend, ptend_s, ptend_q, ptend_u, ptend_v,
-                             evapcdp ? evapcdp : ev_q);
-  }
-  ++tls_launches;
+  // with cam3 ptend_s = heat + tend_s (zm_conv_intr.F90:808), which zm_conv_evap has stored already
+  if (do_mom) { k_add_seten<<<1184, 256, 0, s>>>(n2, ptend_s, seten); ++tls_launches; }
   tick(ws, s, "tend_finalize");
   CK(cudaGetLastError());
   return 0;

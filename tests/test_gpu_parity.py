@@ -546,13 +546,12 @@ def test_conv_tend_with_convtran1_and_cam3(built, ncols, cam3):
 
 
 @pytest.mark.parametrize("pcols,pver", [(16, 32), (13, 29), (24, 26)])
-def test_conv_tend_glue_variants(built, monkeypatch, pcols, pver):
-    """The fused step's glue has two forms, chosen from what the call shows.  Split: momtran reads state%u / state%v
-    and writes ptend_u / ptend_v itself, zm_conv_evap applies physics_update and stores the summed tendencies; it needs
-    momtran, an even nchunks*pcols*pver and 16-byte aligned ptend_u, ptend_v, seten and ptend_s.  Packed: the
-    winds(pcols,pver,2) / wind_tends form of zm_conv_intr.F90:814-826 with separate state update and final sum.
-    (16,32) and (24,26) take the split form, (13,29) and a device-resident ptend_s one element off 16-byte alignment
-    the packed one.  All bit for bit against the oracle, host-pointer and device-resident calls."""
+def test_conv_tend_glue_any_shape_and_alignment(built, monkeypatch, pcols, pver):
+    """The fused step's glue has one form for every shape and alignment: momtran reads state%u / state%v and writes
+    ptend_u / ptend_v itself, zm_conv_evap applies physics_update and stores the summed tendencies, the last kernel adds
+    seten.  (13,29) gives an odd nchunks*pcols*pver; a device-resident step with ptend_s and ptend_u one element off
+    16-byte alignment launches exactly the kernels of the aligned one.  All bit for bit against the oracle,
+    host-pointer and device-resident calls."""
     import torch
     Z = init_cuda(pcols, pver)
     o, _, _ = get_oracle("pm", pcols, pver)
@@ -571,18 +570,17 @@ def test_conv_tend_glue_variants(built, monkeypatch, pcols, pver):
     n_step = L.zm_launch_count(1)
     dout = {k: v.cpu().numpy() for k, v in dev.out.items()}
     assert_same(dout, ref, TEND_KEYS, pcols, exact=True, what="device-resident step")
-    # ptend_s 8 bytes past a 16-byte boundary, pre-filled with garbage
-    ps = dev.out["ptend_s"]
-    buf = torch.full((ps.numel() + 1,), 1.25, dtype=ps.dtype, device=ps.device)
-    dev.out["ptend_s"] = buf[1:].view(ps.shape)
-    assert dev.out["ptend_s"].data_ptr() % 16 == 8
+    # ptend_s (the seten sum) and ptend_u (the zero-fill) 8 bytes past a 16-byte boundary, pre-filled with garbage
+    for k in ("ptend_s", "ptend_u"):
+        a = dev.out[k]
+        buf = torch.full((a.numel() + 1,), 1.25, dtype=a.dtype, device=a.device)
+        dev.out[k] = buf[1:].view(a.shape)
+        assert dev.out[k].data_ptr() % 16 == 8
     dev.step()
     assert dev.check() == 0
-    # the packed form's two state-update halves, momtran's own initialisation and the final sum, against the split
-    # form's ptend_s += seten
-    assert L.zm_launch_count(1) == n_step + (3 if (pcols * pver) % 2 == 0 else 0)
+    assert L.zm_launch_count(1) == n_step
     dout = {k: v.cpu().numpy() for k, v in dev.out.items()}
-    assert_same(dout, ref, TEND_KEYS, pcols, exact=True, what="device-resident step, misaligned ptend_s")
+    assert_same(dout, ref, TEND_KEYS, pcols, exact=True, what="device-resident step, misaligned ptend_s and ptend_u")
     assert np.count_nonzero(ref["ptend_u"]) > 0 and np.count_nonzero(ref["mcon"]) > 0
 
 

@@ -92,7 +92,7 @@ CONFIGS = {
     "cam3": (16, 32, {"cam3": 1, "num_cin": 5}, 16 * 90 - 3),
     "zm_org": (16, 32, {"zm_org": 1}, 16 * 90 - 3),
     "L58_parcel_pbl": (16, 58, {"lparcel_pbl": 1}, 16 * 40 - 3),
-    "odd_13x29": (13, 29, {}, 13 * 91 - 3),          # odd pcols*pver: packed winds and the unfused evap kernel
+    "odd_13x29": (13, 29, {}, 13 * 91 - 3),          # odd nchunks*pcols*pver: the scalar fill and seten sum
 }
 
 
@@ -154,9 +154,9 @@ def test_pipelined_history_fields_and_transfer_bytes(built):
 @pytest.mark.parametrize("pc,nlev", [(16, 32), (13, 29)])
 def test_subset_attach_and_one_shot(built, pc, nlev):
     """A subset attaches only itself (the other arrays keep their contents); the attachment is one-shot and leaves
-    the next step exactly a never-attached step, launch count included.  (16, 32) takes the split-wind glue, whose
-    zero-fill list is at its limit with every field attached (an overflow would fail the call); (13, 29), with an odd
-    pcols*pver, the packed one."""
+    the next step exactly a never-attached step, launch count included, at an even and an odd pcols*pver.  (cam3
+    with every field attached is the case that fills the zero-fill list to its limit: test_host_step_history_fields,
+    where an overflow would fail the call.)"""
     Z = init_cuda(pc, nlev)
     ch = S.make_chunks(pc * 150 - 7, nlev, pc, p_conv=0.6)
     st = state_of(ch)
@@ -190,8 +190,8 @@ def test_subset_attach_and_one_shot(built, pc, nlev):
 def test_device_step_history_graph_replay(built, pc, nlev):
     """DeviceTend(hist=True): direct, captured and replayed steps all write every history field (sentinel-filled
     before each step) with the host-pointer step's values; other pointers attached force a new capture, and the
-    graph never writes to the pointers of an earlier attachment.  (16, 32) takes the split-wind glue, (13, 29) the
-    packed one."""
+    graph never writes to the pointers of an earlier attachment.  (16, 32) and (13, 29): an even and an odd
+    pcols*pver."""
     import torch
     from cam_nor_physics_b200.device import DeviceTend
     Z = init_cuda(pc, nlev)
