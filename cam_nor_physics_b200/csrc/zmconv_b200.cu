@@ -102,6 +102,11 @@ struct Workspace {
     return p;
   }
 };
+// the outputs of zm_convr that momtran (zm_conv.F90:2315) and convtran (:1976) read, device pointers
+struct MassFlux {
+  const double *mu = nullptr, *md = nullptr, *du = nullptr, *eu = nullptr, *ed = nullptr, *dp = nullptr;
+  const int *jt = nullptr, *maxg = nullptr, *ideep = nullptr, *lengath = nullptr;
+};
 // Device-resident copy of the pbuf fields zm_conv_tend hands to zm_conv_tend_2 (ZM_MU..ZM_IDEEP,
 // zm_conv_intr.F90:113-132, 994-1004): they live in an arena of their own (tls_mirror_ws, touched by nothing but
 // zm_conv_tend_batch) until the calling thread's next zm_conv_tend_batch call, so convtran2 needs no second H2D
@@ -109,8 +114,8 @@ struct Workspace {
 // cannot disturb them.  Set only when zm_conv_tend_batch succeeded; cleared on entry and on failure.
 struct PbufMirror {
   int nchunks = 0;
-  const double *mu = nullptr, *md = nullptr, *du = nullptr, *eu = nullptr, *ed = nullptr, *dp = nullptr, *dsubcld = nullptr;
-  const int *jt = nullptr, *maxg = nullptr, *ideep = nullptr, *lengath = nullptr;
+  MassFlux f;
+  const double* dsubcld = nullptr;
 };
 thread_local PbufMirror tls_mirror;
 // zm_org = 1: the pointer dummies org / orgt / org2d of zm_convr (zm_conv.F90:421-423), attached per call
@@ -580,17 +585,19 @@ int chunk_bounds_enqueue(Workspace& ws, cudaStream_t s, int nchunks, const int* 
   return 0;
 }
 
-// own_arena: the bounds come from this call's own arena; otherwise `cb` holds them already
-int momtran_launch(Workspace& ws, cudaStream_t s, MomArgs a, bool own_arena = true, const ChunkBounds* cb = nullptr) {
+// momtran's arguments with the mass-flux fields of f; the caller sets the winds, domom and the outputs
+MomArgs mom_args(int nchunks, const int* ncol, const MassFlux& f, double dt) {
+  MomArgs a{};
+  a.nchunks = nchunks; a.ncnst = 2; a.ncol = ncol; a.dt = dt;
+  a.jt = f.jt; a.mx = f.maxg; a.ideep = f.ideep; a.lengath = f.lengath;
+  a.mu = f.mu; a.md = f.md; a.du = f.du; a.eu = f.eu; a.ed = f.ed; a.dp = f.dp;
+  return a;
+}
+
+int momtran_launch(cudaStream_t s, MomArgs a, const ChunkBounds& cb) {
   const int pcols = g_params.pcols, pver = g_params.pver;
   const int ncolpad = a.nchunks * pcols;
-  ChunkBounds own;
-  if (!cb) {
-    if (own_arena && ws.ensure(chunk_bounds_bytes(a.nchunks, ncolpad))) return -100;
-    if (chunk_bounds_enqueue(ws, s, a.nchunks, a.jt, a.mx, a.lengath, own)) return -100;
-    cb = &own;
-  }
-  a.ktm = cb->ktm; a.kbm = cb->kbm; a.slots = cb->slots; a.count = cb->count;
+  a.ktm = cb.ktm; a.kbm = cb.kbm; a.slots = cb.slots; a.count = cb.count;
   // the fused step (split wind arrays) zero-filled dq_u, dq_v and seten with zm_convr's outputs at its start
   // (k_zero_fill); the standalone packed form initialises its outgoing fields here
   if (!a.q_u) { k_momtran_init<<<592, 256, 0, s>>>(a); ++tls_launches; }
@@ -649,78 +656,53 @@ thread_local TranMeta tls_tmeta1;     // convtran1 attached to zm_conv_tend_batc
 thread_local TranMeta tls_tmeta1c;    // convtran1 of the host-pointer zm_conv_tend_batch (compact: active slices only)
 thread_local std::vector<int> tls_tran1_flags;   // host copy of (doconvtran, cnst_is_dry) given to zm_convtran1_fields
 
-// a.active / a.is_dry / a.nactive and the chunk bounds are set: zero the active slices, transport
-int convtran_enqueue(cudaStream_t s, TranArgs a, const ChunkBounds& cb) {
+// convtran's arguments: `nactive` constituents active[0, nactive) of ncnst with their dry flags, the mass-flux
+// fields of f; convtran_enqueue sets the chunk bounds
+TranArgs tran_args(int nchunks, int ncnst, int nactive, const int* active, const int* is_dry, const MassFlux& f,
+                   const double* q, const double* fracis, const double* dpdry, double* dqdt) {
+  TranArgs a{};
+  a.nchunks = nchunks; a.ncnst = ncnst; a.nactive = nactive; a.active = active; a.is_dry = is_dry;
+  a.jt = f.jt; a.mx = f.maxg; a.ideep = f.ideep; a.lengath = f.lengath;
+  a.mu = f.mu; a.md = f.md; a.du = f.du; a.eu = f.eu; a.ed = f.ed; a.dp = f.dp;
+  a.q = q; a.fracis = fracis; a.dpdry = dpdry; a.dqdt = dqdt;
+  return a;
+}
+
+// Transport with the chunk bounds cb.  rbase == nullptr: the dense form on (pcols,pver,ncnst) chunk arrays, which zeroes
+// the active slices of dqdt.  Otherwise q / fracis / dqdt are the convective columns' records
+// (zm_conv_tend_2_batch_gathered) and rbase[c] is chunk c's first record column (k_lengath_scan): every record element
+// is written, so there is no zero-fill launch, and the block kernel takes any dqdt alignment.
+int convtran_enqueue(cudaStream_t s, TranArgs a, const ChunkBounds& cb, const int* rbase = nullptr) {
   const int pcols = g_params.pcols, pver = g_params.pver;
   const int ncolpad = a.nchunks * pcols;
   if (a.nactive == 0) return 0;
   a.ktm = cb.ktm; a.kbm = cb.kbm; a.slots = cb.slots; a.count = cb.count;
+  const bool gath = rbase != nullptr;
   // block per (chunk, constituent group) with every row of q / fracis / dqdt moved once (ZM_CONVTRAN_KERNEL=t keeps
   // the thread-per-(column, constituent) kernel, which also serves shapes whose work arrays do not fit an SM)
   static const bool force_t = [] { const char* e = getenv("ZM_CONVTRAN_KERNEL"); return e && e[0] == 't'; }();
-  if (!force_t && convtran_c_fits(pver, pcols) && (reinterpret_cast<uintptr_t>(a.dqdt) & 15) == 0) {
+  if (!force_t && convtran_c_fits(pver, pcols) && (gath || (reinterpret_cast<uintptr_t>(a.dqdt) & 15) == 0)) {
+    const auto kc = gath ? k_convtran_c<true> : k_convtran_c<false>;
     const size_t smem = convtran_c_smem_bytes(pver, pcols);
-    static size_t smem_set = 0;
-    if (smem > smem_set) {
-      CK(cudaFuncSetAttribute(k_convtran_c<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      smem_set = smem;
+    static size_t smem_set[2] = {0, 0};      // the opt-in belongs to each instantiation: [gath]
+    if (smem > smem_set[gath]) {
+      CK(cudaFuncSetAttribute(kc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      smem_set[gath] = smem;
     }
     const int bpc = convtran_c_blocks_per_chunk(a.nactive, pcols);
-    k_convtran_c<false><<<(unsigned)((size_t)a.nchunks * bpc), 32 * CTC_NW, smem, s>>>(a, bpc, nullptr); ++tls_launches;
+    kc<<<(unsigned)((size_t)a.nchunks * bpc), 32 * CTC_NW, smem, s>>>(a, bpc, rbase); ++tls_launches;
     CK(cudaGetLastError());
     return 0;
   }
-  k_convtran_zero<<<a.nchunks * a.nactive, 128, 0, s>>>(a); ++tls_launches;
+  if (!gath) { k_convtran_zero<<<a.nchunks * a.nactive, 128, 0, s>>>(a); ++tls_launches; }
   const int cpb = convtran_cnst_per_block(pver);
   dim3 blk(32, cpb);
   dim3 grd((a.nactive + cpb - 1) / cpb, (ncolpad + 31) / 32);       // x: constituent groups, y: column groups
-  k_convtran_t<false><<<grd, blk, 0, s>>>(a, nullptr);
+  const auto kt = gath ? k_convtran_t<true> : k_convtran_t<false>;
+  kt<<<grd, blk, 0, s>>>(a, rbase);
   ++tls_launches;
   CK(cudaGetLastError());
   return 0;
-}
-
-// The same transport on the convective columns' records (zm_conv_tend_2_batch_gathered): q / fracis / dqdt are record
-// buffers and rbase[c] is chunk c's first record column (k_lengath_scan).  Every record element is written, so there
-// is no zero-fill launch; the block kernel takes any dqdt alignment.  One launch.
-int convtran_enqueue_gathered(cudaStream_t s, TranArgs a, const int* rbase, const ChunkBounds& cb) {
-  const int pcols = g_params.pcols, pver = g_params.pver;
-  const int ncolpad = a.nchunks * pcols;
-  if (a.nactive == 0) return 0;
-  a.ktm = cb.ktm; a.kbm = cb.kbm; a.slots = cb.slots; a.count = cb.count;
-  static const bool force_t = [] { const char* e = getenv("ZM_CONVTRAN_KERNEL"); return e && e[0] == 't'; }();
-  if (!force_t && convtran_c_fits(pver, pcols)) {
-    const size_t smem = convtran_c_smem_bytes(pver, pcols);
-    static size_t smem_set = 0;
-    if (smem > smem_set) {
-      CK(cudaFuncSetAttribute(k_convtran_c<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      smem_set = smem;
-    }
-    const int bpc = convtran_c_blocks_per_chunk(a.nactive, pcols);
-    k_convtran_c<true><<<(unsigned)((size_t)a.nchunks * bpc), 32 * CTC_NW, smem, s>>>(a, bpc, rbase); ++tls_launches;
-    CK(cudaGetLastError());
-    return 0;
-  }
-  const int cpb = convtran_cnst_per_block(pver);
-  dim3 blk(32, cpb);
-  dim3 grd((a.nactive + cpb - 1) / cpb, (ncolpad + 31) / 32);
-  k_convtran_t<true><<<grd, blk, 0, s>>>(a, rbase);
-  ++tls_launches;
-  CK(cudaGetLastError());
-  return 0;
-}
-
-int convtran_launch(Workspace& ws, cudaStream_t s, TranArgs a, const int* doconvtran_h,
-                    const int* is_dry_h) {
-  const int ncolpad = a.nchunks * g_params.pcols;
-  if (tls_tmeta.set(doconvtran_h, is_dry_h, a.ncnst)) return -100;
-  a.nactive = tls_tmeta.nactive;
-  if (a.nactive == 0) return 0;
-  a.active = tls_tmeta.active(); a.is_dry = tls_tmeta.dry();
-  if (ws.ensure(chunk_bounds_bytes(a.nchunks, ncolpad))) return -100;
-  ChunkBounds cb;
-  if (chunk_bounds_enqueue(ws, s, a.nchunks, a.jt, a.mx, a.lengath, cb)) return -100;
-  return convtran_enqueue(s, a, cb);
 }
 
 // ---- zm_conv_tend glue (zm_conv_intr.F90:662-836) ------------------------------------------------
@@ -860,6 +842,24 @@ __global__ void k_dpdry_gather_rec(int nchunks, const int* lengath, const int* b
       dpdry[(size_t)c * nper + r] = v;
     }
   }
+}
+
+// zm_conv_tend_2 (zm_conv_intr.F90:1014-1024) on stream s: dpdry gather, chunk bounds, convtran.  ws is sized by the
+// caller for dpdry and the chunk bounds and may hold the caller's staged arrays already, so it is not reset here.
+int conv_tend_2_enqueue(Workspace& ws, cudaStream_t s, int nchunks, const TranMeta& m, const MassFlux& f,
+                        const double* q, const double* fracis, const double* pdeldry, double* dqdt) {
+  double* dpdry = ws.take<double>((size_t)nchunks * g_params.pcols * g_params.pver);
+  for (auto e : ws.tev) cudaEventDestroy(e);
+  ws.tev.clear(); ws.tnames.clear();
+  tick(ws, s, "start");
+  // dpdry(i,:) = pdeldry(ideep(i),:)/100 for i <= lengath, else 0 (zm_conv_intr.F90:1014-1017)
+  k_dpdry_gather<<<1184, 256, 0, s>>>(nchunks, f.ideep, f.lengath, pdeldry, dpdry); ++tls_launches;
+  ChunkBounds cb;
+  if (chunk_bounds_enqueue(ws, s, nchunks, f.jt, f.maxg, f.lengath, cb)) return -100;
+  const int rc = convtran_enqueue(s, tran_args(nchunks, m.ncnst, m.nactive, m.active(), m.dry(), f, q, fracis, dpdry,
+                                               dqdt), cb);
+  tick(ws, s, "convtran2");
+  return rc;
 }
 
 // ---- diagnostics kernels ----------------------------------------------------------------------
@@ -1233,16 +1233,14 @@ int zm_momtran_batch_dev(int nchunks, const int* ncol, const int* domomtran, con
   if (nchunks <= 0) return 0;
   if (ncnst != 2) { tls_err = "momtran: ncnst must be 2 (u,v), as at its only call site zm_conv_intr.F90:822"; return -6; }
   Workspace& ws = tls_work;
-  if (!ws.stream && ws.ensure(0)) return -100;
+  if (ws.ensure(chunk_bounds_bytes(nchunks, nchunks * g_params.pcols))) return -100;
   cudaStream_t s = (cudaStream_t)stream;      // NULL = the CUDA default stream
-  MomArgs a;
-  a.nchunks = nchunks; a.ncnst = ncnst; a.ncol = ncol; a.jt = jt; a.mx = mx; a.ideep = ideep;
-  a.lengath = lengath; a.ktm = nullptr; a.kbm = nullptr; a.slots = nullptr; a.count = nullptr;
+  MomArgs a = mom_args(nchunks, ncol, MassFlux{mu, md, du, eu, ed, dp, jt, mx, ideep, lengath}, dt);
   a.domom[0] = domomtran[0]; a.domom[1] = domomtran[1];
-  a.q = q; a.mu = mu; a.md = md; a.du = du; a.eu = eu; a.ed = ed; a.dp = dp;
-  a.dqdt = dqdt; a.pguall = pguall; a.pgdall = pgdall; a.icwu = icwu; a.icwd = icwd; a.seten = seten;
-  a.dt = dt;
-  return momtran_launch(ws, s, a);
+  a.q = q; a.dqdt = dqdt; a.pguall = pguall; a.pgdall = pgdall; a.icwu = icwu; a.icwd = icwd; a.seten = seten;
+  ChunkBounds cb;
+  if (chunk_bounds_enqueue(ws, s, nchunks, jt, mx, lengath, cb)) return -100;
+  return momtran_launch(s, a, cb);
 }
 
 int zm_momtran_batch(int nchunks, const int* ncol, const int* domomtran, const double* q, int ncnst,
@@ -1287,12 +1285,14 @@ int zm_convtran_batch_dev(int nchunks, const int* doconvtran, const double* q, i
   Workspace& ws = tls_work;
   if (!ws.stream && ws.ensure(0)) return -100;
   cudaStream_t s = (cudaStream_t)stream;      // NULL = the CUDA default stream
-  TranArgs a;
-  a.nchunks = nchunks; a.ncnst = ncnst; a.nactive = 0; a.jt = jt; a.mx = mx; a.ideep = ideep;
-  a.lengath = lengath; a.ktm = nullptr; a.kbm = nullptr; a.active = nullptr; a.is_dry = nullptr;
-  a.q = q; a.fracis = fracis; a.mu = mu; a.md = md; a.du = du; a.eu = eu; a.ed = ed; a.dp = dp;
-  a.dpdry = dpdry; a.dqdt = dqdt;
-  return convtran_launch(ws, s, a, doconvtran, cnst_is_dry);
+  if (tls_tmeta.set(doconvtran, cnst_is_dry, ncnst)) return -100;
+  const TranMeta& m = tls_tmeta;
+  if (m.nactive == 0) return 0;
+  if (ws.ensure(chunk_bounds_bytes(nchunks, nchunks * g_params.pcols))) return -100;
+  ChunkBounds cb;
+  if (chunk_bounds_enqueue(ws, s, nchunks, jt, mx, lengath, cb)) return -100;
+  const MassFlux f{mu, md, du, eu, ed, dp, jt, mx, ideep, lengath};
+  return convtran_enqueue(s, tran_args(nchunks, ncnst, m.nactive, m.active(), m.dry(), f, q, fracis, dpdry, dqdt), cb);
 }
 
 int zm_convtran_batch(int nchunks, const int* doconvtran, const double* q, int ncnst, const double* mu,
@@ -1376,6 +1376,7 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
              mu, md, du, eu, ed, dp, dsubcld, jt, maxg, ideep, lengath, ql, rliq, dif, dnlf, dnif, rice};
   o.mcon_kgm2s = 1;                            // unit conversion of zm_conv_intr.F90:693 inside the plume kernel
   in.org = g_params.zm_org ? org : nullptr;
+  const MassFlux mf{mu, md, du, eu, ed, dp, jt, maxg, ideep, lengath};
   // ptend_u / ptend_v / seten are zero outside the convective columns momtran writes, and everywhere with cam3 (no
   // momtran, zm_conv_intr.F90:808; seten is then filled only when attached) -- filled with zm_convr's own outputs at
   // the start of the step.  momtran's diagnostics: pguall / pgdall are zero outside the convective columns; with cam3
@@ -1430,15 +1431,12 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
     tran_stream = ws.side2;
   }
   if (do_mom) {
-    MomArgs ma;
-    ma.nchunks = nchunks; ma.ncnst = 2; ma.ncol = ncol; ma.jt = jt; ma.mx = maxg; ma.ideep = ideep;
-    ma.lengath = lengath; ma.ktm = nullptr; ma.kbm = nullptr; ma.domom[0] = 1; ma.domom[1] = 1;
-    ma.q = nullptr; ma.mu = mu; ma.md = md; ma.du = du; ma.eu = eu; ma.ed = ed; ma.dp = dp;
-    ma.dqdt = nullptr; ma.pguall = pgu; ma.pgdall = pgd; ma.icwu = icwu; ma.icwd = icwd; ma.seten = seten;
-    ma.dt = ztodt;
+    MomArgs ma = mom_args(nchunks, ncol, mf, ztodt);
+    ma.domom[0] = 1; ma.domom[1] = 1;
+    ma.pguall = pgu; ma.pgdall = pgd; ma.icwu = icwu; ma.icwd = icwd; ma.seten = seten;
     ma.q_u = u; ma.q_v = v; ma.dq_u = ptend_u; ma.dq_v = ptend_v;
     if (hist_mom) { k_icw_init<<<1184, 256, 0, s>>>(nchunks, ncol, u, v, icwu, icwd); ++tls_launches; }
-    rc = momtran_launch(ws, s, ma, false, &cb);
+    rc = momtran_launch(s, ma, cb);
     if (rc) return rc;
   }
   tick(ws, s, "momtran");
@@ -1447,12 +1445,8 @@ int conv_tend_impl(Workspace& ws, int nchunks, const int* ncol, const double* t,
     // was updated); fake_dpdry = 0 (the transported species are moist; a zeroed array stands in if one is 'dry')
     double* fake_dpdry = ws.take<double>(n2);
     if (tr1->any_dry) CK(cudaMemsetAsync(fake_dpdry, 0, n2 * sizeof(double), tran_stream));
-    TranArgs ta;
-    ta.nchunks = nchunks; ta.ncnst = tr1->ncnst; ta.nactive = tr1->nactive; ta.jt = jt; ta.mx = maxg; ta.ideep = ideep;
-    ta.lengath = lengath; ta.active = tr1->active; ta.is_dry = tr1->is_dry;
-    ta.q = tr1->q; ta.fracis = tr1->fracis; ta.mu = mu; ta.md = md; ta.du = du; ta.eu = eu; ta.ed = ed; ta.dp = dp;
-    ta.dpdry = fake_dpdry; ta.dqdt = tr1->dqdt;
-    rc = convtran_enqueue(tran_stream, ta, cb);
+    rc = convtran_enqueue(tran_stream, tran_args(nchunks, tr1->ncnst, tr1->nactive, tr1->active, tr1->is_dry, mf, tr1->q,
+                                                 tr1->fracis, fake_dpdry, tr1->dqdt), cb);
     if (rc) return rc;
     if (tran_stream != s) CK(cudaEventRecord(ws.ev_join2, ws.side2));
     tick(ws, s, "convtran1");
@@ -1612,7 +1606,7 @@ static int conv_tend_batch(int nchunks, const int* ncol, const double* t, const 
   int *d_jt = (int*)dev(jt, s1, 4, 2), *d_maxg = (int*)dev(maxg, s1, 4, 2), *d_ideep = (int*)dev(ideep, s1, 4, 2),
       *d_len = (int*)dev(g ? nullptr : lengath, 1, 4, 2);
   to_mirror = false;
-  const PbufMirror new_mirror{nchunks, d_mu, d_md, d_du, d_eu, d_ed, d_dp, d_dsub, d_jt, d_maxg, d_ideep, d_len};
+  const PbufMirror new_mirror{nchunks, {d_mu, d_md, d_du, d_eu, d_ed, d_dp, d_jt, d_maxg, d_ideep, d_len}, d_dsub};
   double *d_ps = SPF(SF_PS, ptend_s, s2), *d_pq = SPF(SF_PQ, ptend_q, s2), *d_pu = SPF(SF_PU, ptend_u, s2),
          *d_pv = SPF(SF_PV, ptend_v, s2), *d_mcon = SPF(SF_MCON, mcon, s2p), *d_cme = SPE(SF_CME, cme, s2),
          *d_pflx = SPE(SF_PFLX, pflx, s2p), *d_zdu = SPE(SF_ZDU, zdu, s2),
@@ -1965,7 +1959,7 @@ int zm_conv_tend_diag_batch(int nchunks, const int* ncol, const double* ps, cons
   const size_t pc = g_params.pcols, L = g_params.pver, nc = (size_t)nchunks * pc, n2 = nc * L;
   const bool from_mirror = !(mu && md && jt && maxg && ideep && lengath);
   const PbufMirror M = tls_mirror;
-  if (from_mirror && (M.nchunks != nchunks || !M.mu)) {
+  if (from_mirror && (M.nchunks != nchunks || !M.f.mu)) {
     tls_err = "zm_conv_tend_diag_batch: no device mirror from a zm_conv_tend_batch call with the same nchunks on this thread";
     return -7;
   }
@@ -1974,9 +1968,9 @@ int zm_conv_tend_diag_batch(int nchunks, const int* ncol, const double* ps, cons
   Stager S(st);
   const int* d_ncol = S.in(ncol, nchunks);
   const double *d_ps = S.in(ps, nc), *d_pmid = S.in(pmid, n2);
-  const double *d_mu = from_mirror ? M.mu : S.in(mu, n2), *d_md = from_mirror ? M.md : S.in(md, n2);
-  const int *d_jt = from_mirror ? M.jt : S.in(jt, nc), *d_mx = from_mirror ? M.maxg : S.in(maxg, nc),
-            *d_id = from_mirror ? M.ideep : S.in(ideep, nc), *d_len = from_mirror ? M.lengath : S.in(lengath, nchunks);
+  const double *d_mu = from_mirror ? M.f.mu : S.in(mu, n2), *d_md = from_mirror ? M.f.md : S.in(md, n2);
+  const int *d_jt = from_mirror ? M.f.jt : S.in(jt, nc), *d_mx = from_mirror ? M.f.maxg : S.in(maxg, nc),
+            *d_id = from_mirror ? M.f.ideep : S.in(ideep, nc), *d_len = from_mirror ? M.f.lengath : S.in(lengath, nchunks);
   double *d_f = S.out(freqzm, nc), *d_muo = S.out(mu_out, n2), *d_mdo = S.out(md_out, n2), *d_pt = S.out(pcont, nc),
          *d_pb = S.out(pconb, nc);
   int rc = zm_conv_tend_diag_batch_dev(nchunks, d_ncol, d_ps, d_pmid, d_mu, d_md, d_jt, d_mx, d_id, d_len, d_f, d_muo,
@@ -2033,26 +2027,12 @@ int zm_conv_tend_2_batch_dev(int nchunks, const int* doconvtran, const double* q
   (void)dsubcld; (void)ztodt;
   if (nchunks <= 0) return 0;
   const size_t pc = g_params.pcols, L = g_params.pver, nc = (size_t)nchunks * pc, n2 = nc * L;
-  cudaStream_t s = (cudaStream_t)stream;
   if (tls_tmeta.set(doconvtran, cnst_is_dry, pcnst)) return -100;
   if (tls_tmeta.nactive == 0) return 0;
   Workspace& ws = tls_work;
   if (ws.ensure(chunk_bounds_bytes(nchunks, (int)nc) + al(n2, 8) + 1024)) return -100;
-  double* dpdry = ws.take<double>(n2);
-  for (auto e : ws.tev) cudaEventDestroy(e);
-  ws.tev.clear(); ws.tnames.clear();
-  tick(ws, s, "start");
-  k_dpdry_gather<<<1184, 256, 0, s>>>(nchunks, ideep, lengath, pdeldry, dpdry); ++tls_launches;
-  TranArgs a;
-  a.nchunks = nchunks; a.ncnst = pcnst; a.nactive = tls_tmeta.nactive; a.jt = jt; a.mx = maxg; a.ideep = ideep;
-  a.lengath = lengath; a.active = tls_tmeta.active(); a.is_dry = tls_tmeta.dry();
-  a.q = q; a.fracis = fracis; a.mu = mu; a.md = md; a.du = du; a.eu = eu; a.ed = ed; a.dp = dp;
-  a.dpdry = dpdry; a.dqdt = ptend_q;
-  ChunkBounds cb;
-  if (chunk_bounds_enqueue(ws, s, nchunks, jt, maxg, lengath, cb)) return -100;
-  const int rc = convtran_enqueue(s, a, cb);
-  tick(ws, s, "convtran2");
-  return rc;
+  return conv_tend_2_enqueue(ws, (cudaStream_t)stream, nchunks, tls_tmeta,
+                             MassFlux{mu, md, du, eu, ed, dp, jt, maxg, ideep, lengath}, q, fracis, pdeldry, ptend_q);
 }
 
 // zm_conv_tend_2 (zm_conv_intr.F90:955-1028): convtran over the constituents flagged convtran2, with the
@@ -2060,31 +2040,26 @@ int zm_conv_tend_2_batch_dev(int nchunks, const int* doconvtran, const double* q
 int zm_conv_tend_2_batch(int nchunks, const int* doconvtran, const double* q, int pcnst, const double* pdeldry,
                          const double* fracis, double* ptend_q, double ztodt, const int* cnst_is_dry) {
   NEED_INIT();
+  (void)ztodt;
   tls_t2_h2d = tls_t2_d2h = 0;
   if (nchunks <= 0) return 0;
   const PbufMirror M = tls_mirror;
-  if (M.nchunks != nchunks || !M.mu) {
+  if (M.nchunks != nchunks || !M.f.mu) {
     tls_err = "zm_conv_tend_2_batch: no device mirror from a zm_conv_tend_batch call with the same nchunks on this thread";
     return -7;
   }
   const size_t pc = g_params.pcols, L = g_params.pver, nc = (size_t)nchunks * pc, n2 = nc * L, n3 = n2 * pcnst;
+  if (tls_tmeta.set(doconvtran, cnst_is_dry, pcnst)) return -100;
   Workspace& st = tls_stage2;
-  if (st.ensure(2 * al(n2, 8) + 3 * al(n3, 8) + 4096)) return -100;
+  // staged arrays, then dpdry and the chunk bounds of conv_tend_2_enqueue
+  if (st.ensure(2 * al(n2, 8) + 3 * al(n3, 8) + chunk_bounds_bytes(nchunks, (int)nc) + 4096)) return -100;
   Stager S(st);
   const double *d_q = S.in(q, n3), *d_fr = S.in(fracis, n3), *d_pdd = S.in(pdeldry, n2);
-  double* d_dpdry = st.take<double>(n2);
   double* d_dqdt = S.inout(ptend_q, n3);
   tls_t2_h2d = (long long)(3 * n3 + n2) * (long long)sizeof(double);     // q, fracis, pdeldry, ptend_q (inout)
-  // dpdry(i,:) = pdeldry(ideep(i),:)/100 for i <= lengath, else 0 (zm_conv_intr.F90:1014-1017)
-  k_dpdry_gather<<<1184, 256, 0, st.stream>>>(nchunks, M.ideep, M.lengath, d_pdd, d_dpdry); ++tls_launches;
-  for (auto e : st.tev) cudaEventDestroy(e);
-  st.tev.clear(); st.tnames.clear();
-  tick(st, st.stream, "start");
-  int rc = zm_convtran_batch_dev(nchunks, doconvtran, d_q, pcnst, M.mu, M.md, M.du, M.eu, M.ed, M.dp, M.dsubcld,
-                                 M.jt, M.maxg, M.ideep, M.lengath, d_fr, d_dqdt, d_dpdry, ztodt, cnst_is_dry,
-                                 (void*)st.stream);
+  int rc = 0;
+  if (tls_tmeta.nactive > 0) rc = conv_tend_2_enqueue(st, st.stream, nchunks, tls_tmeta, M.f, d_q, d_fr, d_pdd, d_dqdt);
   if (rc) return rc;
-  tick(st, st.stream, "convtran2");
   rc = S.flush();
   if (rc == 0) tls_t2_d2h = (long long)n3 * (long long)sizeof(double);
   return rc;
@@ -2101,7 +2076,7 @@ int zm_conv_tend_2_batch_gathered(int nchunks, const int* lengath, const int* do
   tls_t2_h2d = tls_t2_d2h = 0;
   if (nchunks <= 0) return 0;
   const PbufMirror M = tls_mirror;
-  if (M.nchunks != nchunks || !M.mu) {
+  if (M.nchunks != nchunks || !M.f.mu) {
     tls_err = "zm_conv_tend_2_batch_gathered: no device mirror from a zm_conv_tend_batch call with the same nchunks on "
               "this thread";
     return -7;
@@ -2126,7 +2101,7 @@ int zm_conv_tend_2_batch_gathered(int nchunks, const int* lengath, const int* do
   if (!st.stream && st.ensure(0)) return -100;
   // the caller's lengath must be the mirror's: the records were packed with it and the kernels address them with it
   std::vector<int> mlen(nchunks);
-  CK(cudaMemcpyAsync(mlen.data(), M.lengath, nchunks * sizeof(int), cudaMemcpyDeviceToHost, st.stream));
+  CK(cudaMemcpyAsync(mlen.data(), M.f.lengath, nchunks * sizeof(int), cudaMemcpyDeviceToHost, st.stream));
   CK(cudaStreamSynchronize(st.stream));
   tls_t2_d2h = (long long)nchunks * (long long)sizeof(int);
   long long ncols = 0;
@@ -2155,24 +2130,21 @@ int zm_conv_tend_2_batch_gathered(int nchunks, const int* lengath, const int* do
   double* d_dqdt = S.out(dqdt_rec, nrec);
   tls_t2_h2d = (long long)(2 * nrec + npd) * (long long)sizeof(double);
   int* d_base = st.take<int>(nchunks + 1);
-  k_lengath_scan<<<1, 256, 0, st.stream>>>(nchunks, M.lengath, d_base); ++tls_launches;
+  k_lengath_scan<<<1, 256, 0, st.stream>>>(nchunks, M.f.lengath, d_base); ++tls_launches;
   double* d_dpdry = nullptr;
   if (any_dry) {
     // dpdry(i,:) = pdeldry(ideep(i),:)/100 for i <= lengath, else 0 (zm_conv_intr.F90:1014-1017), slot layout
     d_dpdry = st.take<double>(n2);
-    k_dpdry_gather_rec<<<1184, 256, 0, st.stream>>>(nchunks, M.lengath, d_base, d_pdd, d_dpdry); ++tls_launches;
+    k_dpdry_gather_rec<<<1184, 256, 0, st.stream>>>(nchunks, M.f.lengath, d_base, d_pdd, d_dpdry); ++tls_launches;
   }
   for (auto e : st.tev) cudaEventDestroy(e);
   st.tev.clear(); st.tnames.clear();
   tick(st, st.stream, "start");
-  TranArgs a;
-  a.nchunks = nchunks; a.ncnst = pcnst; a.nactive = tls_tmeta.nactive; a.jt = M.jt; a.mx = M.maxg; a.ideep = M.ideep;
-  a.lengath = M.lengath; a.active = tls_tmeta.active(); a.is_dry = tls_tmeta.dry();
-  a.q = d_q; a.fracis = d_fr; a.mu = M.mu; a.md = M.md; a.du = M.du; a.eu = M.eu; a.ed = M.ed; a.dp = M.dp;
-  a.dpdry = d_dpdry; a.dqdt = d_dqdt;
   ChunkBounds cb;
-  if (chunk_bounds_enqueue(st, st.stream, nchunks, M.jt, M.maxg, M.lengath, cb)) return -100;
-  int rc = convtran_enqueue_gathered(st.stream, a, d_base, cb);
+  if (chunk_bounds_enqueue(st, st.stream, nchunks, M.f.jt, M.f.maxg, M.f.lengath, cb)) return -100;
+  const TranMeta& m = tls_tmeta;
+  int rc = convtran_enqueue(st.stream, tran_args(nchunks, pcnst, m.nactive, m.active(), m.dry(), M.f, d_q, d_fr, d_dpdry,
+                                                 d_dqdt), cb, d_base);
   if (rc) return rc;
   tick(st, st.stream, "convtran2");
   rc = S.flush();
